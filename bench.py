@@ -54,6 +54,7 @@ ALGO_BYTES_PER_ROW = 111  # SURVEY.md 8d
 # SURVEY.md 8d nominal FP64 flop model per log-density-gradient evaluation
 FLOPS_PER_GRAD = {0: 300 * 30 + 55, 1: 190 * 30 + 165, 2: 300 * 15 + 55, 3: 190 * 15 + 165, 4: 300 * 15 + 55, 5: 190 * 15 + 165}
 NCU_METRICS = os.path.join(ROOT, "profiles", "r02_ncu_metrics.json")  # written by tools/ncu_metrics.py from the .ncu-rep files
+DUMP_BYTES = 64 * 10**6  # --dump-outputs: bytes written in all
 
 
 def model_flops(leapfrogs, max_position):
@@ -189,7 +190,7 @@ def cpu_baseline(g, cores, n_sample=None):
             why = f"numpyro importable but the reference did not run: {type(exc).__name__}: {exc}"
     from oracle import oracle as O
 
-    O.build()
+    # loads the library the build left; nothing is compiled at run time, the tree may be read-only
     cfg = O.default_config()
     t0 = time.perf_counter()
     out = O.fit_batch(g["tax_ids"][pick], g["k"][pick], g["N"][pick], cfg, n_threads=cores)
@@ -304,6 +305,70 @@ class DeviceBatch:
                 noise=torch.empty((n_in_tax, 3), dtype=torch.float64, device=dev))
             self.sets.append(dict(outs=outs, res=torch.empty(n_in_tax * FIT_RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev),
                                   med=torch.empty((3, n_in_tax, R), dtype=torch.float32, device=dev)))
+        self.last = None  # (output set, fitted TaxIDs) of the last step submitted
+
+
+def device_step_outputs(s, n_fit):
+    """The outputs of one device-resident step as float32 / float64 host arrays: the per-TaxID group (the
+    counts that fed the fit, every field of the fit result rows, the predictive median and HPDI) and the
+    per-input-row group of the counts stage."""
+    from metadamage_b200._abi import FIT_RESULT_DTYPE
+
+    def host(t, dtype, view=None):  # device tensor -> host array; `view`: the unsigned type its bits hold
+        a = t.cpu().numpy()
+        return (a if view is None else a.view(view)).astype(dtype)
+
+    o = s["outs"]
+    taxa = {"counts_tax_id": host(o["tax_id"][:n_fit], np.float64), "counts_k": host(o["k"][:n_fit], np.float64, np.uint32),
+            "counts_N": host(o["N"][:n_fit], np.float64, np.uint32), "counts_noise": host(o["noise"][:n_fit], np.float64)}
+    res = s["res"][:n_fit * FIT_RESULT_DTYPE.itemsize].cpu().numpy().view(FIT_RESULT_DTYPE)
+    for name in FIT_RESULT_DTYPE.names:
+        if name == "run":
+            for diag in res["run"].dtype.names:
+                taxa[f"fit_run_{diag}"] = res["run"][diag].astype(np.float64)  # [n_fit][6 runs]
+        else:
+            taxa[f"fit_{name}"] = res[name].astype(np.float64)
+    for i, name in enumerate(("median", "hpdi_lo", "hpdi_hi")):
+        taxa[f"fit_{name}"] = host(s["med"][i, :n_fit], np.float32)
+    rows = {"counts_n_fwd_ref": host(o["n_fwd_ref"], np.float64, np.uint32), "counts_n_rev_ref": host(o["n_rev_ref"], np.float64, np.uint32),
+            "counts_f_fwd": host(o["f_fwd"], np.float32), "counts_f_rev": host(o["f_rev"], np.float32), "counts_z": host(o["z"], np.float32),
+            "counts_y_sum_total": host(o["y_sum_total"], np.float64, np.uint64), "counts_keep": host(o["keep"], np.float32)}
+    return [taxa, rows]
+
+
+def finite_parts(group):
+    """Every file of a dump holds finite numbers. An array with NaN or +-inf entries (the noise statistic is NaN,
+    as in the reference, for a TaxID without usable mismatch counts) is written with 0 in their place, beside
+    <name>_nonfinite holding what each entry was: 0 finite, 1 NaN, 2 +inf, 3 -inf."""
+    out = {}
+    for name, a in group.items():
+        bad = ~np.isfinite(a)
+        if bad.any():
+            out[name + "_nonfinite"] = np.where(np.isnan(a), 1, np.where(a == np.inf, 2, np.where(bad, 3, 0))).astype(np.float32)
+            a = np.where(bad, 0, a).astype(a.dtype)
+        out[name] = a
+    return out
+
+
+def dump_outputs(directory, groups, budget, seed=0):
+    """Write every array of `groups` (dicts of arrays that share their first axis) as directory/<name>.npy, made
+    finite by `finite_parts`. The groups are taken in order; one that does not fit in what is left of `budget`
+    bytes (files, headers included) is cut to a fixed, seeded sample of its rows, the same rows in each of its
+    arrays, so equal runs write equal files."""
+    os.makedirs(directory, exist_ok=True)
+    for group in groups:
+        group = finite_parts(group)
+        n = len(next(iter(group.values())))
+        total = sum(a.nbytes for a in group.values())
+        room = max(budget - 256 * len(group), 0)  # an .npy header takes 128 bytes
+        keep = n if total <= room else room // -(-total // n)
+        if keep < n:
+            rows = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+            group = {name: a[rows] for name, a in group.items()}
+        for name, a in group.items():
+            path = os.path.join(directory, name + ".npy")
+            np.save(path, np.ascontiguousarray(a))
+            budget -= os.path.getsize(path)
 
 
 def main():
@@ -324,7 +389,15 @@ def main():
                     help="fitted TaxIDs per GPU of the extra single pass (default: 125 000 at N = 8 = BASELINE config 3's 1M TaxIDs, none otherwise)")
     ap.add_argument("--inflight", type=int, default=1, choices=[1, 2], help="batches in flight per GPU (MDG_MAX_INFLIGHT = 2)")
     ap.add_argument("--heuristic", type=int, default=0, help="find_heuristic_step_size (0 = numpyro 0.4.1 default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the device-resident path returned in its last timed step to DIR/<name>.npy "
+                         "(finite float32 / float64, NaN and inf marked in <name>_nonfinite.npy; at most 64 MB; "
+                         "under torchrun DIR/rank<r>/)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)
@@ -421,6 +494,7 @@ def main():
             o = s["outs"]
             ticket = ctx.fit_submit_device(o["tax_id"][:n_fit], o["k"][:n_fit], o["N"][:n_fit], s["res"], fit_cfg,
                                            median=s["med"][0], hpdi_lo=s["med"][1], hpdi_hi=s["med"][2], noise3=o["noise"][:n_fit])
+            b.last = (s, n_fit)
             return n_fit, ticket, t1
         return submit
 
@@ -430,6 +504,9 @@ def main():
         run_pipelined(args.warmup, submit_device, record=False)
     sampler = ClockSampler(local_rank).start()
     dev_ms, dev_fits, _ = timed(args.steps, submit_device)
+    if args.dump_outputs:  # before the paths below reuse the output buffers
+        where = args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}")
+        dump_outputs(where, device_step_outputs(*batch.last), DUMP_BYTES // world)
 
     # ---------------- host-buffer path (e2e) ----------------
     def pinned(a):

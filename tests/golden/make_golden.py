@@ -1,8 +1,8 @@
 """Generate the golden fixtures under tests/golden/ by running the REFERENCE's own functions.
 
-Run in the build container only (needs /root/reference; the GPU box does not have it):
+Run with a checkout of the reference project (no GPU needed):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py /path/to/reference
 
 The reference imports numpyro / jax / dask / ... at module level; none of them is installable
 offline, so they are replaced by inert stub modules here. Only reference functions that are
@@ -27,13 +27,14 @@ Outputs: counts_golden.npz, fits_golden.npz, topn_golden.npz, lookups_golden.npz
 import importlib
 import os
 import sys
+import tempfile
 import types
 import warnings
 
 import numpy as np
 import pandas as pd
 
-REF = "/root/reference"
+REF = None  # the reference checkout, from the command line
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -82,7 +83,7 @@ def load_reference():
     install_stubs()
     sys.path.insert(0, REF)
     cwd = os.getcwd()
-    os.chdir("/tmp")  # the reference's logger writes ./logs/
+    os.chdir(tempfile.gettempdir())  # the reference's logger writes ./logs/
     try:
         counts = importlib.import_module("metadamage.counts")
         fits = importlib.import_module("metadamage.fits")
@@ -349,7 +350,7 @@ def make_lookups_golden(fit_results_mod):
             our_io.Parquet(os.path.join(folder, "counts", f"{shortname}.parquet")).save(cn, metadata={"shortname": shortname})
             frames.append(df)
         cwd = os.getcwd()
-        os.chdir("/tmp")
+        os.chdir(tempfile.gettempdir())
         try:
             fr = fit_results_mod.FitResults(folder)
         finally:
@@ -401,6 +402,10 @@ def make_lookups_golden(fit_results_mod):
 
 
 def main():
+    global REF
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/make_golden.py /path/to/reference")
+    REF = os.path.abspath(sys.argv[1])
     counts, fits, utils = load_reference()
     c = make_counts_golden(counts)
     f = make_fits_golden(counts, fits)

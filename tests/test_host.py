@@ -322,3 +322,42 @@ def test_bench_workloads_follow_baseline_configs():
     assert eight["taxa_per_gpu"] * 8 == 1_000_000 and "model" not in eight
     src = open(os.path.join(root, "bench.py")).read()
     assert src.count("125_000") >= 2  # the default of both arms
+
+
+def test_bench_dump_outputs_budget_and_sample(tmp_path):
+    """bench.py --dump-outputs: every array lands as <name>.npy holding finite numbers only (NaN / inf marked in a
+    companion file); a group beyond the byte budget is cut to the same seeded rows in each of its arrays, and the
+    files stay within the budget."""
+    import sys
+
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    import bench
+
+    noise = np.linspace(0, 1, 300).reshape(100, 3)
+    noise[[3, 7], 1] = np.nan
+    noise[9] = [np.inf, -np.inf, np.nan]
+    taxa = {"fit_D_max": np.linspace(0, 1, 100), "fit_median": np.ones((100, 30), np.float32), "counts_noise": noise}
+    rows = {"counts_f_fwd": np.arange(50_000, dtype=np.float32), "counts_z": np.arange(50_000, dtype=np.float64) % 31}
+    budget = 200_000
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), [taxa, rows], budget)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["counts_f_fwd.npy", "counts_noise.npy", "counts_noise_nonfinite.npy", "counts_z.npy", "fit_D_max.npy", "fit_median.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= budget
+    for f in files:
+        a = np.load(tmp_path / "a" / f)
+        assert a.dtype in (np.float32, np.float64) and np.all(np.isfinite(a)), f
+        assert np.array_equal(a, np.load(tmp_path / "b" / f))
+    assert np.array_equal(np.load(tmp_path / "a" / "fit_median.npy"), taxa["fit_median"])  # the first group fits whole
+    # NaN / inf entries are written as 0 and marked: 1 NaN, 2 +inf, 3 -inf
+    code = np.load(tmp_path / "a" / "counts_noise_nonfinite.npy")
+    want = np.zeros((100, 3), np.float32)
+    want[[3, 7], 1] = 1
+    want[9] = [2, 3, 1]
+    assert np.array_equal(code, want)
+    ok = want == 0
+    assert np.array_equal(np.load(tmp_path / "a" / "counts_noise.npy")[ok], noise[ok])
+    assert np.all(np.load(tmp_path / "a" / "counts_noise.npy")[~ok] == 0)
+    f_fwd, z = np.load(tmp_path / "a" / "counts_f_fwd.npy"), np.load(tmp_path / "a" / "counts_z.npy")
+    assert 0 < len(f_fwd) < 50_000 and np.all(np.diff(f_fwd) > 0)
+    assert np.array_equal(z, f_fwd.astype(np.int64) % 31)  # the same rows in both arrays

@@ -1,7 +1,7 @@
 """Is a straggler chain posterior-driven or chain luck? The same counts under 64 different Philox keys (development tool)."""
 import os, sys
 import numpy as np
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from metadamage_b200 import _lib
 from metadamage_b200.backend import Context
 K0 = np.array([2, 1, 2, 1, 1, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 2, 1, 1, 2, 1, 1, 2, 0, 1, 0, 0, 0, 0, 1, 0], np.uint32)
