@@ -34,7 +34,14 @@
 #ifndef MDG_H
 #define MDG_H
 
+#include <stddef.h>
 #include <stdint.h>
+
+#ifdef __cplusplus
+#define MDG_STATIC_ASSERT(cond, msg) static_assert(cond, msg)
+#else
+#define MDG_STATIC_ASSERT(cond, msg) _Static_assert(cond, msg)
+#endif
 
 #ifdef __cplusplus
 extern "C" {
@@ -73,6 +80,8 @@ enum mdg_run_kind {
 #define MDG_FIT_BUDGET_EXCEEDED 0x8u /* a run needed more than cfg.max_leapfrogs_per_run gradient evaluations:
                                       * the bounded-work analogue of the reference's per-fit timeout
                                       * (fits.py:37-38, 472-474); always set together with MDG_FIT_FAILED */
+#define MDG_FIT_COV_INVALID 0x10u    /* mdg_map_batch: no Laplace covariance (the MAP fit did not converge, or the
+                                      * Hessian at the mode is not positive definite); the standard deviations are NaN */
 
 #ifndef MDG_MAX_INFLIGHT
 #define MDG_MAX_INFLIGHT 2         /* batches one ctx keeps in flight between mdg_fit_batch_submit and _wait */
@@ -186,6 +195,64 @@ typedef struct mdg_timings {
     float reserved1;
 } mdg_timings;
 
+/*
+ * MAP-only screening (mdg_map_batch). A MAP fit is the mode of the constrained-space posterior
+ * (likelihood x priors, no Jacobian term), found in the unconstrained coordinates u by LM-damped
+ * Newton; it is the same fit as mdg_fit_result.map_*. It is made for the six run kinds of
+ * enum mdg_run_kind (cfg.do_fwd_rev = 0: the two all-position ones only).
+ *
+ * Laplace covariance at the converged u*: H_u is the symmetrised central-difference Hessian of the
+ * analytic gradient of f = -log p (steps h_j = 1e-4 (1 + |u_j|), as in the Newton loop),
+ * Sigma_u = H_u^-1, and Sigma_theta = J Sigma_u J with J = diag(d theta_j / d u_j): theta (1 - theta)
+ * for q, A, c and exp(u_delta) for phi. f has no Jacobian term, so grad_u f = J grad_theta f and the
+ * second-order term of the change of variables vanishes at a stationary point: J H_u^-1 J is the
+ * inverse Hessian of f in theta.
+ */
+typedef struct mdg_map_run {
+    double q, A, c, phi;                 /* mode; null runs: A = c = NaN */
+    double q_std, A_std, c_std, phi_std; /* Laplace standard deviations; NaN with MDG_FIT_COV_INVALID (null: A, c NaN) */
+    double cov_Ac;                       /* Laplace covariance of A and c (PMD runs) */
+    double logp;                         /* log posterior at the mode incl. log C(N,k), no Jacobian (= map_logp) */
+    double loglik;                       /* sum over the run's positions of log BetaBinomial(k | N, alpha, beta) at the
+                                          * mode, incl. log C(N,k) */
+    uint32_t iters;                      /* Newton iterations */
+    uint32_t n_eval;                     /* gradient evaluations: Newton loop, log-likelihood and Laplace Hessian */
+    uint32_t flags;                      /* MDG_FIT_FAILED (no finite starting point), MDG_FIT_MAP_NOT_CONVERGED,
+                                          * MDG_FIT_COV_INVALID of this run; 0 = clean. A run that was not made
+                                          * (do_fwd_rev = 0) is all NaN with flags = n_eval = 0 */
+    uint32_t reserved;
+} mdg_map_run;
+
+/* One row per TaxID. D_max is A + c at the PMD mode, NOT the posterior predictive median that
+ * mdg_fit_result.D_max holds. lambda_LR = 2 (loglik_PMD - loglik_null) of the all-position fits,
+ * lambda_LR_P = exp(-max(lambda_LR, 0) / 2) (chi-square tail, 4 - 2 = 2 degrees of freedom),
+ * lambda_LR_z = -Phi^-1(lambda_LR_P) evaluated from log P (finite where P underflows). The null model
+ * is A = 0, a boundary point of the PMD model at which q is unidentified, so the chi-square
+ * reference does not hold: P and z are a screening scale, not calibrated p-values. */
+typedef struct mdg_map_result {
+    int64_t tax_id;
+    uint32_t status;       /* MDG_FIT_FAILED / MDG_FIT_MAP_NOT_CONVERGED / MDG_FIT_COV_INVALID of the two all-position runs */
+    uint32_t reserved;
+    double D_max;          /* A + c at the PMD mode */
+    double D_max_std;      /* sqrt(Sigma_AA + Sigma_cc + 2 Sigma_Ac) */
+    double significance;   /* D_max / D_max_std */
+    double rho_Ac;         /* Sigma_Ac / sqrt(Sigma_AA Sigma_cc) */
+    double lambda_LR, lambda_LR_P, lambda_LR_z;
+    double forward_D_max, forward_D_max_std, forward_lambda_LR;  /* same from the forward-only pair of fits */
+    double reverse_D_max, reverse_D_max_std, reverse_lambda_LR;  /* same from the reverse-only pair of fits */
+    double normalized_noise, normalized_noise_forward, normalized_noise_reverse;  /* as mdg_fit_result */
+    uint64_t N_z1_forward, N_z1_reverse, N_sum_forward, N_sum_reverse, N_sum_total;
+    uint64_t y_sum_forward, y_sum_reverse, y_sum_total;
+    mdg_map_run run[MDG_NUM_RUNS];
+} mdg_map_result;
+
+MDG_STATIC_ASSERT(sizeof(mdg_map_run) == 104, "mdg_map_run layout");
+MDG_STATIC_ASSERT(offsetof(mdg_map_run, loglik) == 80 && offsetof(mdg_map_run, flags) == 96, "mdg_map_run layout");
+MDG_STATIC_ASSERT(sizeof(mdg_map_result) == 832, "mdg_map_result layout");
+MDG_STATIC_ASSERT(offsetof(mdg_map_result, D_max) == 16 && offsetof(mdg_map_result, normalized_noise) == 120 &&
+                  offsetof(mdg_map_result, N_z1_forward) == 144 && offsetof(mdg_map_result, run) == 208,
+                  "mdg_map_result layout");
+
 int mdg_version(void);
 const char* mdg_last_error(void);
 int mdg_device_count(void);
@@ -270,6 +337,22 @@ int mdg_fit_batch(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
                   mdg_fit_result* out,
                   float* out_median, float* out_hpdi_lo, float* out_hpdi_hi,
                   double* out_samples, double* out_trace, double* out_waic);
+
+/*
+ * K3m — MAP-only screening of a dense batch: the six MAP fits of every TaxID (mdg_map_run), their Laplace
+ * covariances and the likelihood-ratio statistic, with no NUTS run and no NUTS scratch. Synchronous; the
+ * arguments and layouts are those of mdg_fit_batch (k, N: [n_tax][2*max_position]; mism12 / noise3 optional,
+ * both NULL -> noise NaN). From cfg only the priors, phi_min and do_fwd_rev are read. No random numbers: the
+ * result is a pure function of (k, N, cfg), so any partition of a batch is bit-identical, and the
+ * all-position fits equal mdg_fit_batch's map_* fields bit for bit. Any n_tax is taken in one call (the work
+ * is cut into pieces internally). Scratch is the ctx's own, apart from that of batches in flight through
+ * mdg_fit_batch_submit. mdg_ctx_get_timings afterwards: map_ms, assemble_ms, total_ms, n_launches, and
+ * leapfrogs[run] = gradient evaluations of that run kind summed over TaxIDs; the NUTS fields are 0.
+ */
+int mdg_map_batch(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
+                  const int64_t* tax_id, const uint32_t* k, const uint32_t* N,
+                  const uint32_t* mism12, const double* noise3,
+                  const mdg_fit_config* cfg, mdg_map_result* out);
 
 /*
  * K0 — tsv_parse: the step before the hot path (SURVEY.md 8f N2). Tokenises a mismatch-matrix

@@ -19,6 +19,7 @@ FIT_FAILED = 0x1
 FIT_MAP_NOT_CONVERGED = 0x2
 FIT_HAS_DIVERGENCES = 0x4
 FIT_BUDGET_EXCEEDED = 0x8
+FIT_COV_INVALID = 0x10
 
 
 class FitConfig(C.Structure):
@@ -144,6 +145,23 @@ FIT_RESULT_DTYPE = np.dtype(
     + [(name, "<u8") for name in _REFERENCE_INT_FIELDS]
     + [(name, "<f8") for name in _EXTRA_FLOAT_FIELDS]
     + [("run", RUN_DIAG_DTYPE, (NUM_RUNS,))],
+    align=True,
+)
+
+MAP_RUN_DTYPE = np.dtype(
+    [(name, "<f8") for name in ("q", "A", "c", "phi", "q_std", "A_std", "c_std", "phi_std", "cov_Ac", "logp", "loglik")]
+    + [("iters", "<u4"), ("n_eval", "<u4"), ("flags", "<u4"), ("reserved", "<u4")],
+    align=True,
+)
+
+MAP_RESULT_DTYPE = np.dtype(
+    [("tax_id", "<i8"), ("status", "<u4"), ("reserved", "<u4")]
+    + [(name, "<f8") for name in (
+        "D_max", "D_max_std", "significance", "rho_Ac", "lambda_LR", "lambda_LR_P", "lambda_LR_z",
+        "forward_D_max", "forward_D_max_std", "forward_lambda_LR", "reverse_D_max", "reverse_D_max_std", "reverse_lambda_LR",
+        "normalized_noise", "normalized_noise_forward", "normalized_noise_reverse")]
+    + [(name, "<u8") for name in _REFERENCE_INT_FIELDS]
+    + [("run", MAP_RUN_DTYPE, (NUM_RUNS,))],
     align=True,
 )
 

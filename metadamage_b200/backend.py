@@ -6,7 +6,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._abi import FIT_RESULT_DTYPE, MDG_DEVICE, MDG_HOST, NUM_RUNS, Timings, ptr
+from ._abi import FIT_RESULT_DTYPE, MAP_RESULT_DTYPE, MDG_DEVICE, MDG_HOST, NUM_RUNS, Timings, ptr
 
 BASES = "ACGT"
 OFFDIAG_COLUMNS = [r + o for r in BASES for o in BASES if r != o]  # AC,AG,AT,CA,CG,CT,GA,GC,GT,TA,TC,TG
@@ -357,6 +357,38 @@ class Context:
         res = ticket.get("result") or {}
         res["timings"] = self._timings_dict(t)
         return res
+
+    # ------------------------------------------------------------------ K3m MAP-only screening
+    def map_batch(self, tax_id, k, N, cfg=None, mism12=None, noise3=None):
+        """mdg_map_batch on host numpy arrays: six MAP fits per TaxID with Laplace uncertainties and the
+        likelihood-ratio statistic, no NUTS. Returns a MAP_RESULT_DTYPE array."""
+        cfg = cfg or _lib.default_config()
+        tax_id = np.ascontiguousarray(tax_id, dtype=np.int64)
+        k = np.ascontiguousarray(k, dtype=np.uint32)
+        N = np.ascontiguousarray(N, dtype=np.uint32)
+        if k.ndim != 2 or k.shape != N.shape or k.shape[0] != len(tax_id) or k.shape[1] % 2:
+            raise ValueError("k and N must be [n_tax][2*max_position]")
+        n_tax, R = k.shape
+        if mism12 is not None:
+            mism12 = np.ascontiguousarray(mism12, dtype=np.uint32)
+            if mism12.shape != (n_tax, R, 12):
+                raise ValueError("mism12 must be [n_tax][2*max_position][12]")
+        if noise3 is not None:
+            noise3 = np.ascontiguousarray(noise3, dtype=np.float64)
+        res = np.zeros(n_tax, dtype=MAP_RESULT_DTYPE)
+        _lib.check(self._lib.mdg_map_batch(self._h, MDG_HOST, n_tax, R // 2, ptr(tax_id), ptr(k), ptr(N), ptr(mism12),
+                                           ptr(noise3), C.byref(cfg), ptr(res)))
+        return res
+
+    def map_batch_device(self, tax_id, k, N, out, cfg=None, mism12=None, noise3=None):
+        """mdg_map_batch on torch CUDA tensors (k, N: [n_tax][2P] int32 bits of uint32); `out` is a uint8 CUDA tensor
+        of at least n_tax * MAP_RESULT_DTYPE.itemsize bytes. Synchronous."""
+        cfg = cfg or _lib.default_config()
+        n_tax, R = k.shape
+        if out.numel() * out.element_size() < n_tax * MAP_RESULT_DTYPE.itemsize:
+            raise ValueError("out buffer too small")
+        _lib.check(self._lib.mdg_map_batch(self._h, MDG_DEVICE, n_tax, R // 2, _dptr(tax_id), _dptr(k), _dptr(N), _dptr(mism12),
+                                           _dptr(noise3), C.byref(cfg), _dptr(out)))
 
     # ------------------------------------------------------------------ test hooks
     def lgamma_digamma(self, x):

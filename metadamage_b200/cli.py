@@ -1,6 +1,6 @@
 """`metadamage fit` command line (cli.py:97-159): same options and defaults, plus
 `--max-position` (documented upstream, README.md:121, but never wired: cli.py:105,143) and
-`--gpus`. The `dashboard` sub-command is a visualisation front-end outside this build's scope."""
+`--gpus`, and `--map-only` (MAP-only screening). The `dashboard` sub-command is a visualisation front-end outside this build's scope."""
 from pathlib import Path
 from typing import List, Optional
 
@@ -36,6 +36,8 @@ def cli_fit(
     substitution_bases_reverse: utils.SubstitutionBases = typer.Option(utils.SubstitutionBases.GA),
     forced: bool = typer.Option(False, "--forced"),
     gpus: int = typer.Option(1, help="number of B200s of this box to partition the TaxIDs over"),
+    map_only: bool = typer.Option(False, "--map-only", help="MAP fits with Laplace uncertainties and a likelihood-ratio "
+                                  "test only (no MCMC): writes map_results/<name>.parquet instead of the fit_* tables"),
 ):
     """Fitting Ancient Damage. FILENAMES are the mismatch-matrix files to fit, e.g.
 
@@ -52,7 +54,7 @@ def cli_fit(
         forced=forced, version="0.0.0", gpus=gpus,
     )
     cfg.add_filenames(filenames)
-    main(filenames, cfg)
+    main(filenames, cfg, map_only=map_only)
 
 
 @cli_app.command("dashboard")

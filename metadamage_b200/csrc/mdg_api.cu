@@ -12,6 +12,7 @@
 #include "mdg_tsv_kernel.cuh"
 #include "mdg_select_kernel.cuh"
 #include "mdg_post_kernels.cuh"
+#include "mdg_map_batch_kernel.cuh"
 #include "mdg_nuts_kernel.cuh"
 
 namespace mdg {
@@ -103,6 +104,8 @@ struct mdg_ctx {
     int64_t next_ticket_id = 1;
     double nuts_covered_until_ms = 0;  // union of NUTS intervals harvested so far ends here
     mdg_timings timings = {};
+    // mdg_map_batch: staged inputs / outputs (MDG_HOST), per-run records, counters; apart from the fit lanes' scratch
+    mdg::DevBuf map_in_tax, map_in_k, map_in_N, map_in_m12, map_in_noise, map_out, map_rec, map_counters;
 };
 
 using namespace mdg;
@@ -232,6 +235,23 @@ int launch_map(mdg_ctx* ctx, cudaStream_t st, const MapLaunch& ml, int npl) {
     } else {
         int grid = persistent_grid(map_kernel<4, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
         map_kernel<4, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
+    }
+    MDG_CUDA_TRY(cudaGetLastError());
+    ctx->timings.n_launches++;
+    return MDG_OK;
+}
+
+int launch_map_batch(mdg_ctx* ctx, cudaStream_t st, const MapBatchLaunch& ml, int npl) {
+    const long long items = (long long)ml.n_runs * ml.n_tax;
+    if (npl == 1) {
+        int grid = persistent_grid(map_batch_kernel<1, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
+        map_batch_kernel<1, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
+    } else if (npl == 2) {
+        int grid = persistent_grid(map_batch_kernel<2, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
+        map_batch_kernel<2, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
+    } else {
+        int grid = persistent_grid(map_batch_kernel<4, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
+        map_batch_kernel<4, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
     }
     MDG_CUDA_TRY(cudaGetLastError());
     ctx->timings.n_launches++;
@@ -376,6 +396,9 @@ void mdg_ctx_destroy(mdg_ctx* ctx) {
         if (ln.main) cudaStreamDestroy(ln.main);
         if (ln.h_leap) cudaFreeHost(ln.h_leap);
     }
+    for (mdg::DevBuf* b : {&ctx->map_in_tax, &ctx->map_in_k, &ctx->map_in_N, &ctx->map_in_m12, &ctx->map_in_noise, &ctx->map_out,
+                           &ctx->map_rec, &ctx->map_counters})
+        b->release();
     for (auto& tk : ctx->ticket) {
         for (mdg::DevBuf* b : {&tk.in_tax, &tk.in_k, &tk.in_N, &tk.in_m12, &tk.in_noise, &tk.out_res, &tk.out_med, &tk.smp, &tk.trace, &tk.waic})
             b->release();
@@ -1379,6 +1402,89 @@ int mdg_fit_batch(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position, const 
                                   out_hpdi_hi, out_samples, out_trace, out_waic, &ticket);
     if (rc) return rc;
     return mdg_fit_batch_wait(ctx, ticket, nullptr);
+}
+
+int mdg_map_batch(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position, const int64_t* tax_id, const uint32_t* k,
+                  const uint32_t* N, const uint32_t* mism12, const double* noise3, const mdg_fit_config* cfg, mdg_map_result* out) {
+    if (!ctx) { set_error("ctx is NULL"); return MDG_ERR_INVALID; }
+    if (!cfg || n_tax < 0 || max_position < 1 || max_position > MDG_MAX_POSITION || (mem != MDG_HOST && mem != MDG_DEVICE)) {
+        set_error("mdg_map_batch: invalid argument");
+        return MDG_ERR_INVALID;
+    }
+    if (n_tax > 0 && (!tax_id || !k || !N || !out)) { set_error("mdg_map_batch: NULL tax_id/k/N/out"); return MDG_ERR_INVALID; }
+    DeviceGuard guard(ctx->device);
+    cudaStream_t st = ctx->stream;
+    ctx->timings = mdg_timings{};
+    const int P = max_position, R = 2 * P;
+    const int n_runs = cfg->do_fwd_rev ? MDG_NUM_RUNS : 2;
+    const bool host = (mem == MDG_HOST);
+    const size_t nt = (size_t)n_tax;
+    // TaxIDs per piece: bounds the per-run records (624 MB per 2^20 TaxIDs); results go straight to their rows
+    const long long piece = 1ll << 20;
+    const long long piece_max = std::min<long long>(n_tax, piece);
+    int rc;
+    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
+    const int64_t* d_tax = tax_id; const uint32_t* d_k = k; const uint32_t* d_N = N; const uint32_t* d_m12 = mism12;
+    const double* d_noise = noise3;
+    mdg_map_result* d_out = out;
+    if (n_tax > 0 && host) {
+        if ((rc = ctx->map_in_tax.ensure(nt * 8))) return rc;
+        if ((rc = ctx->map_in_k.ensure(nt * R * 4))) return rc;
+        if ((rc = ctx->map_in_N.ensure(nt * R * 4))) return rc;
+        MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_tax.ptr, tax_id, nt * 8, cudaMemcpyHostToDevice, st));
+        MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_k.ptr, k, nt * R * 4, cudaMemcpyHostToDevice, st));
+        MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_N.ptr, N, nt * R * 4, cudaMemcpyHostToDevice, st));
+        d_tax = ctx->map_in_tax.as<int64_t>(); d_k = ctx->map_in_k.as<uint32_t>(); d_N = ctx->map_in_N.as<uint32_t>();
+        if (mism12) {
+            if ((rc = ctx->map_in_m12.ensure(nt * R * 12 * 4))) return rc;
+            MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_m12.ptr, mism12, nt * R * 12 * 4, cudaMemcpyHostToDevice, st));
+            d_m12 = ctx->map_in_m12.as<uint32_t>();
+        }
+        if (noise3) {
+            if ((rc = ctx->map_in_noise.ensure(nt * 24))) return rc;
+            MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_noise.ptr, noise3, nt * 24, cudaMemcpyHostToDevice, st));
+            d_noise = ctx->map_in_noise.as<double>();
+        }
+        if ((rc = ctx->map_out.ensure(nt * sizeof(mdg_map_result)))) return rc;
+        d_out = ctx->map_out.as<mdg_map_result>();
+    }
+    if ((rc = ctx->map_counters.ensure(256))) return rc;
+    unsigned int* d_counter = ctx->map_counters.as<unsigned int>();                           // [1] work counter
+    unsigned long long* d_evals = reinterpret_cast<unsigned long long*>(d_counter + 16);      // [6] gradient evaluations
+    MDG_CUDA_TRY(cudaMemsetAsync(d_counter, 0, 256, st));
+    if (n_tax > 0 && (rc = ctx->map_rec.ensure((size_t)piece_max * MDG_NUM_RUNS * sizeof(mdg_map_run)))) return rc;
+    const Priors pr = make_priors(*cfg);
+    const int npl = npl_for(R, 32);  // map_kernel's layout: the all-position fits are mdg_fit_batch's
+    for (long long c0 = 0; c0 < n_tax; c0 += piece) {
+        const int nc = (int)std::min<long long>(piece, n_tax - c0);
+        if (c0 > 0) MDG_CUDA_TRY(cudaMemsetAsync(d_counter, 0, sizeof(unsigned int), st));
+        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
+        MapBatchLaunch ml = {};
+        ml.k = d_k + (size_t)c0 * R; ml.N = d_N + (size_t)c0 * R; ml.n_tax = nc; ml.P = P; ml.n_runs = n_runs;
+        ml.pr = pr; ml.work_counter = d_counter; ml.rec = ctx->map_rec.as<mdg_map_run>();
+        if ((rc = launch_map_batch(ctx, st, ml, npl))) return rc;
+        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[2], st));
+        MapAssembleLaunch al = {};
+        al.tax_id = d_tax + c0; al.k = ml.k; al.N = ml.N;
+        al.mism12 = d_m12 ? d_m12 + (size_t)c0 * R * 12 : nullptr;
+        al.noise3 = d_noise ? d_noise + (size_t)c0 * 3 : nullptr;
+        al.n_tax = nc; al.P = P; al.n_runs = n_runs; al.rec = ml.rec; al.out = d_out + c0; al.eval_totals = d_evals;
+        map_assemble_kernel<<<(nc + 127) / 128, 128, 0, st>>>(al);
+        MDG_CUDA_TRY(cudaGetLastError());
+        ctx->timings.n_launches++;
+        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[3], st));
+        MDG_CUDA_TRY(cudaEventSynchronize(ctx->ev[3]));  // the events are reused by the next piece
+        ctx->timings.map_ms += elapsed(ctx->ev[1], ctx->ev[2]);
+        ctx->timings.assemble_ms += elapsed(ctx->ev[2], ctx->ev[3]);
+    }
+    if (n_tax > 0 && host) MDG_CUDA_TRY(cudaMemcpyAsync(out, d_out, nt * sizeof(mdg_map_result), cudaMemcpyDeviceToHost, st));
+    unsigned long long evals[MDG_NUM_RUNS];
+    MDG_CUDA_TRY(cudaMemcpyAsync(evals, d_evals, sizeof evals, cudaMemcpyDeviceToHost, st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[4], st));
+    MDG_CUDA_TRY(cudaEventSynchronize(ctx->ev[4]));
+    for (int r = 0; r < MDG_NUM_RUNS; ++r) ctx->timings.leapfrogs[r] = evals[r];
+    ctx->timings.total_ms = elapsed(ctx->ev[0], ctx->ev[4]);
+    return MDG_OK;
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -152,9 +152,17 @@ __device__ __forceinline__ bool chol_solve(const double (&H)[D][D], const double
     return true;
 }
 
-template <int MODEL, int NPL>
+// What the MAP-only path (mdg_map_batch_kernel.cuh) needs beyond MapRecord: the unconstrained mode and the number
+// of gradient evaluations. Only instantiations with TRACE = true fill it; map_kernel's (TRACE = false) compiles
+// to the same code as without it.
+struct MapTrace {
+    double u[4];
+    uint32_t n_eval;
+};
+
+template <int MODEL, int NPL, bool TRACE = false>
 __device__ void map_fit_group(const LaneObs<NPL>& ob, const double (&logC)[NPL], int P, const Priors& pr,
-                              const double2* ptab, bool has_spare, int lig, MapRecord& out) {
+                              const double2* ptab, bool has_spare, int lig, MapRecord& out, MapTrace* trace = nullptr) {
     constexpr int D = ModelDim<MODEL>::value;
     constexpr unsigned gmask = 0xffffffffu;
     constexpr double UMAX = 40.0;
@@ -193,6 +201,7 @@ __device__ void map_fit_group(const LaneObs<NPL>& ob, const double (&logC)[NPL],
     double f, g[D], ll[NPL], lp;
     bool ok;
     eval_model<MODEL, NPL, 32>(ob, u, ptab, pr.phi_min, has_spare, gmask, lig, lp, g, ll, ok);
+    if (TRACE) trace->n_eval = 1;
     // f carries log C(N,k) so that its magnitude (and the step-acceptance slack) matches the
     // constrained-space log posterior; `slack` covers the cancellation noise of the lgamma sums
     double sumC = 0.0, scale = 0.0;
@@ -226,6 +235,7 @@ __device__ void map_fit_group(const LaneObs<NPL>& ob, const double (&logC)[NPL],
             for (int i = 0; i < D; ++i) { up[i] = u[i] + (i == j ? h : 0.0); um[i] = u[i] - (i == j ? h : 0.0); }
             eval_model<MODEL, NPL, 32>(ob, up, ptab, pr.phi_min, has_spare, gmask, lig, t0, gp, ll, okp);
             eval_model<MODEL, NPL, 32>(ob, um, ptab, pr.phi_min, has_spare, gmask, lig, t1, gm, ll, okm);
+            if (TRACE) trace->n_eval += 2;
 #pragma unroll
             for (int i = 0; i < D; ++i) H[i][j] = (okp && okm) ? -(gp[i] - gm[i]) / (2.0 * h) : (i == j ? 1.0 : 0.0);
         }
@@ -252,6 +262,7 @@ __device__ void map_fit_group(const LaneObs<NPL>& ob, const double (&logC)[NPL],
             }
             bool okn;
             eval_model<MODEL, NPL, 32>(ob, un, ptab, pr.phi_min, has_spare, gmask, lig, lpn, gn, ll, okn);
+            if (TRACE) trace->n_eval += 1;
             if (okn && -(lpn + sumC) <= f + slack) {
                 double gmax = 0.0;
 #pragma unroll
@@ -275,6 +286,10 @@ __device__ void map_fit_group(const LaneObs<NPL>& ob, const double (&logC)[NPL],
     out.logp = -f;
     out.iters = (uint32_t)it;
     out.converged = converged ? 1u : 0u;
+    if (TRACE) {
+#pragma unroll
+        for (int j = 0; j < D; ++j) trace->u[j] = u[j];
+    }
 }
 
 #ifndef MDG_MAP_MINBLOCKS

@@ -252,6 +252,67 @@ __device__ inline double nan_std(const double* v, int n) {
     return sqrt(q / m);
 }
 
+// integer bookkeeping of fits.py:272-283 (z = 1 coverage, sums of N and k per strand) into any row type with these fields
+template <typename Row>
+__device__ __forceinline__ void tax_sums(const uint32_t* k, const uint32_t* N, int P, Row& r) {
+    const int R = 2 * P;
+    r.N_z1_forward = N[0];
+    r.N_z1_reverse = N[P];
+    for (int s = 0; s < R; ++s) {
+        if (s < P) { r.N_sum_forward += N[s]; r.y_sum_forward += k[s]; }
+        else { r.N_sum_reverse += N[s]; r.y_sum_reverse += k[s]; }
+    }
+    r.N_sum_total = r.N_sum_forward + r.N_sum_reverse;
+    r.y_sum_total = r.y_sum_forward + r.y_sum_reverse;
+}
+
+// normalized_noise, _forward, _reverse (fits.py:359-376) from the raw off-diagonal counts mism12 [n_tax][2P][12]
+// (CT is column 5 and GA column 6 of the 12), else copied from noise3 [n_tax][3]; fields are left alone (the caller's
+// NaN) if both are NULL
+template <typename Row>
+__device__ __forceinline__ void tax_noise(const uint32_t* mism12, const double* noise3, int tax, int P, Row& r) {
+    const int R = 2 * P;
+    const double qnan = nan("");
+    if (mism12 != nullptr) {
+        const uint32_t* m = mism12 + (size_t)tax * R * 12;
+        double col_mean[12];
+        for (int c = 0; c < 12; ++c) {
+            double s = 0.0; int cnt = 0;
+            for (int row = 0; row < R; ++row) {
+                const bool blank = (row < P && c == 5) || (row >= P && c == 6);
+                if (!blank) { s += (double)m[row * 12 + c]; ++cnt; }
+            }
+            col_mean[c] = cnt ? s / cnt : qnan;
+        }
+        double out3[3];
+        for (int part = 0; part < 3; ++part) {
+            const int r0 = part == 2 ? P : 0, r1 = part == 1 ? P : R;
+            double s = 0.0; int cnt = 0;
+            for (int row = r0; row < r1; ++row)
+                for (int c = 0; c < 12; ++c) {
+                    const bool blank = (row < P && c == 5) || (row >= P && c == 6);
+                    const double v = blank ? qnan : (double)m[row * 12 + c] / col_mean[c];
+                    if (!isnan(v)) { s += v; ++cnt; }
+                }
+            if (cnt == 0) { out3[part] = qnan; continue; }
+            const double mean = s / cnt;
+            double qq = 0.0;
+            for (int row = r0; row < r1; ++row)
+                for (int c = 0; c < 12; ++c) {
+                    const bool blank = (row < P && c == 5) || (row >= P && c == 6);
+                    const double v = blank ? qnan : (double)m[row * 12 + c] / col_mean[c];
+                    if (!isnan(v)) { double d = v - mean; qq += d * d; }
+                }
+            out3[part] = sqrt(qq / cnt);
+        }
+        r.normalized_noise = out3[0]; r.normalized_noise_forward = out3[1]; r.normalized_noise_reverse = out3[2];
+    } else if (noise3 != nullptr) {
+        r.normalized_noise = noise3[(size_t)tax * 3];
+        r.normalized_noise_forward = noise3[(size_t)tax * 3 + 1];
+        r.normalized_noise_reverse = noise3[(size_t)tax * 3 + 2];
+    }
+}
+
 __global__ void assemble_kernel(const AssembleLaunch p) {
     const int tax = blockIdx.x * blockDim.x + threadIdx.x;
     if (tax >= p.n_tax) return;
@@ -265,14 +326,7 @@ __global__ void assemble_kernel(const AssembleLaunch p) {
     memset(&r, 0, sizeof r);
     const double qnan = nan("");
     r.tax_id = p.tax_id[tax];
-    r.N_z1_forward = N[0];
-    r.N_z1_reverse = N[P];
-    for (int s = 0; s < R; ++s) {
-        if (s < P) { r.N_sum_forward += N[s]; r.y_sum_forward += k[s]; }
-        else { r.N_sum_reverse += N[s]; r.y_sum_reverse += k[s]; }
-    }
-    r.N_sum_total = r.N_sum_forward + r.N_sum_reverse;
-    r.y_sum_total = r.y_sum_forward + r.y_sum_reverse;
+    tax_sums(k, N, P, r);
     r.n_sigma_forward = r.D_max_forward = r.q_mean_forward = qnan;
     r.n_sigma_reverse = r.D_max_reverse = r.q_mean_reverse = r.asymmetry = qnan;
     r.normalized_noise = r.normalized_noise_forward = r.normalized_noise_reverse = qnan;
@@ -340,45 +394,7 @@ __global__ void assemble_kernel(const AssembleLaunch p) {
         if (p.out_lo) p.out_lo[(size_t)tax * R + s] = ok ? (float)pred[(size_t)s * 3 + 1] : nanf("");
         if (p.out_hi) p.out_hi[(size_t)tax * R + s] = ok ? (float)pred[(size_t)s * 3 + 2] : nanf("");
     }
-    // noise, fits.py:359-376 (CT is column 5 and GA column 6 of the 12 off-diagonal columns)
-    if (p.mism12 != nullptr) {
-        const uint32_t* m = p.mism12 + (size_t)tax * R * 12;
-        double col_mean[12];
-        for (int c = 0; c < 12; ++c) {
-            double s = 0.0; int cnt = 0;
-            for (int row = 0; row < R; ++row) {
-                const bool blank = (row < P && c == 5) || (row >= P && c == 6);
-                if (!blank) { s += (double)m[row * 12 + c]; ++cnt; }
-            }
-            col_mean[c] = cnt ? s / cnt : qnan;
-        }
-        double out3[3];
-        for (int part = 0; part < 3; ++part) {
-            const int r0 = part == 2 ? P : 0, r1 = part == 1 ? P : R;
-            double s = 0.0; int cnt = 0;
-            for (int row = r0; row < r1; ++row)
-                for (int c = 0; c < 12; ++c) {
-                    const bool blank = (row < P && c == 5) || (row >= P && c == 6);
-                    const double v = blank ? qnan : (double)m[row * 12 + c] / col_mean[c];
-                    if (!isnan(v)) { s += v; ++cnt; }
-                }
-            if (cnt == 0) { out3[part] = qnan; continue; }
-            const double mean = s / cnt;
-            double qq = 0.0;
-            for (int row = r0; row < r1; ++row)
-                for (int c = 0; c < 12; ++c) {
-                    const bool blank = (row < P && c == 5) || (row >= P && c == 6);
-                    const double v = blank ? qnan : (double)m[row * 12 + c] / col_mean[c];
-                    if (!isnan(v)) { double d = v - mean; qq += d * d; }
-                }
-            out3[part] = sqrt(qq / cnt);
-        }
-        r.normalized_noise = out3[0]; r.normalized_noise_forward = out3[1]; r.normalized_noise_reverse = out3[2];
-    } else if (p.noise3 != nullptr) {
-        r.normalized_noise = p.noise3[(size_t)tax * 3];
-        r.normalized_noise_forward = p.noise3[(size_t)tax * 3 + 1];
-        r.normalized_noise_reverse = p.noise3[(size_t)tax * 3 + 2];
-    }
+    tax_noise(p.mism12, p.noise3, tax, P, r);
     r.status = status;
     p.out[tax] = r;
 }

@@ -7,6 +7,10 @@ dtypes; fits.py:242-293, 632-680), same parquet cache rules, same --max-fits sel
 multiprocessing fan-out (fits.py:569-626) are replaced by `mdg_fit_batch` on each GPU's
 contiguous share of the TaxID batch. The MAP fit (new) is written to fit_map/<shortname>.parquet
 so that the two reference schemas stay unchanged.
+
+`get_map_fits` / `compute_map_fits` are the MAP-only screening mode (`metadamage fit --map-only`): six MAP
+fits per TaxID with Laplace uncertainties and a likelihood-ratio statistic through `mdg_map_batch`, no NUTS,
+one table in map_results/<shortname>.parquet.
 """
 import logging
 
@@ -14,7 +18,7 @@ import numpy as np
 import pandas as pd
 
 from . import _lib, io, utils
-from ._abi import FIT_FAILED
+from ._abi import FIT_COV_INVALID, FIT_FAILED, FIT_MAP_NOT_CONVERGED, MAP_RESULT_DTYPE
 from .backend import Context
 from .counts import dense_from_df_counts
 from .parallel import run_on_gpus
@@ -31,6 +35,25 @@ FIT_RESULT_COLUMNS = [
 ]
 FIT_MAP_COLUMNS = ["map_A", "map_q", "map_c", "map_phi", "map_D_max", "map_logp", "map_null_q", "map_null_phi",
                    "map_null_logp"]
+
+# the MAP-only table (map_results/<shortname>.parquet). D_max is A + c at the PMD mode, not the posterior predictive
+# median of fit_results; lambda_LR_P / lambda_LR_z are a screening scale (the null model sits on the boundary A = 0 of
+# the PMD model), not calibrated p-values.
+MAP_RESULT_COLUMNS = [
+    "tax_id", "tax_name", "tax_rank", "N_alignments", "N_z1_forward", "N_z1_reverse", "N_sum_forward", "N_sum_reverse",
+    "N_sum_total", "y_sum_forward", "y_sum_reverse", "y_sum_total",
+    "D_max", "D_max_std", "significance", "q", "q_std", "A", "A_std", "c", "c_std", "phi", "phi_std", "rho_Ac", "logp",
+    "loglik",
+    "null_q", "null_q_std", "null_phi", "null_phi_std", "null_logp", "null_loglik",
+    "lambda_LR", "lambda_LR_P", "lambda_LR_z",
+    "forward_D_max", "forward_D_max_std", "forward_lambda_LR", "reverse_D_max", "reverse_D_max_std", "reverse_lambda_LR",
+    "normalized_noise", "normalized_noise_forward", "normalized_noise_reverse", "valid", "shortname",
+]
+# columns taken from one run's record: column -> (run kind, mdg_map_run field)
+_MAP_RUN_COLUMNS = {
+    **{name: (0, name) for name in ("q", "q_std", "A", "A_std", "c", "c_std", "phi", "phi_std", "logp", "loglik")},
+    **{"null_" + name: (1, name) for name in ("q", "q_std", "phi", "phi_std", "logp", "loglik")},
+}
 
 _contexts = {}
 
@@ -85,6 +108,23 @@ def fit_dense(dense, cfg, fit_cfg, n_gpus=1):
 
     parts = [p for p in run_on_gpus(n_tax, n_dev, worker) if p is not None]
     return {key: np.concatenate([p[key] for p in parts]) for key in ("result", "median", "hpdi_lo", "hpdi_hi")}
+
+
+def map_dense(dense, cfg, fit_cfg, n_gpus=1):
+    """Run mdg_map_batch over `n_gpus` contiguous shares of the dense batch (as fit_dense); host-side concat."""
+    n_tax = len(dense["tax_id"])
+    if n_tax == 0:
+        return np.zeros(0, MAP_RESULT_DTYPE)
+    n_dev = max(1, min(int(n_gpus), _lib.load().mdg_device_count() or 1))
+
+    def worker(rank, start, stop):
+        sl = slice(start, stop)
+        return _context(rank).map_batch(dense["tax_id"][sl], dense["k"][sl], dense["N"][sl], fit_cfg,
+                                        mism12=dense["mism12"][sl] if dense.get("mism12") is not None else None,
+                                        noise3=dense["noise"][sl] if dense.get("noise") is not None else None)
+
+    parts = [p for p in run_on_gpus(n_tax, n_dev, worker) if p is not None]
+    return np.concatenate(parts)
 
 
 def select_top_dense(df_counts, dense, n_fits, ctx=None):
@@ -175,6 +215,46 @@ def make_df_fit_map(res, dense, ok, cfg):
     return pd.DataFrame(data, copy=False)
 
 
+def make_df_map_results(res, dense, cfg):
+    """The MAP-only table: one row per TaxID in df_counts order, columns MAP_RESULT_COLUMNS in their final dtypes
+    (as make_df_fit_results). TaxIDs whose all-position PMD or null fit had no finite starting point are dropped with
+    the same warning. `valid`: both all-position fits converged and have a Laplace covariance."""
+    ok = (res["status"] & FIT_FAILED) == 0
+    for tax in dense["tax_id"][~ok]:
+        logger.warning("Fit: no valid fit for tax_id %s. Skipping for now", tax)
+    n = int(ok.sum())
+    r = res[ok]
+    data = {}
+    for col in MAP_RESULT_COLUMNS:
+        if col in ("tax_id", "tax_name", "tax_rank"):
+            vals = dense[col][ok]
+            if col == "tax_id" and n:
+                uniq, codes = _category_of(vals)
+                data[col] = pd.Categorical.from_codes(codes, categories=uniq)
+            else:
+                data[col] = pd.Categorical(np.asarray(vals, dtype=np.int64 if col == "tax_id" else object))
+        elif col == "N_alignments":
+            data[col] = _final_dtype(dense[col][ok], col)
+        elif col in _MAP_RUN_COLUMNS:
+            run, field = _MAP_RUN_COLUMNS[col]
+            data[col] = _final_dtype(r["run"][:, run][field], col)
+        elif col == "valid":
+            data[col] = (r["status"] & (FIT_MAP_NOT_CONVERGED | FIT_COV_INVALID)) == 0
+        elif col == "shortname":
+            data[col] = pd.Categorical.from_codes(np.zeros(n, np.int8), categories=[cfg.shortname])
+        else:
+            data[col] = _final_dtype(r[col], col)
+    return pd.DataFrame(data, copy=False)
+
+
+def compute_map_fits(df_counts, cfg, n_fits=None):
+    """MAP-only screening of every TaxID of df_counts (or of the top `n_fits`, as compute_fits): the table of
+    make_df_map_results."""
+    dense = select_top_dense(df_counts, dense_from_df_counts(df_counts, cfg), n_fits)
+    res = map_dense(dense, cfg, fit_config_from(cfg), n_gpus=getattr(cfg, "gpus", 1))
+    return make_df_map_results(res, dense, cfg)
+
+
 def compute_fits(df_counts, cfg, mcmc_kwargs=None, return_map=False, n_fits=None):
     """The GPU replacement of fits.compute_fits (fits.py:709-730). `n_fits`: fit only the top TaxIDs of
     fits.py:736-744 (what get_fits does by filtering the frame first), selected on the device."""
@@ -210,3 +290,16 @@ def get_fits(df_counts, cfg):
     pq_predictions.save(df_fit_predictions, metadata=meta)
     io.Parquet(cfg.filename_fit_map).save(df_fit_map, metadata=meta)
     return df_fit_results, df_fit_predictions
+
+
+def get_map_fits(df_counts, cfg):
+    """`metadamage fit --map-only`: the cache rules of get_fits on map_results/<shortname>.parquet."""
+    pq = io.Parquet(cfg.filename_map_results)
+    if pq.exists(cfg.forced):
+        if utils.metadata_is_similar(pq.load_metadata(), cfg.to_dict(), include=CACHE_KEYS):
+            logger.info("Fit: Loading MAP fits from parquet-file.")
+            return pq.load()
+    logger.info("Fit: Generating MAP fits and saving to file.")
+    df_map_results = compute_map_fits(df_counts, cfg, n_fits=cfg.N_fits)
+    pq.save(df_map_results, metadata=cfg.to_dict())
+    return df_map_results

@@ -161,6 +161,20 @@ def dense_fit_batch(n_fit, max_position=15, seed=SEEDS["cfg2"], **kw):
     return g["tax_ids"][sel], np.ascontiguousarray(g["k"][sel]), np.ascontiguousarray(g["N"][sel]), g
 
 
+def dense_fit_batch_shares(n_fit, parts, max_position=15, seed=SEEDS["cfg3"]):
+    """Dense (tax_id, k, N) of `n_fit` passing TaxIDs generated as `parts` independent shares (share r = jumped block r,
+    tax ids from 1 + r * 10^8), the way bench.py's multi-GPU workload cuts config 3; no share is held twice in memory."""
+    tid, k, N = [], [], []
+    for r in range(parts):
+        g = make_mismatch_matrix(0, max_position=max_position, seed=seed, n_fit=n_fit // parts + (r < n_fit % parts), jump=r,
+                                 tax_id_start=1 + r * 100_000_000)
+        sel = g["passes"]
+        tid.append(g["tax_ids"][sel])
+        k.append(g["k"][sel])
+        N.append(g["N"][sel])
+    return np.concatenate(tid), np.ascontiguousarray(np.vstack(k)), np.ascontiguousarray(np.vstack(N))
+
+
 def mism12_from_counts16(counts16, first_rows, max_position):
     """[n_tax][2P][12] off-diagonal raw counts (AC..TG) of complete 2P-row TaxIDs, for the noise estimate."""
     R = 2 * int(max_position)

@@ -105,6 +105,10 @@ class Config:
     def filename_fit_map(self):
         return self._out("fit_map")
 
+    @property
+    def filename_map_results(self):
+        return self._out("map_results")
+
     def set_number_of_fits(self, df_counts):
         self.N_tax_ids = len(pd.unique(df_counts.tax_id))
         if self.max_fits is not None and self.max_fits > 0:
