@@ -13,8 +13,8 @@ HEADERS = [os.path.join(_ROOT, "include", "mdg.h")] + sorted(glob.glob(os.path.j
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",
-    # no implicit mul+add contraction: every kernel variant (warp / half-warp groups, 1-4 positions
-    # per lane) must give bit-identical results; fused operations are written as fma() explicitly
+    # no implicit mul+add contraction: every kernel variant (MAP's 1, 2 or 4 positions per lane)
+    # must give bit-identical results; fused operations are written as fma() explicitly
     "-fmad=false",
     "-Xcompiler", "-fPIC", "-shared", "-cudart", "static",
 ]

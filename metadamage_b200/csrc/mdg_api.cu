@@ -52,7 +52,6 @@ struct DevBuf {
     template <typename T> T* as() const { return reinterpret_cast<T*>(ptr); }
 };
 
-constexpr int kNumBufs = 24;
 constexpr int kNumEvents = 16;
 
 }  // namespace mdg
@@ -61,10 +60,10 @@ constexpr int kNumEvents = 16;
 // same batch or of the next submitted batch) starts under the tail of chunk c, which is a handful of long
 // sequential chains on an otherwise idle GPU.
 struct mdg_fit_lane {
-    cudaStream_t main = nullptr, side[4] = {nullptr, nullptr, nullptr, nullptr};  // main: high priority; side: the four NUTS launches
+    cudaStream_t main = nullptr, side[2] = {nullptr, nullptr};  // main: high priority; side[m]: the NUTS launch of model m (0 PMD, 1 null)
     cudaEvent_t ev[5] = {};  // chunk begin, MAP end, NUTS end, predictive end, done (after assembly + D2H)
-    cudaEvent_t fork_ev = nullptr, join_ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    mdg::DevBuf rec, map, pred, counters, samples, waic, waic_acc[4];
+    cudaEvent_t fork_ev = nullptr, join_ev[2] = {nullptr, nullptr};  // join_ev[m]: end of side[m]'s NUTS launch
+    mdg::DevBuf rec, map, pred, counters, samples, waic, waic_acc[2];
     mdg::DevBuf chain_clock;  // development switch MDG_CHAIN_CLOCK=<file>
     mdg::DevBuf order;        // queue order of the chunk's TaxIDs: [chunk] int order, [chunk] bucket bytes, 3 x kOrderBuckets counters
     int clock_items = 0;
@@ -96,7 +95,16 @@ struct mdg_ctx {
     cudaEvent_t ev[mdg::kNumEvents] = {};
     cudaEvent_t epoch = nullptr;       // time zero of mdg_timings.nuts_begin_ms / nuts_end_ms
     cudaEvent_t inputs_ready = nullptr;
-    mdg::DevBuf buf[mdg::kNumBufs];
+    // scratch of the synchronous entry points, each named after the entry points that use it (they share a buffer
+    // only where the calls never overlap: each synchronises before it returns)
+    mdg::DevBuf reduce_in;              // mdg_counts_reduce: staged input columns (MDG_HOST)
+    mdg::DevBuf reduce_tsv_out;         // mdg_counts_reduce, mdg_tsv_parse: staged output columns (MDG_HOST)
+    mdg::DevBuf reduce_tsv_scalars;     // mdg_counts_reduce, mdg_tsv_parse: 64 B of device counters and error flags
+    mdg::DevBuf reduce_tiles;           // mdg_counts_reduce: per-tile block bookkeeping and scan chunk totals
+    mdg::DevBuf reduce_tmp;             // mdg_counts_reduce: per-TaxID rows before the permute puts them in order
+    mdg::DevBuf order_tsv_top_in;       // mdg_counts_order, mdg_select_top: staged inputs (MDG_HOST); mdg_tsv_parse: the text
+    mdg::DevBuf order_tsv_top_scratch;  // mdg_counts_order, mdg_tsv_parse, mdg_select_top: per-block counts, scans, histograms
+    mdg::DevBuf test_scratch;           // mdg_test_*, mdg_measure_fp64_peak
     mdg::DevBuf da_tables;             // sqrt(t) and t^-0.75 for t < kDaTable (dual averaging), filled at the first fit
     mdg_fit_lane lane[kFitLanes];
     mdg_fit_ticket_slot ticket[kFitTickets];
@@ -165,15 +173,12 @@ int persistent_grid(K kernel, int threads, size_t smem, int num_sms, long long i
     int per_sm = 1;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
     if (per_sm < 1) per_sm = 1;
-    if (const char* cap_env = getenv("MDG_MAX_CTAS_PER_SM")) {  // occupancy experiments
-        int c = atoi(cap_env);
-        if (c >= 1 && c < per_sm) per_sm = c;
-    }
     long long want = (items + items_per_block - 1) / items_per_block;
     long long cap = (long long)per_sm * num_sms;
     return (int)std::max<long long>(1, std::min(want, cap));
 }
 
+constexpr int kNutsGroupLanes = 8;  // lanes per chain
 constexpr int kNutsWarps = 4;
 constexpr int kOrderMinChunk = 32768;  // TaxIDs per chunk from which the NUTS queue is ordered by coverage
 constexpr int kMapWarps = 4;
@@ -185,8 +190,9 @@ int env_int(const char* name, int dflt) {
 }
 
 // K4, group layout: GW lanes per chain, rolled position loop (mdg_nuts_kernel.cuh)
-template <int MODEL, int GW, int WARPS>
+template <int MODEL>
 int launch_nuts_group(mdg_ctx* ctx, cudaStream_t st, FitLaunch fl, DevBuf& acc) {
+    constexpr int GW = kNutsGroupLanes, WARPS = kNutsWarps;
     auto kern = nuts_group_kernel<MODEL, GW, WARPS>;
     const int n_obs = fl.n_items_all > 0 ? 2 * fl.P : fl.P;  // the launch's longest run
     fl.n_slots = (n_obs + 1 + GW - 1) / GW;  // index 0 is the spare
@@ -195,7 +201,7 @@ int launch_nuts_group(mdg_ctx* ctx, cudaStream_t st, FitLaunch fl, DevBuf& acc) 
     // contiguously, so a retiring CTA's hole must fit the next launch's CTA: every launch asks for the same footprint
     // (static + dynamic), the largest one (PMD with all-position runs). Otherwise the SMs end up with three resident
     // CTAs instead of four (profiles/r02_chain_timeline.md: 8 016 live chains instead of 9 472).
-    if (env_int("MDG_NUTS_UNIFORM_SMEM", 1)) {
+    {
         cudaFuncAttributes mine, big;
         MDG_CUDA_TRY(cudaFuncGetAttributes(&mine, kern));
         MDG_CUDA_TRY(cudaFuncGetAttributes(&big, nuts_group_kernel<0, GW, WARPS>));
@@ -206,8 +212,7 @@ int launch_nuts_group(mdg_ctx* ctx, cudaStream_t st, FitLaunch fl, DevBuf& acc) 
     // One group slot per item up to the whole GPU. (Smaller grids that leave every group several items were measured:
     // 3 / 6 / 12 items per group cost 14 / 21 / 39 % at 10 000 TaxIDs per batch and 0 / 9 / 35 % at 40 000 — fewer
     // resident chains, and different kernels sharing an SM's instruction cache; profiles/r02_nuts_tuning.md.)
-    const int per_group = std::max(1, env_int("MDG_ITEMS_PER_GROUP", 1));
-    const int grid = persistent_grid(kern, WARPS * 32, smem, ctx->num_sms, fl.n_items, WARPS * (32 / GW) * per_group);
+    const int grid = persistent_grid(kern, WARPS * 32, smem, ctx->num_sms, fl.n_items, WARPS * (32 / GW));
     int rc = acc.ensure((size_t)grid * WARPS * 4 * fl.n_slots * 32 * sizeof(double));
     if (rc) return rc;
     fl.waic_acc = acc.as<double>();
@@ -215,13 +220,6 @@ int launch_nuts_group(mdg_ctx* ctx, cudaStream_t st, FitLaunch fl, DevBuf& acc) 
     MDG_CUDA_TRY(cudaGetLastError());
     ctx->timings.n_launches++;
     return MDG_OK;
-}
-
-template <int MODEL>
-int launch_nuts_group_dispatch(mdg_ctx* ctx, cudaStream_t st, const FitLaunch& fl, DevBuf& acc, int gw) {
-    if (gw == 16) return launch_nuts_group<MODEL, 16, kNutsWarps>(ctx, st, fl, acc);
-    if (env_int("MDG_NUTS_WARPS", kNutsWarps) == 2) return launch_nuts_group<MODEL, 8, 2>(ctx, st, fl, acc);  // A/B: CTAs of two warps
-    return launch_nuts_group<MODEL, 8, kNutsWarps>(ctx, st, fl, acc);
 }
 
 int launch_map(mdg_ctx* ctx, cudaStream_t st, const MapLaunch& ml, int npl) {
@@ -352,13 +350,13 @@ int mdg_ctx_create(int device, mdg_ctx** out) {
     if ((e = cudaDeviceGetStreamPriorityRange(&prio_low, &prio_high)) != cudaSuccess) return fail(e, "cudaDeviceGetStreamPriorityRange");
     for (auto& ln : ctx->lane) {
         if ((e = cudaStreamCreateWithPriority(&ln.main, cudaStreamNonBlocking, prio_high)) != cudaSuccess) return fail(e, "cudaStreamCreate");
-        for (int i = 0; i < 4; ++i)
-            if ((e = cudaStreamCreateWithPriority(&ln.side[i], cudaStreamNonBlocking, prio_low)) != cudaSuccess) return fail(e, "cudaStreamCreate");
+        for (auto& sd : ln.side)
+            if ((e = cudaStreamCreateWithPriority(&sd, cudaStreamNonBlocking, prio_low)) != cudaSuccess) return fail(e, "cudaStreamCreate");
         for (int i = 0; i < 5; ++i)
             if ((e = cudaEventCreate(&ln.ev[i])) != cudaSuccess) return fail(e, "cudaEventCreate");
         if ((e = cudaEventCreateWithFlags(&ln.fork_ev, cudaEventDisableTiming)) != cudaSuccess) return fail(e, "cudaEventCreate");
-        for (int i = 0; i < 4; ++i)
-            if ((e = cudaEventCreateWithFlags(&ln.join_ev[i], cudaEventDisableTiming)) != cudaSuccess) return fail(e, "cudaEventCreate");
+        for (auto& je : ln.join_ev)
+            if ((e = cudaEventCreateWithFlags(&je, cudaEventDisableTiming)) != cudaSuccess) return fail(e, "cudaEventCreate");
         if ((e = cudaHostAlloc((void**)&ln.h_leap, MDG_NUM_RUNS * sizeof(unsigned long long), cudaHostAllocDefault)) != cudaSuccess)
             return fail(e, "cudaHostAlloc");
     }
@@ -375,23 +373,24 @@ void mdg_ctx_destroy(mdg_ctx* ctx) {
     DeviceGuard guard(ctx->device);
     for (auto& ln : ctx->lane) {
         if (ln.main) cudaStreamSynchronize(ln.main);
-        for (int i = 0; i < 4; ++i) if (ln.side[i]) cudaStreamSynchronize(ln.side[i]);
+        for (cudaStream_t sd : ln.side) if (sd) cudaStreamSynchronize(sd);
     }
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    for (auto& b : ctx->buf) b.release();
-    ctx->da_tables.release();
+    for (mdg::DevBuf* b : {&ctx->reduce_in, &ctx->reduce_tsv_out, &ctx->reduce_tsv_scalars, &ctx->reduce_tiles, &ctx->reduce_tmp,
+                           &ctx->order_tsv_top_in, &ctx->order_tsv_top_scratch, &ctx->test_scratch, &ctx->da_tables})
+        b->release();
     for (int i = 0; i < kNumEvents; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     if (ctx->epoch) cudaEventDestroy(ctx->epoch);
     if (ctx->inputs_ready) cudaEventDestroy(ctx->inputs_ready);
     for (auto& ln : ctx->lane) {
         for (mdg::DevBuf* b : {&ln.rec, &ln.map, &ln.pred, &ln.counters, &ln.samples, &ln.waic, &ln.waic_acc[0], &ln.waic_acc[1],
-                               &ln.waic_acc[2], &ln.waic_acc[3], &ln.chain_clock, &ln.order})
+                               &ln.chain_clock, &ln.order})
             b->release();
         for (int i = 0; i < 5; ++i) if (ln.ev[i]) cudaEventDestroy(ln.ev[i]);
         if (ln.fork_ev) cudaEventDestroy(ln.fork_ev);
-        for (int i = 0; i < 4; ++i) {
-            if (ln.join_ev[i]) cudaEventDestroy(ln.join_ev[i]);
-            if (ln.side[i]) cudaStreamDestroy(ln.side[i]);
+        for (int m = 0; m < 2; ++m) {
+            if (ln.join_ev[m]) cudaEventDestroy(ln.join_ev[m]);
+            if (ln.side[m]) cudaStreamDestroy(ln.side[m]);
         }
         if (ln.main) cudaStreamDestroy(ln.main);
         if (ln.h_leap) cudaFreeHost(ln.h_leap);
@@ -466,9 +465,9 @@ int mdg_counts_reduce(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_
     if (host) {
         // one arena for inputs, one for outputs
         size_t in_bytes = n * (8 + 4 + 1 + 1) + 256 * 5 + 16 * ((n * 4 + 255) & ~(size_t)255);
-        int rc = ctx->buf[0].ensure(in_bytes);
+        int rc = ctx->reduce_in.ensure(in_bytes);
         if (rc) return rc;
-        unsigned char* base = ctx->buf[0].as<unsigned char>();
+        unsigned char* base = ctx->reduce_in.as<unsigned char>();
         size_t off = 0;
         auto put = [&](const void* src, size_t bytes) -> void* {
             void* d = base + off;
@@ -489,9 +488,9 @@ int mdg_counts_reduce(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_
         MDG_CUDA_TRY(cudaGetLastError());
         const size_t ncap = (size_t)out_capacity;
         size_t out_bytes = n * (4 + 4 + 4 + 4 + 1 + 8 + 1) + ncap * (8 + 4 + 8) + ncap * (size_t)R * 8 + ncap * 24 + 256 * 16;
-        rc = ctx->buf[1].ensure(out_bytes);
+        rc = ctx->reduce_tsv_out.ensure(out_bytes);
         if (rc) return rc;
-        unsigned char* ob = ctx->buf[1].as<unsigned char>();
+        unsigned char* ob = ctx->reduce_tsv_out.as<unsigned char>();
         size_t oo = 0;
         auto take = [&](void* host_ptr, size_t elem, size_t count, bool per_tax) -> void* {
             if (!host_ptr) return nullptr;
@@ -524,159 +523,77 @@ int mdg_counts_reduce(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_
     cl.n_rows = n_rows;
     cl.fwd_ref = fwd_ref; cl.fwd_obs = fwd_obs; cl.rev_ref = rev_ref; cl.rev_obs = rev_obs;
     cl.P = P; cl.min_align = min_alignments; cl.min_y = min_y_sum;
-    // staged columns: the reference-base rows of the two substitutions (+ all off-diagonals for noise)
-    bool need[16] = {};
-    for (int o = 0; o < 4; ++o) { need[fwd_ref * 4 + o] = true; need[rev_ref * 4 + o] = true; }
-    if (cl.out_noise) for (int r = 0; r < 4; ++r) for (int o = 0; o < 4; ++o) if (r != o) need[r * 4 + o] = true;
-    cl.ncols = 0;
-    for (int c = 0; c < 16; ++c) {
-        cl.col_slot[c] = -1;
-        if (need[c]) { cl.col_slot[c] = cl.ncols; cl.col_id[cl.ncols++] = c; }
-    }
     auto aligned16 = [](const void* p) { return ((uintptr_t)p & 15u) == 0; };
-    cl.use_tma = aligned16(cl.tax_id) && aligned16(cl.n_align) && aligned16(cl.is_rev) && aligned16(cl.pos0) &&
-                 aligned16(cl.counts16) && (cl.stride % 4 == 0);
+    cl.vec_in = aligned16(cl.tax_id) && aligned16(cl.n_align) && aligned16(cl.is_rev) && aligned16(cl.pos0) &&
+                aligned16(cl.counts16) && (cl.stride % 4 == 0);
 
     // output bases 16-byte aligned -> 128-bit stores
     cl.vec_out = aligned16(cl.n_fwd_row) && aligned16(cl.n_rev_row) && aligned16(cl.f_fwd_row) && aligned16(cl.f_rev_row) &&
                  aligned16(cl.z_row) && aligned16(cl.y_row) && aligned16(cl.keep_row);
-    int rc = ctx->buf[2].ensure(64);
+    int rc = ctx->reduce_tsv_scalars.ensure(64);
     if (rc) return rc;
-    long long* d_ntax = ctx->buf[2].as<long long>();
+    long long* d_ntax = ctx->reduce_tsv_scalars.as<long long>();  // [0] kept TaxIDs, [1] error flag (int), [2] dense rows reserved
     int* d_err = reinterpret_cast<int*>(d_ntax + 1);
-    unsigned int* d_ticket = reinterpret_cast<unsigned int*>(d_ntax + 2);
     int h_err = 0;
     long long h_ntax = 0;
-    const bool stream_design = getenv("MDG_COUNTS_TILES") == nullptr;  // the round-1 tile kernel stays selectable for A/B runs
-    if (stream_design) {
-        // ---- warp-synchronous streaming kernel (mdg_counts_stream.cuh): one warp per 128 rows ----
-        const long long n_tiles = (n_rows + kStreamRows - 1) / kStreamRows;
-        const size_t ncap_t = (size_t)out_capacity;
-        const long long n_chunks_cap = (n_tiles + kScanChunk - 1) / kScanChunk;
-        rc = ctx->buf[3].ensure((size_t)n_tiles * (8 + 8 + 4) + (size_t)n_chunks_cap * 8 + 64);
-        if (rc) return rc;
-        long long* d_tile_base = ctx->buf[3].as<long long>();
-        long long* d_final_base = d_tile_base + n_tiles;
-        long long* d_chunk = d_final_base + n_tiles;
-        int* d_tile_cnt = reinterpret_cast<int*>(d_chunk + n_chunks_cap);
-        const size_t tmp_bytes = ncap_t * (8 + 4 + 8 + 8 + (size_t)R * 8) + 256 * 8;
-        rc = ctx->buf[21].ensure(tmp_bytes);
-        if (rc) return rc;
-        unsigned char* tb = ctx->buf[21].as<unsigned char>();
-        size_t to = 0;
-        auto tmp = [&](size_t bytes) { void* q = tb + to; to += (bytes + 255) & ~(size_t)255; return q; };
-        // the noise kernel needs the first rows in final order even if the caller does not want them
-        long long* d_first_final = cl.out_first ? cl.out_first : (cl.out_noise ? (long long*)tmp(ncap_t * 8) : nullptr);
-        CountsPermute cp = {};
-        cp.n_tiles = n_tiles; cp.tile_base = d_tile_base; cp.final_base = d_final_base; cp.tile_cnt = d_tile_cnt; cp.R = R;
-        cp.chunk_off = d_chunk;
-        cp.out_tax = cl.out_tax; cp.out_nal = cl.out_nal; cp.out_first = d_first_final; cp.out_k = cl.out_k; cp.out_N = cl.out_N;
-        cp.out_noise = nullptr;
-        CountsLaunch kl = cl;  // the tile kernel writes the per-TaxID rows into the temporaries
-        kl.out_noise = nullptr;
-        kl.out_first = nullptr;
-        if (cl.out_tax) { cp.t_tax = (long long*)tmp(ncap_t * 8); kl.out_tax = (long long*)cp.t_tax; }
-        if (cl.out_nal) { cp.t_nal = (uint32_t*)tmp(ncap_t * 4); kl.out_nal = (uint32_t*)cp.t_nal; }
-        if (d_first_final) { cp.t_first = (long long*)tmp(ncap_t * 8); kl.out_first = (long long*)cp.t_first; }
-        if (cl.out_k) { cp.t_k = (uint32_t*)tmp(ncap_t * R * 4); kl.out_k = (uint32_t*)cp.t_k; }
-        if (cl.out_N) { cp.t_N = (uint32_t*)tmp(ncap_t * R * 4); kl.out_N = (uint32_t*)cp.t_N; }
-        kl.tile_ticket = d_ticket;
-        kl.kept_counter = reinterpret_cast<unsigned long long*>(d_ntax + 3);
-        kl.tile_base = d_tile_base;
-        kl.tile_cnt = d_tile_cnt;
-        kl.capacity = out_capacity;
-        kl.error_flag = d_err;
-        MDG_CUDA_TRY(cudaMemsetAsync(d_ntax, 0, 64, st));
-        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
-        counts_stream_kernel<<<(unsigned)((n_tiles + kStreamWarps - 1) / kStreamWarps), kStreamWarps * 32, 0, st>>>(kl);
-        MDG_CUDA_TRY(cudaGetLastError());
-        const long long n_chunks = (n_tiles + kScanChunk - 1) / kScanChunk;
-        counts_scan_local_kernel<<<(unsigned)n_chunks, kScanChunk, 0, st>>>(d_tile_cnt, n_tiles, d_final_base, d_chunk);
-        counts_scan_chunks_kernel<<<1, 32, 0, st>>>(d_chunk, n_chunks, d_ntax);
+    // ---- warp-synchronous streaming kernel (mdg_counts_stream.cuh): one warp per 128 rows ----
+    const long long n_tiles = (n_rows + kStreamRows - 1) / kStreamRows;
+    const size_t ncap_t = (size_t)out_capacity;
+    const long long n_chunks = (n_tiles + kScanChunk - 1) / kScanChunk;
+    rc = ctx->reduce_tiles.ensure((size_t)n_tiles * (8 + 8 + 4) + (size_t)n_chunks * 8 + 64);
+    if (rc) return rc;
+    long long* d_tile_base = ctx->reduce_tiles.as<long long>();
+    long long* d_final_base = d_tile_base + n_tiles;
+    long long* d_chunk = d_final_base + n_tiles;
+    int* d_tile_cnt = reinterpret_cast<int*>(d_chunk + n_chunks);
+    const size_t tmp_bytes = ncap_t * (8 + 4 + 8 + 8 + (size_t)R * 8) + 256 * 8;
+    rc = ctx->reduce_tmp.ensure(tmp_bytes);
+    if (rc) return rc;
+    unsigned char* tb = ctx->reduce_tmp.as<unsigned char>();
+    size_t to = 0;
+    auto tmp = [&](size_t bytes) { void* q = tb + to; to += (bytes + 255) & ~(size_t)255; return q; };
+    // the noise kernel needs the first rows in final order even if the caller does not want them
+    long long* d_first_final = cl.out_first ? cl.out_first : (cl.out_noise ? (long long*)tmp(ncap_t * 8) : nullptr);
+    CountsPermute cp = {};
+    cp.n_tiles = n_tiles; cp.tile_base = d_tile_base; cp.final_base = d_final_base; cp.tile_cnt = d_tile_cnt; cp.R = R;
+    cp.chunk_off = d_chunk;
+    cp.out_tax = cl.out_tax; cp.out_nal = cl.out_nal; cp.out_first = d_first_final; cp.out_k = cl.out_k; cp.out_N = cl.out_N;
+    CountsLaunch kl = cl;  // the stream kernel writes the per-TaxID rows into the temporaries, the permute moves them
+    kl.out_noise = nullptr;
+    kl.out_first = nullptr;
+    if (cl.out_tax) { cp.t_tax = (long long*)tmp(ncap_t * 8); kl.out_tax = (long long*)cp.t_tax; }
+    if (cl.out_nal) { cp.t_nal = (uint32_t*)tmp(ncap_t * 4); kl.out_nal = (uint32_t*)cp.t_nal; }
+    if (d_first_final) { cp.t_first = (long long*)tmp(ncap_t * 8); kl.out_first = (long long*)cp.t_first; }
+    if (cl.out_k) { cp.t_k = (uint32_t*)tmp(ncap_t * R * 4); kl.out_k = (uint32_t*)cp.t_k; }
+    if (cl.out_N) { cp.t_N = (uint32_t*)tmp(ncap_t * R * 4); kl.out_N = (uint32_t*)cp.t_N; }
+    kl.kept_counter = reinterpret_cast<unsigned long long*>(d_ntax + 2);
+    kl.tile_base = d_tile_base;
+    kl.tile_cnt = d_tile_cnt;
+    kl.capacity = out_capacity;
+    kl.error_flag = d_err;
+    MDG_CUDA_TRY(cudaMemsetAsync(d_ntax, 0, 64, st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
+    counts_stream_kernel<<<(unsigned)((n_tiles + kStreamWarps - 1) / kStreamWarps), kStreamWarps * 32, 0, st>>>(kl);
+    MDG_CUDA_TRY(cudaGetLastError());
+    counts_scan_local_kernel<<<(unsigned)n_chunks, kScanChunk, 0, st>>>(d_tile_cnt, n_tiles, d_final_base, d_chunk);
+    counts_scan_chunks_kernel<<<1, 32, 0, st>>>(d_chunk, n_chunks, d_ntax);
+    MDG_CUDA_TRY(cudaGetLastError());
+    counts_permute_kernel<<<(unsigned)((n_tiles + kPermuteWarps * kPermuteTiles - 1) / (kPermuteWarps * kPermuteTiles)), kPermuteWarps * 32, 0, st>>>(cp);
+    MDG_CUDA_TRY(cudaGetLastError());
+    ctx->timings.n_launches += 4;
+    if (cl.out_noise) {
+        NoiseLaunch nl = {};
+        nl.n_rows = n_rows; nl.tax_id = cl.tax_id; nl.is_rev = cl.is_rev; nl.pos0 = cl.pos0; nl.counts16 = cl.counts16;
+        nl.stride = cl.stride; nl.P = P; nl.n_tax = d_ntax; nl.first_row = d_first_final; nl.out_noise = cl.out_noise;
+        nl.capacity = out_capacity;
+        counts_noise_kernel<<<(unsigned)std::max<long long>(1, std::min<long long>((out_capacity + 3) / 4, 16LL * ctx->num_sms)), 128, 0, st>>>(nl);
         MDG_CUDA_TRY(cudaGetLastError());
         ctx->timings.n_launches += 1;
-        counts_permute_kernel<<<(unsigned)((n_tiles + kPermuteWarps * kPermuteTiles - 1) / (kPermuteWarps * kPermuteTiles)), kPermuteWarps * 32, 0, st>>>(cp);
-        MDG_CUDA_TRY(cudaGetLastError());
-        ctx->timings.n_launches += 3;
-        if (cl.out_noise) {
-            NoiseLaunch nl = {};
-            nl.n_rows = n_rows; nl.tax_id = cl.tax_id; nl.is_rev = cl.is_rev; nl.pos0 = cl.pos0; nl.counts16 = cl.counts16;
-            nl.stride = cl.stride; nl.P = P; nl.n_tax = d_ntax; nl.first_row = d_first_final; nl.out_noise = cl.out_noise;
-            nl.capacity = out_capacity;
-            counts_noise_kernel<<<(unsigned)std::max<long long>(1, std::min<long long>((out_capacity + 3) / 4, 16LL * ctx->num_sms)), 128, 0, st>>>(nl);
-            MDG_CUDA_TRY(cudaGetLastError());
-            ctx->timings.n_launches += 1;
-        }
-        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[2], st));
-        MDG_CUDA_TRY(cudaMemcpyAsync(&h_err, d_err, sizeof(int), cudaMemcpyDeviceToHost, st));
-        MDG_CUDA_TRY(cudaMemcpyAsync(&h_ntax, d_ntax, sizeof(long long), cudaMemcpyDeviceToHost, st));
-        MDG_CUDA_TRY(cudaStreamSynchronize(st));
-    } else {
-    static const int ladder_T[3] = {448, 512, 512};
-    static const int ladder_L[3] = {64, 512, MDG_MAX_SEGMENT_ROWS};
-    const size_t row_bytes = (size_t)kCountsBytesPerRow + 4 * (size_t)cl.ncols;
-    const size_t fixed_bytes = 16 + 16 + (size_t)kCountsWarps * 2 * R * 4 + 256;
-    for (int step = 0; step < 3; ++step) {
-        cl.T = ladder_T[step];
-        cl.L = ladder_L[step];
-        if (step == 0) if (const char* t_env = getenv("MDG_COUNTS_T")) { int tv = atoi(t_env); if (tv >= 64 && tv % 16 == 0) cl.T = tv; }  // tile-size experiments
-        // shrink the tile (never the lookahead) until it fits the 227 KB of shared memory
-        while (cl.T > 16 && fixed_bytes + row_bytes * (size_t)(cl.T + cl.L) > 227 * 1024 - 1024) cl.T -= 16;
-        const int cap = cl.T + cl.L;
-        const size_t smem = fixed_bytes + row_bytes * (size_t)cap;
-        if (smem > 227 * 1024 - 1024) {
-            set_error("mdg_counts_reduce: a TaxID spans more rows than one shared-memory tile can stage (%d with these options)",
-                      (int)((227 * 1024 - 1024 - fixed_bytes) / row_bytes) - 16);
-            return MDG_ERR_SEGMENT_TOO_LONG;
-        }
-        const long long n_tiles = (n_rows + cl.T - 1) / cl.T;
-        // per-tile block bookkeeping + temporaries for the (unordered) dense rows
-        const size_t ncap_t = (size_t)out_capacity;
-        rc = ctx->buf[3].ensure((size_t)n_tiles * (8 + 8 + 4) + 64);
-        if (rc) return rc;
-        long long* d_tile_base = ctx->buf[3].as<long long>();
-        long long* d_final_base = d_tile_base + n_tiles;
-        int* d_tile_cnt = reinterpret_cast<int*>(d_final_base + n_tiles);
-        const size_t tmp_bytes = ncap_t * (8 + 4 + 8 + 24 + (size_t)R * 8) + 256 * 8;
-        rc = ctx->buf[21].ensure(tmp_bytes);
-        if (rc) return rc;
-        unsigned char* tb = ctx->buf[21].as<unsigned char>();
-        size_t to = 0;
-        auto tmp = [&](size_t bytes) { void* q = tb + to; to += (bytes + 255) & ~(size_t)255; return q; };
-        CountsPermute cp = {};
-        cp.n_tiles = n_tiles; cp.tile_base = d_tile_base; cp.final_base = d_final_base; cp.tile_cnt = d_tile_cnt; cp.R = R;
-        cp.out_tax = cl.out_tax; cp.out_nal = cl.out_nal; cp.out_first = cl.out_first; cp.out_k = cl.out_k; cp.out_N = cl.out_N;
-        cp.out_noise = cl.out_noise;
-        CountsLaunch kl = cl;  // the tile kernel writes the per-TaxID rows into the temporaries
-        if (cl.out_tax) { cp.t_tax = (long long*)tmp(ncap_t * 8); kl.out_tax = (long long*)cp.t_tax; }
-        if (cl.out_nal) { cp.t_nal = (uint32_t*)tmp(ncap_t * 4); kl.out_nal = (uint32_t*)cp.t_nal; }
-        if (cl.out_first) { cp.t_first = (long long*)tmp(ncap_t * 8); kl.out_first = (long long*)cp.t_first; }
-        if (cl.out_k) { cp.t_k = (uint32_t*)tmp(ncap_t * R * 4); kl.out_k = (uint32_t*)cp.t_k; }
-        if (cl.out_N) { cp.t_N = (uint32_t*)tmp(ncap_t * R * 4); kl.out_N = (uint32_t*)cp.t_N; }
-        if (cl.out_noise) { cp.t_noise = (double*)tmp(ncap_t * 24); kl.out_noise = (double*)cp.t_noise; }
-        kl.tile_ticket = d_ticket;
-        kl.kept_counter = reinterpret_cast<unsigned long long*>(d_ntax + 3);
-        kl.tile_base = d_tile_base;
-        kl.tile_cnt = d_tile_cnt;
-        kl.capacity = out_capacity;
-        kl.error_flag = d_err;
-        MDG_CUDA_TRY(cudaMemsetAsync(d_ntax, 0, 64, st));
-        MDG_CUDA_TRY(cudaFuncSetAttribute(counts_reduce_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
-        counts_reduce_kernel<<<(unsigned)n_tiles, kCountsThreads, smem, st>>>(kl);
-        MDG_CUDA_TRY(cudaGetLastError());
-        counts_scan_kernel<<<1, 1024, 0, st>>>(d_tile_cnt, n_tiles, d_final_base, d_ntax);
-        MDG_CUDA_TRY(cudaGetLastError());
-        counts_permute_kernel<<<(unsigned)((n_tiles + kPermuteWarps * kPermuteTiles - 1) / (kPermuteWarps * kPermuteTiles)), kPermuteWarps * 32, 0, st>>>(cp);
-        MDG_CUDA_TRY(cudaGetLastError());
-        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[2], st));
-        ctx->timings.n_launches += 3;
-        MDG_CUDA_TRY(cudaMemcpyAsync(&h_err, d_err, sizeof(int), cudaMemcpyDeviceToHost, st));
-        MDG_CUDA_TRY(cudaMemcpyAsync(&h_ntax, d_ntax, sizeof(long long), cudaMemcpyDeviceToHost, st));
-        MDG_CUDA_TRY(cudaStreamSynchronize(st));
-        if (h_err != CE_SEGMENT_TOO_LONG) break;
     }
-    }
+    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[2], st));
+    MDG_CUDA_TRY(cudaMemcpyAsync(&h_err, d_err, sizeof(int), cudaMemcpyDeviceToHost, st));
+    MDG_CUDA_TRY(cudaMemcpyAsync(&h_ntax, d_ntax, sizeof(long long), cudaMemcpyDeviceToHost, st));
+    MDG_CUDA_TRY(cudaStreamSynchronize(st));
     if (h_err == CE_SEGMENT_TOO_LONG) {
         set_error("mdg_counts_reduce: a TaxID has more than %d rows (rows must be grouped by tax_id)", MDG_MAX_SEGMENT_ROWS);
         return MDG_ERR_SEGMENT_TOO_LONG;
@@ -732,8 +649,8 @@ int mdg_counts_order(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_i
     ol.perm = reinterpret_cast<long long*>(out_perm);
     MDG_CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
     if (host) {
-        if ((rc = ctx->buf[22].ensure(up(nr * 8) + up(nr) + up(nr) + 2 * up(nt * 8) + up((size_t)perm_capacity * 8)))) return rc;
-        unsigned char* b = ctx->buf[22].as<unsigned char>();
+        if ((rc = ctx->order_tsv_top_in.ensure(up(nr * 8) + up(nr) + up(nr) + 2 * up(nt * 8) + up((size_t)perm_capacity * 8)))) return rc;
+        unsigned char* b = ctx->order_tsv_top_in.as<unsigned char>();
         size_t o = 0;
         auto put = [&](const void* src, size_t bytes) -> void* {
             void* d = b + o; o += up(bytes);
@@ -749,8 +666,8 @@ int mdg_counts_order(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_i
         ol.perm = (long long*)put(nullptr, (size_t)perm_capacity * 8);
         MDG_CUDA_TRY(cudaGetLastError());
     }
-    if ((rc = ctx->buf[23].ensure(up(nt * 4) + up(nt * 8) + 256))) return rc;
-    unsigned char* sb = ctx->buf[23].as<unsigned char>();
+    if ((rc = ctx->order_tsv_top_scratch.ensure(up(nt * 4) + up(nt * 8) + 256))) return rc;
+    unsigned char* sb = ctx->order_tsv_top_scratch.as<unsigned char>();
     ol.len_sorted = reinterpret_cast<int*>(sb);
     long long* d_start = reinterpret_cast<long long*>(sb + up(nt * 4));
     long long* d_total = reinterpret_cast<long long*>(sb + up(nt * 4) + up(nt * 8));
@@ -838,23 +755,23 @@ int mdg_tsv_parse(mdg_ctx* ctx, int mem, const char* text, int64_t n_bytes, int6
     tl.n_bytes = n_bytes; tl.first = first; tl.n_cols = n_cols; tl.capacity = capacity;
     tl.n_blocks = (n_bytes - first + kTsvBlockBytes - 1) / kTsvBlockBytes;
     int rc;
-    if ((rc = ctx->buf[22].ensure((size_t)n_bytes + 16))) return rc;
-    MDG_CUDA_TRY(cudaMemcpyAsync(ctx->buf[22].ptr, text, (size_t)n_bytes, cudaMemcpyHostToDevice, st));
-    tl.text = ctx->buf[22].as<char>();
-    if ((rc = ctx->buf[23].ensure((size_t)tl.n_blocks * 12 + (cap + 2) * 8 + 256))) return rc;
-    tl.block_base = ctx->buf[23].as<long long>();
+    if ((rc = ctx->order_tsv_top_in.ensure((size_t)n_bytes + 16))) return rc;
+    MDG_CUDA_TRY(cudaMemcpyAsync(ctx->order_tsv_top_in.ptr, text, (size_t)n_bytes, cudaMemcpyHostToDevice, st));
+    tl.text = ctx->order_tsv_top_in.as<char>();
+    if ((rc = ctx->order_tsv_top_scratch.ensure((size_t)tl.n_blocks * 12 + (cap + 2) * 8 + 256))) return rc;
+    tl.block_base = ctx->order_tsv_top_scratch.as<long long>();
     tl.line_start = tl.block_base + tl.n_blocks;
     tl.block_cnt = reinterpret_cast<int*>(tl.line_start + cap + 2);
-    if ((rc = ctx->buf[2].ensure(64))) return rc;
-    long long* d_scal = ctx->buf[2].as<long long>();  // [0] newline total, [1] error flag (int), [2] error line
+    if ((rc = ctx->reduce_tsv_scalars.ensure(64))) return rc;
+    long long* d_scal = ctx->reduce_tsv_scalars.as<long long>();  // [0] newline total, [1] error flag (int), [2] error line
     tl.n_lines = d_scal; tl.error_flag = reinterpret_cast<int*>(d_scal + 1); tl.error_line = d_scal + 2;
     MDG_CUDA_TRY(cudaMemsetAsync(d_scal, 0, 64, st));
     struct OutCopy { void* host_ptr; const void* dev_ptr; size_t bytes_per_row; };
     std::vector<OutCopy> copies;
     if (host) {
         const size_t stride_dev = (cap + 63) & ~(size_t)63;
-        if ((rc = ctx->buf[1].ensure(cap * (8 + 4 + 1 + 1 + 32) + 16 * stride_dev * 4 + 4096))) return rc;
-        unsigned char* ob = ctx->buf[1].as<unsigned char>();
+        if ((rc = ctx->reduce_tsv_out.ensure(cap * (8 + 4 + 1 + 1 + 32) + 16 * stride_dev * 4 + 4096))) return rc;
+        unsigned char* ob = ctx->reduce_tsv_out.as<unsigned char>();
         size_t oo = 0;
         auto take = [&](void* hp, size_t elem) -> void* {
             void* d = ob + oo;
@@ -951,8 +868,8 @@ int mdg_select_top(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_id_
     auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
     if (host) {
         const size_t in_bytes = up(nr * 8) + up(nr * 4) + up(nr) + 2 * up(nt * 8);
-        if ((rc = ctx->buf[22].ensure(in_bytes))) return rc;
-        unsigned char* b = ctx->buf[22].as<unsigned char>();
+        if ((rc = ctx->order_tsv_top_in.ensure(in_bytes))) return rc;
+        unsigned char* b = ctx->order_tsv_top_in.as<unsigned char>();
         size_t o = 0;
         auto put = [&](const void* src, size_t bytes) -> void* {
             void* d = b + o; o += up(bytes);
@@ -970,8 +887,8 @@ int mdg_select_top(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_id_
     const int n_blocks = (int)((n_tax + kTopThreads - 1) / kTopThreads);
     const size_t scratch = up(kTopPasses * 256 * 4) + up((size_t)n_blocks * 4) + up((size_t)n_blocks * 8) + up(8) +
                            ((host || !out_weight) ? up(nt * 8) : 0) + (host ? up((size_t)take * 8 + 8) : 0);
-    if ((rc = ctx->buf[23].ensure(scratch))) return rc;
-    unsigned char* sb = ctx->buf[23].as<unsigned char>();
+    if ((rc = ctx->order_tsv_top_scratch.ensure(scratch))) return rc;
+    unsigned char* sb = ctx->order_tsv_top_scratch.as<unsigned char>();
     size_t so = 0;
     auto carve = [&](size_t bytes) { void* q = sb + so; so += up(bytes); return q; };
     TopLaunch tl = {};
@@ -1110,7 +1027,7 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
 
     const int sample_runs = out_samples ? MDG_NUM_RUNS : (fwd_rev ? 3 : 1);
     const int items_per_tax = R + (fwd_rev ? 2 : 0);
-    // TaxIDs per chunk: every chunk ends with the tail of its four NUTS launches (the next chunk starts under
+    // TaxIDs per chunk: every chunk ends with the tail of its NUTS launches (the next chunk starts under
     // it on the other lane), so chunks are as large as ~8 GB of scratch per lane allows (posterior draws
     // dominate: 96 KB per TaxID at S = 1000)
     long long chunk_cap = 65536;
@@ -1223,7 +1140,7 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
         }
         MDG_CUDA_TRY(cudaEventRecord(ln.ev[1], ls));
 
-        // ---- K4 NUTS: four launches on four streams (they share the SMs as CTAs retire) ----
+        // ---- K4 NUTS: one launch per model, each on its own stream (they share the SMs as CTAs retire) ----
         FitLaunch fl = {};
         fl.tax_id = d_tax + c0; fl.k = d_k + (size_t)c0 * R; fl.N = d_N + (size_t)c0 * R;
         fl.n_tax = nc; fl.P = P; fl.cfg = *cfg; fl.pr = pr;
@@ -1266,50 +1183,31 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
         // Overlap with the chunk in flight on another lane is wanted for its TAIL only (a few long chains on an
         // otherwise idle GPU), not for its bulk: two different NUTS kernels sharing the SMs evict each other from
         // the instruction cache (measured: -2..-5 % with unrestricted overlap). So this chunk's NUTS launches wait
-        // until the other chunk's first three launches are through and only its last one (null model, all
-        // positions: short, uniform chains) is still running.
+        // until the other chunk's PMD launch is through and only its null launch (short, uniform chains) is still
+        // running.
         for (auto& other : ctx->lane)
-            if (&other != &ln && other.busy)
-                for (int i = 1; i < 4; ++i) MDG_CUDA_TRY(cudaStreamWaitEvent(ls, other.join_ev[i], 0));
+            if (&other != &ln && other.busy) MDG_CUDA_TRY(cudaStreamWaitEvent(ls, other.join_ev[0], 0));
         MDG_CUDA_TRY(cudaEventRecord(ln.fork_ev, ls));
-        for (int i = 0; i < 4; ++i) MDG_CUDA_TRY(cudaStreamWaitEvent(ln.side[i], ln.fork_ev, 0));
+        for (cudaStream_t sd : ln.side) MDG_CUDA_TRY(cudaStreamWaitEvent(sd, ln.fork_ev, 0));
         {
             // Launch order = dispatch order of the persistent CTAs: the kernels share the SMs as CTAs
             // retire, so the whole step behaves like one list schedule over all (TaxID, run) items.
             // PMD chains are long and heavy-tailed (adapted step size; max ~8x the mean), null chains
             // short and uniform: PMD first, null last fills the tail (profiles/r01_nuts_tuning.md).
-            FitLaunch a = fl;  // PMD, all positions
-            a.n_items = nc; a.n_items_all = nc; a.n_prio = 0; a.work_counter = d_counters + 1;
-            FitLaunch b = a;   // null, all positions
+            // One launch and ONE queue per model: the all-position runs first (the longest chains), then the
+            // forward-only / reverse-only runs. A group that finishes a chain always finds the next item until the
+            // model's whole queue is empty, so the only hand-over between launches (CTA slots are released per CTA,
+            // i.e. when the last of its 16 chains ends) is PMD -> null.
+            FitLaunch a = fl;  // PMD
+            a.n_items = fwd_rev ? 3 * nc : nc; a.n_items_all = nc; a.work_counter = d_counters + 1;
+            FitLaunch b = a;   // null
             b.work_counter = d_counters + 2;
-            FitLaunch c = fl, d = fl;  // PMD / null, forward-only and reverse-only
-            c.work_counter = d_counters + 3; d.work_counter = d_counters + 4;
-            c.n_items = 2 * nc; d.n_items = 2 * nc; c.n_items_all = 0; d.n_items_all = 0; c.n_prio = 0; d.n_prio = 0;
-            const int gw_all = env_int("MDG_GW_ALL", 8), gw_half = env_int("MDG_GW_HALF", 8);  // lanes per chain (A/B runs: 16)
-            if (fwd_rev && env_int("MDG_NUTS_MERGE", 1)) {
-                // One launch and ONE queue per model: the all-position runs first (the longest chains), then the
-                // forward-only / reverse-only runs. A group that finishes a chain always finds the next item until the
-                // model's whole queue is empty, so the only hand-over between launches (CTA slots are released per CTA,
-                // i.e. when the last of its 16 chains ends) is PMD -> null.
-                a.n_items = 3 * nc; b.n_items = 3 * nc;
-                a.n_prio = fl.n_prio; b.n_prio = fl.n_prio;
-                if ((rc = launch_nuts_group_dispatch<0>(ctx, ln.side[3], a, ln.waic_acc[0], gw_all))) return bail(rc);
-                if ((rc = launch_nuts_group_dispatch<1>(ctx, ln.side[0], b, ln.waic_acc[1], gw_all))) return bail(rc);
-            } else if (env_int("MDG_NUTS_A_FIRST", 1)) {
-                if ((rc = launch_nuts_group_dispatch<0>(ctx, ln.side[3], a, ln.waic_acc[0], gw_all))) return bail(rc);
-                if (fwd_rev && (rc = launch_nuts_group_dispatch<0>(ctx, ln.side[1], c, ln.waic_acc[2], gw_half))) return bail(rc);
-                if (fwd_rev && (rc = launch_nuts_group_dispatch<1>(ctx, ln.side[2], d, ln.waic_acc[3], gw_half))) return bail(rc);
-                if ((rc = launch_nuts_group_dispatch<1>(ctx, ln.side[0], b, ln.waic_acc[1], gw_all))) return bail(rc);
-            } else {
-                if (fwd_rev && (rc = launch_nuts_group_dispatch<0>(ctx, ln.side[1], c, ln.waic_acc[2], gw_half))) return bail(rc);
-                if ((rc = launch_nuts_group_dispatch<0>(ctx, ln.side[3], a, ln.waic_acc[0], gw_all))) return bail(rc);
-                if (fwd_rev && (rc = launch_nuts_group_dispatch<1>(ctx, ln.side[2], d, ln.waic_acc[3], gw_half))) return bail(rc);
-                if ((rc = launch_nuts_group_dispatch<1>(ctx, ln.side[0], b, ln.waic_acc[1], gw_all))) return bail(rc);
-            }
+            if ((rc = launch_nuts_group<0>(ctx, ln.side[0], a, ln.waic_acc[0]))) return bail(rc);
+            if ((rc = launch_nuts_group<1>(ctx, ln.side[1], b, ln.waic_acc[1]))) return bail(rc);
         }
-        for (int i = 0; i < 4; ++i) {
-            MDG_CUDA_TRY(cudaEventRecord(ln.join_ev[i], ln.side[i]));
-            MDG_CUDA_TRY(cudaStreamWaitEvent(ls, ln.join_ev[i], 0));
+        for (int m = 0; m < 2; ++m) {
+            MDG_CUDA_TRY(cudaEventRecord(ln.join_ev[m], ln.side[m]));
+            MDG_CUDA_TRY(cudaStreamWaitEvent(ls, ln.join_ev[m], 0));
         }
         MDG_CUDA_TRY(cudaEventRecord(ln.ev[2], ls));
 
@@ -1575,9 +1473,9 @@ int mdg_test_lgamma_digamma(mdg_ctx* ctx, int64_t n, const double* x, double* ou
     if (!ctx || n < 0) { set_error("invalid argument"); return MDG_ERR_INVALID; }
     if (n == 0) return MDG_OK;
     DeviceGuard guard(ctx->device);
-    int rc = ctx->buf[20].ensure((size_t)n * 24);
+    int rc = ctx->test_scratch.ensure((size_t)n * 24);
     if (rc) return rc;
-    double* d = ctx->buf[20].as<double>();
+    double* d = ctx->test_scratch.as<double>();
     MDG_CUDA_TRY(cudaMemcpyAsync(d, x, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
     test_lgam_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(n, d, d + n, d + 2 * n);
     MDG_CUDA_TRY(cudaGetLastError());
@@ -1591,9 +1489,9 @@ int mdg_test_exp_log(mdg_ctx* ctx, int64_t n, const double* x, double* out_exp, 
     if (!ctx || n < 0) { set_error("invalid argument"); return MDG_ERR_INVALID; }
     if (n == 0) return MDG_OK;
     DeviceGuard guard(ctx->device);
-    int rc = ctx->buf[20].ensure((size_t)n * 24);
+    int rc = ctx->test_scratch.ensure((size_t)n * 24);
     if (rc) return rc;
-    double* d = ctx->buf[20].as<double>();
+    double* d = ctx->test_scratch.as<double>();
     MDG_CUDA_TRY(cudaMemcpyAsync(d, x, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
     test_exp_log_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(n, d, d + n, d + 2 * n);
     MDG_CUDA_TRY(cudaGetLastError());
@@ -1607,9 +1505,9 @@ int mdg_test_philox(mdg_ctx* ctx, int64_t n, const uint32_t* key2, const uint32_
     if (!ctx || n < 0) { set_error("invalid argument"); return MDG_ERR_INVALID; }
     if (n == 0) return MDG_OK;
     DeviceGuard guard(ctx->device);
-    int rc = ctx->buf[20].ensure((size_t)n * 40);
+    int rc = ctx->test_scratch.ensure((size_t)n * 40);
     if (rc) return rc;
-    uint32_t* d = ctx->buf[20].as<uint32_t>();
+    uint32_t* d = ctx->test_scratch.as<uint32_t>();
     MDG_CUDA_TRY(cudaMemcpyAsync(d, key2, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
     MDG_CUDA_TRY(cudaMemcpyAsync(d + 2 * n, ctr4, (size_t)n * 16, cudaMemcpyHostToDevice, ctx->stream));
     test_philox_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(n, d, d + 2 * n, d + 6 * n);
@@ -1631,9 +1529,9 @@ int mdg_test_logp_grad(mdg_ctx* ctx, int max_position, const uint32_t* k, const 
     DeviceGuard guard(ctx->device);
     const int P = max_position, R = 2 * P;
     const size_t ne = (size_t)n_eval;
-    int rc = ctx->buf[20].ensure((size_t)R * 8 + ne * (32 + 8 + 32 + (size_t)R * 8) + 1024);
+    int rc = ctx->test_scratch.ensure((size_t)R * 8 + ne * (32 + 8 + 32 + (size_t)R * 8) + 1024);
     if (rc) return rc;
-    unsigned char* base = ctx->buf[20].as<unsigned char>();
+    unsigned char* base = ctx->test_scratch.as<unsigned char>();
     uint32_t* dk = (uint32_t*)base;
     uint32_t* dN = dk + R;
     double* du = (double*)(base + (((size_t)R * 8 + 255) & ~(size_t)255));
@@ -1664,15 +1562,15 @@ int mdg_test_logp_grad(mdg_ctx* ctx, int max_position, const uint32_t* k, const 
 int mdg_measure_fp64_peak(mdg_ctx* ctx, double* out_tflops) {
     if (!ctx || !out_tflops) { set_error("invalid argument"); return MDG_ERR_INVALID; }
     DeviceGuard guard(ctx->device);
-    int rc = ctx->buf[20].ensure(64);
+    int rc = ctx->test_scratch.ensure(64);
     if (rc) return rc;
     cudaStream_t st = ctx->stream;
     const int iters = 20000, threads = 512, blocks = ctx->num_sms * 4;
-    fp64_peak_kernel<<<blocks, threads, 0, st>>>(ctx->buf[20].as<double>(), 1000);  // warm-up
+    fp64_peak_kernel<<<blocks, threads, 0, st>>>(ctx->test_scratch.as<double>(), 1000);  // warm-up
     double best = 0.0;
     for (int rep = 0; rep < 3; ++rep) {
         MDG_CUDA_TRY(cudaEventRecord(ctx->ev[10], st));
-        fp64_peak_kernel<<<blocks, threads, 0, st>>>(ctx->buf[20].as<double>(), iters);
+        fp64_peak_kernel<<<blocks, threads, 0, st>>>(ctx->test_scratch.as<double>(), iters);
         MDG_CUDA_TRY(cudaEventRecord(ctx->ev[11], st));
         MDG_CUDA_TRY(cudaStreamSynchronize(st));
         MDG_CUDA_TRY(cudaGetLastError());

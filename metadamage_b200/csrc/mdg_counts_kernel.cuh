@@ -4,32 +4,20 @@
 // handling 117-129, fillna 175-176, y_sum_total 179-204, cuts 207-209) and the dense extraction
 // of fits.py:398-419; optionally the noise statistic of fits.py:359-376.
 //
-// HBM-bound (111 algorithmic bytes per row, SURVEY.md 8d). Design:
-//   * one CTA per tile of T rows plus an L-row lookahead; the tile's SoA column chunks come into
-//     shared memory through 1-D TMA bulk copies (cp.async.bulk -> UBLKCP) on one mbarrier;
-//   * the CTA owns every TaxID whose first row lies in [row0, row0+T): no carry crosses tiles,
-//     the only inter-CTA traffic is ONE atomicAdd per tile that reserves the tile's block of dense
-//     output rows; a one-CTA scan and a block-permute kernel then put the blocks into input order
-//     (a decoupled look-back was measured to stall 28-42 % of the warp samples: with 448-row tiles
-//     the inclusive prefix cannot propagate as fast as tiles retire);
-//   * per-row work is vectorised: one thread handles 4 consecutive rows with 128-bit shared
-//     loads and writes the row-local outputs (reference sums, error rates, z) of the tile's
-//     nominal rows straight from registers with 128-bit stores (tile starts are 16-byte aligned
-//     for every column type); y_sum_total and the cut flag follow once the TaxID sums are known;
-//   * per-TaxID sums are a short serial loop of one thread per TaxID over staged values (a warp
-//     per TaxID with a shuffle reduction was measured 7 % slower); the
-//     dense k/N (and the optional noise) of KEPT TaxIDs use one warp per TaxID, lane = row.
-// The first version (one warp per TaxID for everything) was instruction-issue bound at 30 warp
-// instructions per row (profiles/r01_counts_ncu.md); this layout needs a few.
+// This file holds what the streaming kernel (mdg_counts_stream.cuh) is built on: the launch struct,
+// the bit-exact error rate, and the scans and block permute that put its per-TaxID rows into input
+// order; also K1d, the row order of df_counts. counts_scan_kernel serves K0 and K8 as well.
+//
+// HBM-bound (111 algorithmic bytes per row, SURVEY.md 8d). A tile of rows owns every TaxID whose
+// first row it holds, so no carry crosses tiles: the only traffic between tiles is ONE atomicAdd per
+// tile that reserves the tile's block of dense output rows (in no particular order); a scan of the
+// per-tile counts and a block permute then put the blocks into input order. A decoupled look-back
+// that writes the rows straight to their final places was measured slower: every tile then waits
+// for its predecessors to publish their counts (DESIGN.md §4, profiles/r01_counts_ncu.md).
 #pragma once
 #include "mdg_common.cuh"
 
 namespace mdg {
-
-constexpr int kCountsThreads = 128;
-constexpr int kCountsWarps = kCountsThreads / 32;
-// shared bytes per staged row, without the count columns (4 bytes per staged column on top)
-constexpr int kCountsBytesPerRow = 8 + 4 + 1 + 1 + 8 + 4 + 1 + 1 + 4 + 8 + 1 + 1;
 
 enum CountsError : int { CE_NONE = 0, CE_SEGMENT_TOO_LONG = 1, CE_OVERFLOW = 2, CE_CAPACITY = 3 };
 
@@ -60,27 +48,14 @@ struct CountsLaunch {
     uint32_t* out_k;
     uint32_t* out_N;
     double* out_noise;
-    // tiling
-    int T, L;               // owned rows per tile (multiple of 16), lookahead rows; T + L multiple of 16
-    int ncols;              // count columns staged in shared memory
-    int col_id[16];         // which of the 16 columns
-    int col_slot[16];       // column -> staged slot (or -1)
-    int use_tma;            // all column bases 16-byte aligned
+    int vec_in;             // input column bases 16-byte aligned and stride % 4 == 0 -> 128-bit loads
     int vec_out;            // per-row output bases 16-byte aligned -> 128-bit stores
-    unsigned int* tile_ticket;
     unsigned long long* kept_counter;  // device scalar: dense rows reserved so far (unordered, one atomicAdd per tile)
     long long* tile_base;              // [n_tiles] start of the tile's block in the temporary dense arrays
     int* tile_cnt;                     // [n_tiles] kept TaxIDs of the tile
     long long capacity;                // rows available in the per-TaxID arrays
     int* error_flag;
 };
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void tma_load_1d(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 :: "r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
 
 __device__ __forceinline__ double warp_sum_f64(double v) {
 #pragma unroll
@@ -106,388 +81,9 @@ __device__ __forceinline__ float error_rate(uint32_t k, uint32_t n) {
     return (k && n) ? (float)q : 0.0f;
 }
 
-#ifndef MDG_COUNTS_MINBLOCKS
-#define MDG_COUNTS_MINBLOCKS 6
-#endif
-
-__global__ void __launch_bounds__(kCountsThreads, MDG_COUNTS_MINBLOCKS) counts_reduce_kernel(const CountsLaunch p) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int cap = p.T + p.L;  // rows staged per tile (multiple of 16)
-    // ---- shared layout (every array starts 16-byte aligned because cap % 16 == 0) ----
-    long long* s_tax = reinterpret_cast<long long*>(smem_raw);  // s_tax[2+i] = tax id of staged row i; s_tax[1] = row before
-    uint32_t* s_cnt = reinterpret_cast<uint32_t*>(s_tax + cap + 2);
-    uint32_t* s_nal = s_cnt + (size_t)p.ncols * cap;
-    uint32_t* o_nf = s_nal + cap;
-    uint32_t* o_nr = o_nf + cap;
-    uint32_t* o_yc = o_nr + cap;                                // y contribution of the row; later: rank of the segment
-    int* s_seg = reinterpret_cast<int*>(o_yc + cap);            // head row of segment s; s_seg[nseg] = nload
-    unsigned long long* s_ysum = reinterpret_cast<unsigned long long*>(s_seg + cap + 4);
-    uint8_t* s_rev = reinterpret_cast<uint8_t*>(s_ysum + cap);
-    uint8_t* s_pos = s_rev + cap;
-    int8_t* o_z = reinterpret_cast<int8_t*>(s_pos + cap);
-    uint8_t* o_head = reinterpret_cast<uint8_t*>(o_z + cap);
-    uint8_t* s_kept = o_head + cap;
-    int* s_gseg = reinterpret_cast<int*>(s_kept + cap);              // [cap / 4] segment of each 4-row group's first row
-    uint32_t* s_dense = reinterpret_cast<uint32_t*>(s_gseg + cap / 4);  // [warps][2][2P]
-    __shared__ uint64_t s_bar;
-    __shared__ int s_warp_cnt[kCountsWarps];
-    __shared__ int s_nseg, s_nowned, s_kept_total;
-    __shared__ long long s_base;
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid == 0) s_nowned = 0;  // (made visible by the barrier that ends the staging step)
-    const unsigned tile = blockIdx.x;  // tiles are independent: no ticket, no ordering between CTAs
-    const long long row0 = (long long)tile * p.T;
-    const long long remaining = p.n_rows - row0;
-    const int nload = (int)(remaining < cap ? remaining : cap);
-    const int nown = nload < p.T ? nload : p.T;
-    const bool last_rows = (row0 + nload == p.n_rows);
-    const int P = p.P, R = 2 * P;
-
-    // ---------------- stage the tile ----------------
-    const bool tma = p.use_tma && (nload % 16 == 0);
-    if (tma) {
-        if (tid == 0) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(&s_bar)), "r"(1));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            const uint32_t total = (uint32_t)nload * (8u + 4u + 1u + 1u + 4u * (uint32_t)p.ncols);
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(&s_bar)), "r"(total) : "memory");
-            tma_load_1d(s_tax + 2, p.tax_id + row0, (uint32_t)nload * 8u, &s_bar);
-            for (int c = 0; c < p.ncols; ++c)
-                tma_load_1d(s_cnt + (size_t)c * cap, p.counts16 + (long long)p.col_id[c] * p.stride + row0, (uint32_t)nload * 4u, &s_bar);
-            tma_load_1d(s_nal, p.n_align + row0, (uint32_t)nload * 4u, &s_bar);
-            tma_load_1d(s_rev, p.is_rev + row0, (uint32_t)nload, &s_bar);
-            tma_load_1d(s_pos, p.pos0 + row0, (uint32_t)nload, &s_bar);
-            s_tax[1] = row0 > 0 ? p.tax_id[row0 - 1] : 0;
-            // one thread sleeps on the barrier; the rest of the CTA waits in bar.sync (no issue slots)
-            uint32_t done = 0;
-            while (!done) {
-                asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                             : "=r"(done) : "r"(smem_u32(&s_bar)), "r"(0), "r"(2000000) : "memory");
-            }
-        }
-        __syncthreads();
-    } else {
-        for (int i = tid; i < nload; i += kCountsThreads) {
-            s_tax[2 + i] = p.tax_id[row0 + i];
-            s_nal[i] = p.n_align[row0 + i];
-            s_rev[i] = p.is_rev[row0 + i];
-            s_pos[i] = p.pos0[row0 + i];
-        }
-        for (int c = 0; c < p.ncols; ++c) {
-            const uint32_t* src = p.counts16 + (long long)p.col_id[c] * p.stride + row0;
-            for (int i = tid; i < nload; i += kCountsThreads) s_cnt[(size_t)c * cap + i] = src[i];
-        }
-        if (tid == 0) s_tax[1] = row0 > 0 ? p.tax_id[row0 - 1] : 0;
-        __syncthreads();
-    }
-    const long long* taxv = s_tax + 2;  // taxv[i], i in [-1, nload)
-
-    const int sf0 = p.col_slot[p.fwd_ref * 4], sr0 = p.col_slot[p.rev_ref * 4];
-    const int skf = p.col_slot[p.fwd_ref * 4 + p.fwd_obs], skr = p.col_slot[p.rev_ref * 4 + p.rev_obs];
-
-    // ---------------- phase 1: 4 rows per thread; per-row values + ordered list of TaxID heads ----------------
-    const int ngroups = (nload + 3) >> 2;
-    int seg_base = 0;  // heads found in earlier trips of this loop
-    for (int g0 = 0; g0 < ngroups; g0 += kCountsThreads) {
-        const int g = g0 + tid;
-        const int i0 = g << 2;
-        int nheads = 0;
-        uint32_t headbits = 0;
-        if (g < ngroups) {
-            uint32_t nf[4] = {0, 0, 0, 0}, nr[4] = {0, 0, 0, 0};
-            uint32_t ovfmask = 0;
-            {
-                // a uint32 sum of four terms can only wrap if some term has one of its top two bits
-                // set: OR everything, and only then (never on real data) redo the sums with carries
-                uint4 a[4], b[4];
-                uint32_t any = 0;
-#pragma unroll
-                for (int o = 0; o < 4; ++o) {
-                    a[o] = *reinterpret_cast<const uint4*>(s_cnt + (size_t)(sf0 + o) * cap + i0);
-                    b[o] = *reinterpret_cast<const uint4*>(s_cnt + (size_t)(sr0 + o) * cap + i0);
-                    any |= a[o].x | a[o].y | a[o].z | a[o].w | b[o].x | b[o].y | b[o].z | b[o].w;
-                }
-#pragma unroll
-                for (int o = 0; o < 4; ++o) {
-                    nf[0] += a[o].x; nf[1] += a[o].y; nf[2] += a[o].z; nf[3] += a[o].w;
-                    nr[0] += b[o].x; nr[1] += b[o].y; nr[2] += b[o].z; nr[3] += b[o].w;
-                }
-                if (any >> 30) {
-                    unsigned long long wf[4] = {0, 0, 0, 0}, wr[4] = {0, 0, 0, 0};
-#pragma unroll
-                    for (int o = 0; o < 4; ++o) {
-                        wf[0] += a[o].x; wf[1] += a[o].y; wf[2] += a[o].z; wf[3] += a[o].w;
-                        wr[0] += b[o].x; wr[1] += b[o].y; wr[2] += b[o].z; wr[3] += b[o].w;
-                    }
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) ovfmask |= (uint32_t)(((wf[j] | wr[j]) >> 32) != 0) << j;
-                }
-            }
-            const uint4 kfv = *reinterpret_cast<const uint4*>(s_cnt + (size_t)skf * cap + i0);
-            const uint4 krv = *reinterpret_cast<const uint4*>(s_cnt + (size_t)skr * cap + i0);
-            const uint32_t kf[4] = {kfv.x, kfv.y, kfv.z, kfv.w}, kr[4] = {krv.x, krv.y, krv.z, krv.w};
-            const uchar4 pv = *reinterpret_cast<const uchar4*>(s_pos + i0);
-            const uchar4 rv = *reinterpret_cast<const uchar4*>(s_rev + i0);
-            const int pos[4] = {pv.x, pv.y, pv.z, pv.w};
-            const bool rev[4] = {rv.x != 0, rv.y != 0, rv.z != 0, rv.w != 0};
-            long long tx[5];
-            tx[0] = taxv[i0 - 1];
-            {
-                const longlong2 t01 = *reinterpret_cast<const longlong2*>(taxv + i0);
-                const longlong2 t23 = *reinterpret_cast<const longlong2*>(taxv + i0 + 2);
-                tx[1] = t01.x; tx[2] = t01.y; tx[3] = t23.x; tx[4] = t23.y;
-            }
-            float ff[4], fr[4];
-            uint32_t yc[4], zpack = 0;
-            bool ovf = false;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const int i = i0 + j;
-                const bool valid = i < nload;
-                ovf |= valid && ((ovfmask >> j) & 1u);
-                const int zabs = pos[j] + 1;
-                ff[j] = error_rate(kf[j], nf[j]);
-                fr[j] = error_rate(kr[j], nr[j]);
-                yc[j] = (valid && zabs <= P) ? (rev[j] ? kr[j] : kf[j]) : 0u;
-                const int z = rev[j] ? -zabs : zabs;
-                zpack |= ((uint32_t)(uint8_t)(int8_t)z) << (8 * j);
-                const bool head = valid && ((row0 + i == 0) || (tx[j + 1] != tx[j]));
-                headbits |= (head ? 1u : 0u) << (8 * j);
-                nheads += head ? 1 : 0;
-            }
-            if (ovf) atomicMax(p.error_flag, (int)CE_OVERFLOW);
-            *reinterpret_cast<uint4*>(o_nf + i0) = make_uint4(nf[0], nf[1], nf[2], nf[3]);
-            *reinterpret_cast<uint4*>(o_nr + i0) = make_uint4(nr[0], nr[1], nr[2], nr[3]);
-            *reinterpret_cast<uint4*>(o_yc + i0) = make_uint4(yc[0], yc[1], yc[2], yc[3]);
-            *reinterpret_cast<uint32_t*>(o_z + i0) = zpack;
-            *reinterpret_cast<uint32_t*>(o_head + i0) = headbits;
-            // row-local outputs of the tile's nominal rows [0, nown): every row has exactly one nominal tile
-            const long long gi = row0 + i0;
-            if (p.vec_out && i0 + 4 <= nown) {
-                if (p.n_fwd_row) *reinterpret_cast<uint4*>(p.n_fwd_row + gi) = make_uint4(nf[0], nf[1], nf[2], nf[3]);
-                if (p.n_rev_row) *reinterpret_cast<uint4*>(p.n_rev_row + gi) = make_uint4(nr[0], nr[1], nr[2], nr[3]);
-                if (p.f_fwd_row) *reinterpret_cast<float4*>(p.f_fwd_row + gi) = make_float4(ff[0], ff[1], ff[2], ff[3]);
-                if (p.f_rev_row) *reinterpret_cast<float4*>(p.f_rev_row + gi) = make_float4(fr[0], fr[1], fr[2], fr[3]);
-                if (p.z_row) *reinterpret_cast<uint32_t*>(p.z_row + gi) = zpack;
-            } else {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    if (i0 + j >= nown) continue;
-                    if (p.n_fwd_row) p.n_fwd_row[gi + j] = nf[j];
-                    if (p.n_rev_row) p.n_rev_row[gi + j] = nr[j];
-                    if (p.f_fwd_row) p.f_fwd_row[gi + j] = ff[j];
-                    if (p.f_rev_row) p.f_rev_row[gi + j] = fr[j];
-                    if (p.z_row) p.z_row[gi + j] = (int8_t)((zpack >> (8 * j)) & 0xffu);
-                }
-            }
-        }
-        // ordered compaction of the head rows: warp scan + block offsets
-        int incl = nheads;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
-        if (lane == 31) s_warp_cnt[warp] = incl;
-        __syncthreads();
-        int off = seg_base + incl - nheads, total = 0;
-#pragma unroll
-        for (int w = 0; w < kCountsWarps; ++w) { const int c = s_warp_cnt[w]; off += (w < warp) ? c : 0; total += c; }
-        // segment (index into s_seg) that this group's first row belongs to; -1 = a TaxID of the previous tile
-        if (g < ngroups) s_gseg[g] = off - ((headbits & 1u) ? 0 : 1);
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-            if ((headbits >> (8 * j)) & 1u) s_seg[off++] = i0 + j;
-        seg_base += total;
-        __syncthreads();
-    }
-    if (tid == 0) { s_nseg = seg_base; s_seg[seg_base] = nload; }
-    __syncthreads();
-    const int nseg = s_nseg;
-
-    // ---------------- phase 2: one thread per owned TaxID: y_sum_total and the cut ----------------
-    {
-        int local_owned = 0;
-        for (int s = tid; s < nseg; s += kCountsThreads) {
-            const int a = s_seg[s];
-            if (a >= nown) break;  // heads are sorted: the rest belongs to the next tile
-            ++local_owned;
-            const int b = s_seg[s + 1];
-            unsigned long long ysum = 0;
-            bool any_row = false;
-            for (int r = a; r < b; ++r) {
-                ysum += o_yc[r];
-                const int z = o_z[r];
-                any_row |= (s_nal[r] >= p.min_align) && ((z < 0 ? -z : z) <= P);
-            }
-            s_ysum[s] = ysum;
-            s_kept[s] = (any_row && ysum >= p.min_y) ? 1 : 0;
-        }
-        local_owned = __reduce_add_sync(0xffffffffu, local_owned);
-        if (lane == 0 && local_owned) atomicAdd(&s_nowned, local_owned);
-    }
-    __syncthreads();
-    const int nowned = s_nowned;
-    // the last owned TaxID must end inside the staged rows (or at the end of the data)
-    if (tid == 0 && nowned > 0 && !((nowned < nseg) || last_rows)) atomicMax(p.error_flag, (int)CE_SEGMENT_TOO_LONG);
-
-    // ---------------- phase 3 (warp 0): ranks of the kept TaxIDs, publish the tile aggregate ----------------
-    uint32_t* s_rank = o_yc;  // o_yc is dead after phase 2
-    if (warp == 0) {
-        int running = 0;
-        for (int b0 = 0; b0 < nowned; b0 += 32) {
-            const int s = b0 + lane;
-            const int v = (s < nowned) ? (int)s_kept[s] : 0;
-            int incl = v;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
-            if (s < nowned) s_rank[s] = (uint32_t)(running + incl - v);
-            running += __shfl_sync(0xffffffffu, incl, 31);
-        }
-        if (lane == 0) {
-            s_kept_total = running;
-            const long long base = running ? (long long)atomicAdd(p.kept_counter, (unsigned long long)running) : 0;
-            s_base = base;
-            p.tile_base[tile] = base;
-            p.tile_cnt[tile] = running;
-            if (base + running > p.capacity) atomicMax(p.error_flag, (int)CE_CAPACITY);
-        }
-        __syncwarp();
-    }
-
-    // ---------------- phase 4: y_sum_total and the cut flag of the owned rows ----------------
-    if (nowned > 0 && (p.y_row || p.keep_row)) {
-        const int a0 = s_seg[0], a1 = s_seg[nowned];
-        for (int g = tid + (a0 >> 2); g < ((a1 + 3) >> 2); g += kCountsThreads) {
-            const int i0 = g << 2;
-            // TaxID of the first owned row of this group (recorded by the head compaction of phase 1)
-            const int ifirst = i0 < a0 ? a0 : i0;
-            int s = i0 < a0 ? 0 : s_gseg[g];
-            const uint32_t headbits = *reinterpret_cast<const uint32_t*>(o_head + i0);
-            const uint32_t zpack = *reinterpret_cast<const uint32_t*>(o_z + i0);
-            const uint4 nal4 = *reinterpret_cast<const uint4*>(s_nal + i0);
-            const uint32_t nal[4] = {nal4.x, nal4.y, nal4.z, nal4.w};
-            unsigned long long y[4];
-            uint32_t keeppack = 0;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const int i = i0 + j;
-                if (i > ifirst && ((headbits >> (8 * j)) & 1u)) ++s;
-                const int z = (int)(int8_t)((zpack >> (8 * j)) & 0xffu);
-                const unsigned long long ys = s_ysum[s < nowned ? s : nowned - 1];
-                y[j] = ys;
-                const bool keep = (nal[j] >= p.min_align) && (ys >= p.min_y) && ((z < 0 ? -z : z) <= P);
-                keeppack |= (keep ? 1u : 0u) << (8 * j);
-            }
-            const long long gi = row0 + i0;
-            if (p.vec_out && i0 >= a0 && i0 + 4 <= a1) {
-                if (p.y_row) {
-                    *reinterpret_cast<ulonglong2*>(p.y_row + gi) = make_ulonglong2(y[0], y[1]);
-                    *reinterpret_cast<ulonglong2*>(p.y_row + gi + 2) = make_ulonglong2(y[2], y[3]);
-                }
-                if (p.keep_row) *reinterpret_cast<uint32_t*>(p.keep_row + gi) = keeppack;
-            } else {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const int i = i0 + j;
-                    if (i < a0 || i >= a1) continue;
-                    if (p.y_row) p.y_row[gi + j] = y[j];
-                    if (p.keep_row) p.keep_row[gi + j] = (uint8_t)((keeppack >> (8 * j)) & 1u);
-                }
-            }
-        }
-    }
-
-    __syncthreads();
-    const long long base = s_base;
-    if (s_kept_total == 0) return;
-
-    // ---------------- phase 6: dense k/N (+ noise) of the kept TaxIDs, one warp per TaxID ----------------
-    uint32_t* dk = s_dense + (size_t)warp * 2 * R;
-    uint32_t* dN = dk + R;
-    for (int s = warp; s < nowned; s += kCountsWarps) {
-        if (!s_kept[s]) continue;
-        const long long o = base + (long long)s_rank[s];
-        if (o >= p.capacity) continue;
-        const int a = s_seg[s], b = s_seg[s + 1];
-        for (int i = lane; i < 2 * R; i += 32) dk[i] = 0;
-        __syncwarp();
-        for (int r = a + lane; r < b; r += 32) {
-            const int zabs = (int)s_pos[r] + 1;
-            if (zabs > P) continue;
-            const bool rev = s_rev[r] != 0;
-            const int slot = rev ? P + zabs - 1 : zabs - 1;
-            atomicAdd(&dk[slot], s_cnt[(size_t)(rev ? skr : skf) * cap + r]);
-            atomicAdd(&dN[slot], rev ? o_nr[r] : o_nf[r]);
-        }
-        __syncwarp();
-        if (p.out_k) for (int i = lane; i < R; i += 32) p.out_k[o * R + i] = dk[i];
-        if (p.out_N) for (int i = lane; i < R; i += 32) p.out_N[o * R + i] = dN[i];
-        if (lane == 0) {
-            if (p.out_tax) p.out_tax[o] = taxv[a];
-            if (p.out_nal) p.out_nal[o] = s_nal[a];
-            if (p.out_first) p.out_first[o] = row0 + a;
-        }
-        if (p.out_noise) {
-            // fits.py:359-376 over the TaxID's rows with |z| <= P: blank CT on forward rows and GA on
-            // reverse rows, divide every column by its nan-mean, nan-std over all / forward / reverse
-            const int OFF[12] = {1, 2, 3, 4, 6, 7, 8, 9, 11, 12, 13, 14};
-            double inv_mean[12];
-#pragma unroll
-            for (int c = 0; c < 12; ++c) {
-                double sm = 0.0, cn = 0.0;
-                const int slotc = p.col_slot[OFF[c]];
-                for (int r = a + lane; r < b; r += 32) {
-                    const int zabs = (int)s_pos[r] + 1;
-                    const bool rev = s_rev[r] != 0;
-                    const bool blank = (zabs > P) || (!rev && c == 5) || (rev && c == 6);
-                    if (!blank) { sm += (double)s_cnt[(size_t)slotc * cap + r]; cn += 1.0; }
-                }
-                sm = warp_sum_f64(sm); cn = warp_sum_f64(cn);
-                inv_mean[c] = (cn > 0.0 && sm > 0.0) ? cn / sm : nan("");
-            }
-            double s1[3] = {0, 0, 0}, n1[3] = {0, 0, 0};
-            for (int r = a + lane; r < b; r += 32) {
-                const int zabs = (int)s_pos[r] + 1;
-                const bool rev = s_rev[r] != 0;
-                if (zabs > P) continue;
-#pragma unroll
-                for (int c = 0; c < 12; ++c) {
-                    const bool blank = (!rev && c == 5) || (rev && c == 6);
-                    const double v = (double)s_cnt[(size_t)p.col_slot[OFF[c]] * cap + r] * inv_mean[c];
-                    if (!blank && !isnan(v)) { s1[0] += v; n1[0] += 1.0; s1[rev ? 2 : 1] += v; n1[rev ? 2 : 1] += 1.0; }
-                }
-            }
-            double mean3[3];
-#pragma unroll
-            for (int q = 0; q < 3; ++q) { s1[q] = warp_sum_f64(s1[q]); n1[q] = warp_sum_f64(n1[q]); mean3[q] = s1[q] / n1[q]; }
-            double s2[3] = {0, 0, 0};
-            for (int r = a + lane; r < b; r += 32) {
-                const int zabs = (int)s_pos[r] + 1;
-                const bool rev = s_rev[r] != 0;
-                if (zabs > P) continue;
-#pragma unroll
-                for (int c = 0; c < 12; ++c) {
-                    const bool blank = (!rev && c == 5) || (rev && c == 6);
-                    const double v = (double)s_cnt[(size_t)p.col_slot[OFF[c]] * cap + r] * inv_mean[c];
-                    if (!blank && !isnan(v)) {
-                        const double d0 = v - mean3[0], d1 = v - mean3[rev ? 2 : 1];
-                        s2[0] += d0 * d0; s2[rev ? 2 : 1] += d1 * d1;
-                    }
-                }
-            }
-#pragma unroll
-            for (int q = 0; q < 3; ++q) s2[q] = warp_sum_f64(s2[q]);
-            if (lane == 0) {
-#pragma unroll
-                for (int q = 0; q < 3; ++q) p.out_noise[o * 3 + q] = n1[q] > 0.0 ? sqrt(s2[q] / n1[q]) : nan("");
-            }
-        }
-        __syncwarp();
-    }
-}
-
-
 // ---------------------------------------------------------------------------------------------
-// K1b: exclusive scan of the per-tile kept counts (one CTA) -> final block starts and the total
+// exclusive scan of per-block counts (one CTA) -> final block starts and the total; K1d, K0 and K8
+// scan with it, K1 with the two-level form below
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(1024) counts_scan_kernel(const int* __restrict__ tile_cnt, long long n_tiles,
                                                            long long* __restrict__ final_base, long long* __restrict__ n_tax_out) {
@@ -580,7 +176,6 @@ struct CountsPermute {
     const long long* t_first; long long* out_first;
     const uint32_t* t_k; uint32_t* out_k;
     const uint32_t* t_N; uint32_t* out_N;
-    const double* t_noise; double* out_noise;
 };
 
 constexpr int kPermuteWarps = 4;
@@ -626,10 +221,6 @@ __global__ void __launch_bounds__(kPermuteWarps * 32, 8) counts_permute_kernel(c
         if (p.out_tax) p.out_tax[dst0 + j] = p.t_tax[s];
         if (p.out_nal) p.out_nal[dst0 + j] = p.t_nal[s];
         if (p.out_first) p.out_first[dst0 + j] = p.t_first[s];
-        if (p.out_noise) {
-#pragma unroll
-            for (int c = 0; c < 3; ++c) p.out_noise[(dst0 + j) * 3 + c] = p.t_noise[s * 3 + c];
-        }
     }
     const int R = p.R;
     for (int j0 = 0; j0 < total; j0 += 4) {

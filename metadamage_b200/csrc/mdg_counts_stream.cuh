@@ -1,9 +1,8 @@
-// mdg_counts_stream.cuh — K1, second design: warp-synchronous streaming counts_reduce.
+// mdg_counts_stream.cuh — K1 counts_stream_kernel: warp-synchronous streaming counts_reduce (counts.py:237-256 +
+// the dense extraction of fits.py:398-419), and the noise statistic of the kept TaxIDs (fits.py:359-376).
 //
-// Same outputs as counts_reduce_kernel (mdg_counts_kernel.cuh; counts.py:237-256 + the dense extraction of
-// fits.py:398-419), different structure. ncu on the tile kernel (profiles/r01_counts_ncu.md, r02_ncu_metrics.json):
-// 36 % DRAM utilisation, top stall `barrier` 3.4 warps per issue — seven CTA barriers per 448-row tile and a fixed
-// tile lifetime of ~6 us bound it, not HBM. Here NOTHING is shared between warps:
+// NOTHING is shared between warps: staged through shared memory in CTA-wide tiles, the same work is bound by CTA
+// barriers, not by HBM (profiles/r01_counts_ncu.md: 36 % DRAM utilisation, top stall `barrier`).
 //   * one warp owns 128 consecutive rows, four per lane, loaded straight into registers with 128-bit coalesced
 //     global loads (12 independent loads per lane in flight; no shared-memory staging, no TMA: the rows are used
 //     once) and written back with 128-bit stores;
@@ -11,9 +10,9 @@
 //     129-entry shared-memory table private to the warp; the only synchronisation is __syncwarp;
 //   * a warp owns every TaxID whose FIRST row is among its 128 rows; if its last TaxID runs past them it reads on,
 //     32 rows at a time (those rows are L2 hits: they are some other warp's own rows), up to MDG_MAX_SEGMENT_ROWS;
-//   * kept TaxIDs get their dense k/N row from the same registers; the order is restored by the same
-//     reserve-with-one-atomic / scan / block-permute triple as before;
-//   * the optional noise statistic (fits.py:359-376) moved to its own kernel over the kept TaxIDs.
+//   * kept TaxIDs get their dense k/N row from the same registers; the order is restored by the
+//     reserve-with-one-atomic / scan / block-permute triple of mdg_counts_kernel.cuh;
+//   * the optional noise statistic has its own kernel over the kept TaxIDs (counts_noise_kernel, below).
 #pragma once
 #include "mdg_counts_kernel.cuh"
 
@@ -56,7 +55,7 @@ __global__ void __launch_bounds__(kStreamWarps * 32, MDG_STREAM_MINBLOCKS) count
     bool rev[4], valid[4];
     const uint32_t* ca = p.counts16 + (long long)(p.fwd_ref * 4) * p.stride;
     const uint32_t* cb = p.counts16 + (long long)(p.rev_ref * 4) * p.stride;
-    if (p.use_tma && n_in == kStreamRows) {  // (`use_tma`: every column base is 16-byte aligned and stride % 4 == 0)
+    if (p.vec_in && n_in == kStreamRows) {
         const longlong2 t01 = *reinterpret_cast<const longlong2*>(p.tax_id + gi);
         const longlong2 t23 = *reinterpret_cast<const longlong2*>(p.tax_id + gi + 2);
         tax[0] = t01.x; tax[1] = t01.y; tax[2] = t23.x; tax[3] = t23.y;

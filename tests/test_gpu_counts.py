@@ -80,8 +80,9 @@ def ragged_input(rng, n_tax, max_rows, P):
 
 
 @pytest.mark.parametrize("max_rows,n_tax", [(1, 5000), (9, 4000), (70, 2000), (400, 300), (1500, 40)])
-def test_counts_ragged_segments_and_tile_ladder(ctx, oracle, max_rows, n_tax):
-    """Segment lengths from 1 to 1500 rows exercise the lookahead ladder (128 -> 512 -> 2048)."""
+def test_counts_ragged_segments(ctx, oracle, max_rows, n_tax):
+    """Segment lengths from 1 to 1500 rows: a TaxID that runs past its warp's 128 rows is read on, 32 rows at a
+    time, up to MDG_MAX_SEGMENT_ROWS."""
     rng = np.random.default_rng(max_rows)
     tax, nal, rev, pos, c16 = ragged_input(rng, n_tax, max_rows, 15)
     kw = dict(max_position=15, min_alignments=20, min_y_sum=5)

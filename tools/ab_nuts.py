@@ -1,5 +1,5 @@
-"""A/B of the NUTS kernels on the GPU box (development tool): fits `n` TaxIDs of BASELINE config 2 with the
-kernel selection given by the MDG_* environment variables and prints the CUDA-event times and leapfrog counts."""
+"""A/B of the NUTS kernels on the GPU box (development tool): fits `n` TaxIDs of BASELINE config 2 with the library
+MDG_LIB_PATH names (e.g. a build of tools/ab_build.sh) and prints the CUDA-event times and leapfrog counts."""
 import os
 import sys
 import time

@@ -3,7 +3,7 @@
     python tools/ncu_metrics.py nuts=gpurun_out/r2_nuts.ncu-rep counts=gpurun_out/r2_counts.ncu-rep > profiles/r02_ncu_metrics.json
 
 For every `name=report` the FIRST kernel of the report whose name contains the given key
-(`nuts` -> nuts_group_kernel, `counts` -> counts_reduce_kernel) is read with `ncu --page raw --csv`:
+(`nuts` -> nuts_group_kernel, `counts` -> counts_stream_kernel) is read with `ncu --page raw --csv`:
 DRAM bytes, duration, issue / pipe utilisation, instruction counts, stall ratios."""
 import csv
 import json

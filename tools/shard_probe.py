@@ -20,7 +20,7 @@ lo, hi = (spec.split("-") + [spec])[:2]
 args = argparse.Namespace(max_position=15, taxa_per_gpu=int(sys.argv[2]) if len(sys.argv) > 2 else 10000)
 ctx = Context(0)
 cfg = _lib.default_config()
-# scheduling variants (environment knobs of mdg_fit_batch), e.g. MDG_PROBE_VARIANTS="MDG_HOLD_AFTER=0;MDG_HOLD_AFTER=48000"
+# scheduling variants (environment knobs of mdg_fit_batch), e.g. MDG_PROBE_VARIANTS="MDG_NUTS_ORDER=0;MDG_NUTS_ORDER=2,MDG_NUTS_PRIO_FRAC=8"
 VARIANTS = [dict(kv.split("=") for kv in v.split(",") if kv) for v in os.environ.get("MDG_PROBE_VARIANTS", "").split(";")] or [{}]
 for rank in range(int(lo), int(hi) + 1):
     g = bench.workload(args, rank, 8)
