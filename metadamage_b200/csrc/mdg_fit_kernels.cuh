@@ -45,6 +45,7 @@ struct FitLaunch {
     unsigned long long* chain_clock;  // development (MDG_CHAIN_CLOCK): [n_tax][6][2] globaltimer at chain start / end, or NULL
 };
 
+// D-vectors: component j is written by lane j of the group only (the lane that holds it in registers)
 template <int D>
 struct GroupShared {
     double zl[D], rl[D], gl[D], zr[D], rr[D], gr[D];  // main tree edges
@@ -60,35 +61,40 @@ struct GroupShared {
     double da_x, da_xavg, da_gavg, da_prox, mean_accept, h_step, h_Er;
     double m_weight, m_sum_acc, m_pe_p, u_main, pe_cur, eps, s_pe_p;
     double m_rsum[D];
-    // group-uniform values that are live ACROSS the gradient evaluation but not used inside it:
-    // parked here so that the evaluation's five interleaved special-function chains get the registers
-    double imm[D], s_rsum[D], zn_park[D], rh_park[D], E0, s_weight, s_sum_acc;
+    // values that are live ACROSS the gradient evaluation but not used inside it: kept here so that the
+    // evaluation's five interleaved special-function chains get the registers
+    double imm[D], s_rsum[D], E0, s_weight, s_sum_acc;
     double isd[D];  // 1 / sqrt(imm) = sqrt of the mass matrix diagonal (momentum r ~ N(0, M) is n * isd)
     int da_t, wf_n, window_idx, h_last, h_dir, m_nprop;
     uint32_t h_att, h_call, init_attempt, n_div;
 };
 
 
-template <int D>
-__device__ __forceinline__ double kinetic(const double (&imm)[D], const double (&r)[D]) {
-    double e = 0.0;
+// The dot products of K4 over a chain's D-vectors, held one component per lane (lane j < D of the GW-lane group
+// holds component j). The terms are added in the order j = 0, 1, ..., D-1 of a serial loop: lane j adds its own
+// term to the partial sum lane j - 1 passes up, so lane D - 1 ends with the sum, bit for bit the serial one.
+
+// r^T M^-1 r / 2 (diagonal M^-1 = imm)
+template <int D, int GW>
+__device__ __forceinline__ double kinetic(double imm, double r, unsigned gmask) {
+    double e = fma(imm * r, r, 0.0);
 #pragma unroll
-    for (int j = 0; j < D; ++j) e = fma(imm[j] * r[j], r[j], e);
-    return 0.5 * e;
+    for (int j = 1; j < D; ++j) e = fma(imm * r, r, __shfl_up_sync(gmask, e, 1, GW));
+    return 0.5 * __shfl_sync(gmask, e, D - 1, GW);
 }
 
 // generalised U-turn test (hmc_util._is_turning, diagonal mass matrix)
-template <int D>
-__device__ __forceinline__ bool is_turning(const double (&imm)[D], const double* r_left, const double* r_right,
-                                           const double* r_sum) {
-    double dl = 0.0, dr = 0.0;
+template <int D, int GW>
+__device__ __forceinline__ bool is_turning(double imm, double r_left, double r_right, double r_sum, unsigned gmask) {
+    const double rho = r_sum - (r_left + r_right) / 2;
+    const double tl = imm * r_left * rho, tr = imm * r_right * rho;
+    double dl = 0.0 + tl, dr = 0.0 + tr;
 #pragma unroll
-    for (int j = 0; j < D; ++j) {
-        double rho = r_sum[j] - (r_left[j] + r_right[j]) / 2;
-        dl += imm[j] * r_left[j] * rho;
-        dr += imm[j] * r_right[j] * rho;
+    for (int j = 1; j < D; ++j) {
+        dl = __shfl_up_sync(gmask, dl, 1, GW) + tl;
+        dr = __shfl_up_sync(gmask, dr, 1, GW) + tr;
     }
-    return (dl <= 0.0) || (dr <= 0.0);
+    return __shfl_sync(gmask, (int)((dl <= 0.0) || (dr <= 0.0)), D - 1, GW) != 0;
 }
 
 struct Vec4 { double v[4]; };

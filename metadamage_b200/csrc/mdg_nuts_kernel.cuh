@@ -32,22 +32,14 @@
 namespace mdg {
 
 // momentum r ~ N(0, M), M^-1 = diag(imm): r_j = n_j * isd_j with isd = 1 / sqrt(imm) kept per chain (it changes at
-// the four adaptation-window ends only). The D standard normals are drawn ACROSS the lanes: lane j < D evaluates the
-// Philox block j / 2 and keeps component j % 2 of its Box-Muller pair (one Philox + one Box-Muller in the
-// instruction stream instead of two of each), then the values are broadcast.
+// the four adaptation-window ends only). The D standard normals are drawn ACROSS the lanes: the lane that owns
+// component j evaluates the Philox block j / 2 and keeps component j % 2 of its Box-Muller pair (one Philox + one
+// Box-Muller in the instruction stream instead of two of each).
 template <int D>
-__device__ MDG_COLD double draw_normal_lane_cold(uint2 key, uint32_t c1, uint32_t c2, uint32_t c3, int lig) {
+__device__ MDG_COLD double draw_normal_lane_cold(uint2 key, uint32_t c1, uint32_t c2, uint32_t c3, int j) {
     double n0, n1;
-    normal2(philox4x32(key, (uint32_t)((lig >> 1) & ((D + 1) / 2 - 1)), c1, c2, c3), n0, n1);
-    return (lig & 1) ? n1 : n0;
-}
-
-template <int D, int GW>
-__device__ __forceinline__ void draw_momentum_scaled(uint2 key, uint32_t c1, uint32_t c2, uint32_t c3, const double (&isd)[D],
-                                                     int lig, unsigned gmask, double (&r)[D]) {
-    const double mine = draw_normal_lane_cold<D>(key, c1, c2, c3, lig);
-#pragma unroll
-    for (int j = 0; j < D; ++j) r[j] = __shfl_sync(gmask, mine, j, GW) * isd[j];
+    normal2(philox4x32(key, (uint32_t)((j >> 1) & ((D + 1) / 2 - 1)), c1, c2, c3), n0, n1);
+    return (j & 1) ? n1 : n0;
 }
 
 // The five lgamma/digamma evaluations of one PMD position, x = {k + alpha, N - k + beta, N + phi, alpha, beta}
@@ -100,6 +92,17 @@ __device__ __forceinline__ void pmd_special(const double (&x)[5], double& d14, d
 }
 
 enum GroupPhase : int { GP_FETCH = 0, GP_INIT = 1, GP_HEUR = 2, GP_LEAF = 3, GP_IDLE = 4 };
+// What a leapfrog's bookkeeping leaves for the end of the trip, where each of these routines exists once (inlined at
+// every place that wants it, they made the kernel outgrow the instruction cache). Each step falls through to the
+// next one as far as it has to: a heuristic search that ends starts a transition, a transition starts a doubling.
+enum PendingStep : int {
+    PS_NONE = 0,
+    PS_HEUR_BEGIN = 1,  // start the step-size search (hmc_util.find_reasonable_step_size) at eps
+    PS_HEUR = 2,        // its next trial, or its end: eps = the step found, reset dual averaging, start a transition
+    PS_RESET = 3,       // reset dual averaging, then start a transition
+    PS_TRANSITION = 4,  // begin a transition from the chain state held in sh.zp / sh.gp / pe_cur
+    PS_DOUBLING = 5     // start one tree doubling: pick direction, aim the next leapfrog at the chosen edge
+};
 
 // bytes of dynamic shared memory per warp: {k, N} as doubles + four log-likelihood buffers, [n_slots][32] each
 __host__ __device__ constexpr size_t nuts_warp_smem_bytes(int n_slots) { return (size_t)n_slots * 32 * (16 + 4 * 8); }
@@ -118,16 +121,14 @@ enum : int { LL_X = 0, LL_SUB = 1, LL_MAIN = 2, LL_CUR = 3 };
 
 // K2: log p(y | theta(u)) + log prior(theta(u)) + log |d theta / d u| and its gradient for the chain of one
 // group; writes the per-position log-likelihood (without log C(N,k)) of every linear index to `llw`.
+// `myu` and `grad` are the lane's component jc of u and of the gradient (the layout of nuts_group_kernel).
 template <int MODEL, int GW>
 __device__ __forceinline__ void eval_group(const double2* __restrict__ kn, double* __restrict__ llw, int n_slots, int lane,
-                                           int lig, unsigned gmask, int P, int mask, int n_obs,
-                                           const double (&u)[ModelDim<MODEL>::value], const double2* __restrict__ ptab,
-                                           double phi_min, double& logp, double (&grad)[ModelDim<MODEL>::value], bool& valid) {
+                                           int lig, int jc, unsigned gmask, int P, int mask, int n_obs, double myu,
+                                           const double2* __restrict__ ptab, double phi_min, double& logp, double& grad,
+                                           bool& valid) {
     constexpr int D = ModelDim<MODEL>::value;
     // --- group-uniform transforms, one parameter per lane, then broadcast (mdg_model.cuh eval_model) ---
-    double myu = u[0];
-#pragma unroll
-    for (int j = 1; j < D; ++j) myu = (lig == j) ? u[j] : myu;
     const bool in_range = fabs(myu) < 700.0;  // false for NaN
     const double E = exp_core(lig == D - 1 ? myu : -fabs(myu));
     const double l1p = log_pos(1.0 + E);
@@ -214,23 +215,21 @@ __device__ __forceinline__ void eval_group(const double2* __restrict__ kn, doubl
         s_dDw = group_sum<GW>(s_dDw, gmask);
         s_dDxw = group_sum<GW>(s_dDxw, gmask);
     }
-    const bool any_bad = (__ballot_sync(gmask, bad) & gmask) != 0u;
 
-    // --- chain rule to the unconstrained parameters ---------------------------------------------------
+    // --- chain rule to the unconstrained parameters: component jc of the gradient ---------------------
     logp = s_ll;
+    double dlogp_dtheta, dtheta_du;
     if (MODEL == 0) {
-        grad[0] = fma(-A * q, s_dDxw, __shfl_sync(gmask, gp_lane, 0, GW));
-        grad[1] = fma(A * (1.0 - A), s_dDw, __shfl_sync(gmask, gp_lane, 1, GW));
-        grad[2] = fma(c * (1.0 - c), s_dD, __shfl_sync(gmask, gp_lane, 2, GW));
-        grad[3] = fma(delta, s_dphi, __shfl_sync(gmask, gp_lane, 3, GW));
+        dtheta_du = jc == 0 ? -A * q : (jc == 1 ? A * (1.0 - A) : (jc == 2 ? c * (1.0 - c) : delta));
+        dlogp_dtheta = jc == 0 ? s_dDxw : (jc == 1 ? s_dDw : (jc == 2 ? s_dD : s_dphi));
     } else {
-        grad[0] = fma(q * (1.0 - q), s_dD, __shfl_sync(gmask, gp_lane, 0, GW));
-        grad[1] = fma(delta, s_dphi, __shfl_sync(gmask, gp_lane, 1, GW));
+        dtheta_du = jc == 0 ? q * (1.0 - q) : delta;
+        dlogp_dtheta = jc == 0 ? s_dD : s_dphi;
     }
-    bool fin = isfinite(logp);
-#pragma unroll
-    for (int j = 0; j < D; ++j) fin = fin && isfinite(grad[j]);
-    valid = fin && !any_bad;
+    grad = fma(dtheta_du, dlogp_dtheta, __shfl_sync(gmask, gp_lane, jc, GW));
+    // a lane >= D mirrors component 0, so a vote over the whole group sees every component once
+    const bool any_bad = (__ballot_sync(gmask, bad || !isfinite(grad)) & gmask) != 0u;
+    valid = isfinite(logp) && !any_bad;
 }
 
 #ifndef MDG_NUTS_MINBLOCKS
@@ -240,12 +239,18 @@ template <int MODEL, int GW, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nuts_group_kernel(const FitLaunch p) {
     constexpr int D = ModelDim<MODEL>::value;
     constexpr int GROUPS = 32 / GW;
+    // one lane per component (the lane-order sums of kinetic / is_turning) and one per trace column
+    static_assert(GW >= D && GW >= 4, "a group needs a lane for each of the D parameters and each of the 4 trace columns");
     __shared__ GroupShared<D> sh_all[WARPS * GROUPS];
     __shared__ double2 sh_prior[64];
     extern __shared__ __align__(16) unsigned char sh_dyn[];
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int grp = lane / GW, lig = lane % GW;
+    // The chain's D-vectors are held one component per lane: lane lig < D of the group owns component lig; a lane
+    // lig >= D mirrors component 0 (the evaluation needs a valid parameter on every lane) and never stores it.
+    const bool own = lig < D;
+    const int jc = own ? lig : 0;
     const unsigned gmask = group_mask<GW>();
     GroupShared<D>& sh = sh_all[warp * GROUPS + grp];
     const int NS = p.n_slots;
@@ -281,98 +286,31 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
     int s_nprop = 0;
     bool s_div = false;
     uint32_t leaf_counter = 0;
-    double zf[D], rf[D], gf[D], e = 0.0;  // leapfrog source
+    double zf = 0.0, rf = 0.0, gf = 0.0, e = 0.0;  // leapfrog source (component jc)
     int t = 0;
-#pragma unroll
-    for (int j = 0; j < D; ++j) { zf[j] = 0.0; rf[j] = 0.0; gf[j] = 0.0; }
 
-    // ---- cold chain state: references into shared memory (single writer or all lanes writing the same
-    // value at a converged point; reads are broadcasts) ----
-    double (&imm)[D] = sh.imm;
-    double& E0 = sh.E0; double (&s_rsum)[D] = sh.s_rsum; double& s_weight = sh.s_weight; double& s_sum_acc = sh.s_sum_acc;
+    // ---- cold chain state: references into shared memory (scalars: single writer or all lanes writing the same
+    // value at a converged point, reads are broadcasts; D-vectors: lane j < D writes component j) ----
+    double& E0 = sh.E0; double& s_weight = sh.s_weight; double& s_sum_acc = sh.s_sum_acc;
     double& eps = sh.eps; double& pe_cur = sh.pe_cur;
     double& da_x = sh.da_x; double& da_xavg = sh.da_xavg; double& da_gavg = sh.da_gavg; double& da_prox = sh.da_prox;
     int& da_t = sh.da_t; int& wf_n = sh.wf_n; int& window_idx = sh.window_idx;
     double& mean_accept = sh.mean_accept; uint32_t& n_div = sh.n_div;
     double& m_weight = sh.m_weight; double& m_sum_acc = sh.m_sum_acc; double& m_pe_p = sh.m_pe_p; double& u_main = sh.u_main;
-    double (&m_rsum)[D] = sh.m_rsum; int& m_nprop = sh.m_nprop; double& s_pe_p = sh.s_pe_p;
+    int& m_nprop = sh.m_nprop; double& s_pe_p = sh.s_pe_p;
     double& h_step = sh.h_step; double& h_Er = sh.h_Er; int& h_last = sh.h_last; int& h_dir = sh.h_dir;
     uint32_t& h_att = sh.h_att; uint32_t& h_call = sh.h_call; uint32_t& init_attempt = sh.init_attempt;
 
     auto init_candidate = [&]() {
-#pragma unroll
-        for (int b = 0; b < (D + 1) / 2; ++b) {
-            double u0, u1;
-            uniform2(philox4x32(key, (uint32_t)b, init_attempt, c2word(run_kind, P_INIT), 0u), u0, u1);
-            zf[2 * b] = p.cfg.init_radius * (2.0 * u0 - 1.0);
-            if (2 * b + 1 < D) zf[2 * b + 1] = p.cfg.init_radius * (2.0 * u1 - 1.0);
-        }
-#pragma unroll
-        for (int j = 0; j < D; ++j) { rf[j] = 0.0; gf[j] = 0.0; }
+        // component j is the (j % 2)-th uniform of the Philox block j / 2
+        double u0, u1;
+        uniform2(philox4x32(key, (uint32_t)(jc >> 1), init_attempt, c2word(run_kind, P_INIT), 0u), u0, u1);
+        zf = p.cfg.init_radius * (2.0 * ((jc & 1) ? u1 : u0) - 1.0);
+        rf = 0.0; gf = 0.0;
         e = 0.0;
         phase = GP_INIT;
     };
 
-    // start one tree doubling: pick direction, aim the next leapfrog at the chosen edge
-    auto start_doubling = [&]() {
-        double u_dir;
-        uniform2(philox4x32(key, (uint32_t)m_depth, (uint32_t)t, c2word(run_kind, P_DIR), 0u), u_dir, u_main);
-        going_right = u_dir < 0.5;
-        s_nprop = 0;
-        __syncwarp(gmask);
-#pragma unroll
-        for (int j = 0; j < D; ++j) {
-            zf[j] = going_right ? sh.zr[j] : sh.zl[j];
-            rf[j] = going_right ? sh.rr[j] : sh.rl[j];
-            gf[j] = going_right ? sh.gr[j] : sh.gl[j];
-        }
-        e = going_right ? eps : -eps;
-        phase = GP_LEAF;
-    };
-
-    // begin a transition from the chain state held in sh.zp / sh.gp / pe_cur
-    auto start_transition = [&]() {
-        double r0[D];
-        draw_momentum_scaled<D, GW>(key, (uint32_t)t, c2word(run_kind, P_MOM), 0u, sh.isd, lig, gmask, r0);
-        E0 = pe_cur + kinetic<D>(imm, r0);
-        __syncwarp(gmask);
-        if (lig == 0) {
-#pragma unroll
-            for (int j = 0; j < D; ++j) {
-                double zj = sh.zp[j], gj = sh.gp[j];
-                sh.zl[j] = zj; sh.zr[j] = zj; sh.gl[j] = gj; sh.gr[j] = gj;
-                sh.rl[j] = r0[j]; sh.rr[j] = r0[j];
-            }
-        }
-#pragma unroll
-        for (int j = 0; j < D; ++j) m_rsum[j] = r0[j];
-        m_weight = 0.0; m_sum_acc = 0.0; m_nprop = 0; m_depth = 0; m_turning = false; m_div = false;
-        m_pe_p = pe_cur;
-        m_is_c = true;  // the tree's proposal is the current state until a subtree's proposal is taken
-        leaf_counter = 0;
-        start_doubling();
-    };
-
-    // heuristic step-size search (hmc_util.find_reasonable_step_size): next trial or finish
-    auto heur_try = [&]() -> bool {
-        bool small_ok = (h_step > 2.2250738585072014e-308) || (h_dir >= 0);
-        bool large_ok = (h_step < 1.7976931348623157e308) || (h_dir <= 0);
-        if (!(small_ok && large_ok && (h_last == 0 || h_dir == h_last))) return false;
-        h_step *= (h_dir > 0 ? 2.0 : (h_dir < 0 ? 0.5 : 1.0));
-        draw_momentum_scaled<D, GW>(key, h_call, c2word(run_kind, P_HEUR), h_att, sh.isd, lig, gmask, rf);
-        ++h_att;
-        h_Er = kinetic<D>(imm, rf) + pe_cur;
-        __syncwarp(gmask);
-#pragma unroll
-        for (int j = 0; j < D; ++j) { zf[j] = sh.zp[j]; gf[j] = sh.gp[j]; }
-        e = h_step;
-        phase = GP_HEUR;
-        return true;
-    };
-    auto begin_heuristic = [&]() -> bool {
-        h_step = eps; h_last = 0; h_dir = 0; h_att = 0;
-        return heur_try();
-    };
     auto reset_dual_averaging = [&]() {
         da_x = 0.0; da_xavg = 0.0; da_gavg = 0.0; da_t = 0; da_prox = log_cold(10.0 * eps);
     };
@@ -417,8 +355,7 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                 n_grad = 0; failed = 0; m_depth = 0; m_turning = false; m_div = false; going_right = true;
                 s_nprop = 0; s_div = false; leaf_counter = 0; t = 0;
                 __syncwarp(gmask);
-#pragma unroll
-                for (int j = 0; j < D; ++j) { imm[j] = 1.0; sh.isd[j] = 1.0; }
+                if (own) { sh.imm[lig] = 1.0; sh.isd[lig] = 1.0; sh.wf_mean[lig] = 0.0; sh.wf_m2[lig] = 0.0; }
                 E0 = 0.0; s_weight = 0.0; s_sum_acc = 0.0;
                 eps = p.cfg.init_step_size; pe_cur = 0.0;
                 da_x = 0.0; da_xavg = 0.0; da_gavg = 0.0; da_prox = 0.0; da_t = 0; wf_n = 0; window_idx = 0;
@@ -426,8 +363,6 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                 m_weight = 0.0; m_sum_acc = 0.0; m_pe_p = 0.0; u_main = 0.0; m_nprop = 0; s_pe_p = 0.0;
                 h_step = 0.0; h_Er = 0.0; h_last = 0; h_dir = 0; h_att = 0u; h_call = 0u; init_attempt = 0u;
                 if (lig == 0) {
-#pragma unroll
-                    for (int j = 0; j < D; ++j) { sh.wf_mean[j] = 0.0; sh.wf_m2[j] = 0.0; }
 #pragma unroll
                     for (int j = 0; j < 5; ++j) { sh.acc_mean[j] = 0.0; sh.acc_m2[j] = 0.0; }
                 }
@@ -441,25 +376,18 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
         // =========================== one leapfrog ===========================
         bool done = false;
         {
-            double zn[D], rn[D], gn[D], pen;
-            double rh[D];
-#pragma unroll
-            for (int j = 0; j < D; ++j) { rh[j] = fma(-0.5 * e, gf[j], rf[j]); zn[j] = fma(e * imm[j], rh[j], zf[j]); }
-            double logp, grad[D];
+            int pend = PS_NONE;
+            const double imm = sh.imm[jc];
+            const double rh = fma(-0.5 * e, gf, rf);
+            const double zn = fma(e * imm, rh, zf);
+            double logp, grad;
             bool valid;
-            // group-uniform values that are live across the evaluation but not used inside it are parked in
-            // shared memory: the evaluation's interleaved special-function chains get the registers
-#pragma unroll
-            for (int j = 0; j < D; ++j) { sh.zn_park[j] = zn[j]; sh.rh_park[j] = rh[j]; }
-            eval_group<MODEL, GW>(kn, llb + (size_t)roles.get(LL_X) * wstride, ns, lane, lig, gmask, P, mask, n_obs, zn, sh_prior,
+            eval_group<MODEL, GW>(kn, llb + (size_t)roles.get(LL_X) * wstride, ns, lane, lig, jc, gmask, P, mask, n_obs, zn, sh_prior,
                                   phi_min, logp, grad, valid);
-            __syncwarp(gmask);
-#pragma unroll
-            for (int j = 0; j < D; ++j) { zn[j] = sh.zn_park[j]; rh[j] = sh.rh_park[j]; }
             ++n_grad;
-            pen = valid ? -logp : nan("");
-#pragma unroll
-            for (int j = 0; j < D; ++j) { gn[j] = valid ? -grad[j] : nan(""); rn[j] = fma(-0.5 * e, gn[j], rh[j]); }
+            const double pen = valid ? -logp : nan("");
+            const double gn = valid ? -grad : nan("");
+            const double rn = fma(-0.5 * e, gn, rh);
 
             if (budget != 0u && n_grad > budget) {
                 // bounded work per run: the analogue of the reference's per-fit timeout (fits.py:472-474)
@@ -467,19 +395,19 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                 done = true;
             } else if (phase == GP_LEAF) {
                 // ---- hmc_util._build_basetree ----
-                double dE = pen + kinetic<D>(imm, rn) - E0;
+                double dE = pen + kinetic<D, GW>(sh.imm[jc], rn, gmask) - E0;
                 if (isnan(dE)) dE = INFINITY;
                 const double leaf_w = -dE;
                 const bool leaf_div = dE > p.cfg.max_delta_energy;
                 const double leaf_acc = dE <= 0.0 ? 1.0 : exp_nonpos(-dE);  // min(1, e^-dE); dE is never NaN here
                 const int leaf_idx = s_nprop;
                 bool take;
+                double s_rsum;  // component jc of the subtree's momentum sum
                 if (leaf_idx == 0) {
                     take = true;
                     s_weight = leaf_w;
                     s_sum_acc = leaf_acc;
-#pragma unroll
-                    for (int j = 0; j < D; ++j) s_rsum[j] = rn[j];
+                    s_rsum = rn;
                 } else {
                     // ---- _combine_tree(..., biased_transition=False) ----
                     double us, unused;
@@ -492,8 +420,7 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                     take = us < prob;  // NaN -> false
                     s_weight = isnan(dlt) ? -INFINITY : fmax(s_weight, leaf_w) + log_pos(1.0 + ed);
                     s_sum_acc += leaf_acc;
-#pragma unroll
-                    for (int j = 0; j < D; ++j) s_rsum[j] += rn[j];
+                    s_rsum = sh.s_rsum[jc] + rn;
                 }
                 s_div = leaf_div;
                 s_nprop = leaf_idx + 1;
@@ -507,31 +434,23 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                 const int n_trail = __ffs(~(unsigned)leaf_idx) - 1;
                 const int idx_min = idx_max - n_trail + 1;
                 __syncwarp(gmask);
-                if (lig == 0) {
-                    if (take) {
-#pragma unroll
-                        for (int j = 0; j < D; ++j) { sh.szp[j] = zn[j]; sh.sgp[j] = gn[j]; }
-                    }
-                    if ((leaf_idx & 1) == 0) {
-#pragma unroll
-                        for (int j = 0; j < D; ++j) { sh.rck[idx_max][j] = rn[j]; sh.rsck[idx_max][j] = s_rsum[j]; }
-                    }
+                if (own) {
+                    sh.s_rsum[lig] = s_rsum;
+                    if (take) { sh.szp[lig] = zn; sh.sgp[lig] = gn; }
+                    if ((leaf_idx & 1) == 0) { sh.rck[idx_max][lig] = rn; sh.rsck[idx_max][lig] = s_rsum; }
                 }
                 __syncwarp(gmask);
                 bool turning = false;
                 if (leaf_idx & 1) {
                     // ---- _is_iterative_turning ----
                     for (int i = idx_max; i >= idx_min && !turning; --i) {
-                        double sub[D], rc[D];
-#pragma unroll
-                        for (int j = 0; j < D; ++j) { rc[j] = sh.rck[i][j]; sub[j] = s_rsum[j] - sh.rsck[i][j] + rc[j]; }
-                        turning = is_turning<D>(imm, rc, rn, sub);
+                        const double rc = sh.rck[i][jc];
+                        turning = is_turning<D, GW>(sh.imm[jc], rc, rn, s_rsum - sh.rsck[i][jc] + rc, gmask);
                     }
                 }
                 if (s_nprop < (1 << m_depth) && !turning && !s_div) {
                     // keep extending the subtree from the leaf just built
-#pragma unroll
-                    for (int j = 0; j < D; ++j) { zf[j] = zn[j]; rf[j] = rn[j]; gf[j] = gn[j]; }
+                    zf = zn; rf = rn; gf = gn;
                 } else {
                     // ---- subtree finished: _combine_tree(..., biased_transition=True) ----
                     const double dlt_m = s_weight - m_weight;
@@ -540,25 +459,16 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                     const double em = exp_nonpos(-fabs(dlt_m));
                     const double prob = (turning || s_div) ? 0.0 : (dlt_m >= 0.0 ? 1.0 : em);
                     const bool take_main = u_main < prob;
+                    const double m_rsum = sh.m_rsum[jc] + s_rsum;
                     __syncwarp(gmask);
-                    if (lig == 0) {
-#pragma unroll
-                        for (int j = 0; j < D; ++j) {
-                            if (going_right) { sh.zr[j] = zn[j]; sh.rr[j] = rn[j]; sh.gr[j] = gn[j]; }
-                            else { sh.zl[j] = zn[j]; sh.rl[j] = rn[j]; sh.gl[j] = gn[j]; }
-                            if (take_main) { sh.zp[j] = sh.szp[j]; sh.gp[j] = sh.sgp[j]; }
-                        }
+                    if (own) {
+                        if (going_right) { sh.zr[lig] = zn; sh.rr[lig] = rn; sh.gr[lig] = gn; }
+                        else { sh.zl[lig] = zn; sh.rl[lig] = rn; sh.gl[lig] = gn; }
+                        if (take_main) { sh.zp[lig] = sh.szp[lig]; sh.gp[lig] = sh.sgp[lig]; }
+                        sh.m_rsum[lig] = m_rsum;
                     }
-                    __syncwarp(gmask);  // lane 0 is back before anybody touches group-uniform state again
-#pragma unroll
-                    for (int j = 0; j < D; ++j) m_rsum[j] += s_rsum[j];
-                    __syncwarp(gmask);
-                    {
-                        double rl[D], rr[D];
-#pragma unroll
-                        for (int j = 0; j < D; ++j) { rl[j] = sh.rl[j]; rr[j] = sh.rr[j]; }
-                        m_turning = turning || is_turning<D>(imm, rl, rr, m_rsum);
-                    }
+                    __syncwarp(gmask);  // the owners are back before anybody reads the tree edges
+                    m_turning = turning || is_turning<D, GW>(sh.imm[jc], sh.rl[jc], sh.rr[jc], m_rsum, gmask);
                     if (take_main) {
                         m_pe_p = s_pe_p;
                         roles.swap(LL_SUB, LL_MAIN);
@@ -571,16 +481,14 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                     m_sum_acc += s_sum_acc;
                     m_nprop += s_nprop;
                     if (m_depth < max_depth && !m_turning && !m_div) {
-                        start_doubling();
+                        pend = PS_DOUBLING;
                     } else {
                         // ================= transition finished (hmc.py sample_kernel) =================
                         const double accept_prob = m_sum_acc * rcp_pos((double)m_nprop);
                         pe_cur = m_pe_p;
                         if (!m_is_c) roles.swap(LL_MAIN, LL_CUR);
                         __syncwarp(gmask);
-                        double zc[D];
-#pragma unroll
-                        for (int j = 0; j < D; ++j) zc[j] = sh.zp[j];
+                        const double zc = sh.zp[jc];
                         bool want_heur = false;
                         if (t < W) {
                             // ---- warmup_adapter.update_fn ----
@@ -598,15 +506,12 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                             const bool is_middle = (0 < window_idx) && (window_idx < p.n_windows - 1);
                             if (is_middle) {
                                 wf_n += 1;
-                                if (lig == 0) {
+                                if (own) {
                                     const double inv_wf = rcp_pos((double)wf_n);
-#pragma unroll
-                                    for (int j = 0; j < D; ++j) {
-                                        double dpre = zc[j] - sh.wf_mean[j];
-                                        double mn = sh.wf_mean[j] + dpre * inv_wf;
-                                        sh.wf_mean[j] = mn;
-                                        sh.wf_m2[j] += dpre * (zc[j] - mn);
-                                    }
+                                    const double dpre = zc - sh.wf_mean[lig];
+                                    const double mn = sh.wf_mean[lig] + dpre * inv_wf;
+                                    sh.wf_mean[lig] = mn;
+                                    sh.wf_m2[lig] += dpre * (zc - mn);
                                 }
                                 __syncwarp(gmask);
                             }
@@ -615,17 +520,12 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                             if (at_end) window_idx += 1;
                             if (at_end && is_middle) {
                                 __syncwarp(gmask);
-#pragma unroll
-                                for (int j = 0; j < D; ++j) {
-                                    double cov = sh.wf_m2[j] / (wf_n - 1);
+                                if (own) {
+                                    const double cov = sh.wf_m2[lig] / (wf_n - 1);
                                     const double v = ((double)wf_n / (wf_n + 5.0)) * cov + 1e-3 * (5.0 / (wf_n + 5.0));
-                                    imm[j] = v;
-                                    sh.isd[j] = 1.0 / sqrt(v);
-                                }
-                                __syncwarp(gmask);
-                                if (lig == 0) {
-#pragma unroll
-                                    for (int j = 0; j < D; ++j) { sh.wf_mean[j] = 0.0; sh.wf_m2[j] = 0.0; }
+                                    sh.imm[lig] = v;
+                                    sh.isd[lig] = 1.0 / sqrt(v);
+                                    sh.wf_mean[lig] = 0.0; sh.wf_m2[lig] = 0.0;
                                 }
                                 __syncwarp(gmask);
                                 wf_n = 0;
@@ -641,9 +541,7 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                             // constrained draw (q, A, c, phi): lane j < D transforms parameter j, then a broadcast
                             double th[4];
                             {
-                                double myu = zc[0];
-#pragma unroll
-                                for (int j = 1; j < D; ++j) myu = (lig == j) ? zc[j] : myu;
+                                const double myu = zc;
                                 const double Ev = exp_fast(lig == D - 1 ? myu : -fabs(myu));
                                 const double iv = rcp_pos(1.0 + Ev);
                                 const double val = (lig == D - 1) ? Ev + p.pr.phi_min : (myu >= 0.0 ? iv : Ev * iv);
@@ -686,63 +584,103 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                                 wacc[2 * wstride + s * 32] = wmean; wacc[3 * wstride + s * 32] = wm2;
                             }
                         }
-                        if (p.trace != nullptr && lig == 0) {
-                            double* dst = p.trace + (((size_t)tax * MDG_NUM_RUNS + run_kind) * (W + S) + t) * 4;
-#pragma unroll
-                            for (int j = 0; j < 4; ++j) dst[j] = j < D ? zc[j] : nan("");
-                        }
+                        if (p.trace != nullptr && lig < 4)
+                            p.trace[(((size_t)tax * MDG_NUM_RUNS + run_kind) * (W + S) + t) * 4 + lig] = own ? zc : nan("");
                         __syncwarp(gmask);
                         t += 1;
                         if (t >= W + S) {
                             done = true;
+                        } else if (want_heur) {
+                            ++h_call;
+                            pend = PS_HEUR_BEGIN;
                         } else {
-                            bool heur_running = false;
-                            if (want_heur) {
-                                ++h_call;
-                                heur_running = begin_heuristic();
-                                if (!heur_running) { eps = h_step; reset_dual_averaging(); }
-                            }
-                            if (!heur_running) start_transition();
+                            pend = PS_TRANSITION;
                         }
                     }
                 }
             } else if (phase == GP_HEUR) {
-                const double delta = (kinetic<D>(imm, rn) + pen) - h_Er;
+                const double delta = (kinetic<D, GW>(sh.imm[jc], rn, gmask) + pen) - h_Er;
                 const int dir_new = (log_target_heur < -delta) ? 1 : -1;  // NaN -> -1
                 h_last = h_dir;
                 h_dir = dir_new;
-                if (!heur_try()) {
-                    eps = h_step;
-                    reset_dual_averaging();
-                    start_transition();
-                }
+                pend = PS_HEUR;
             } else {
                 // ---- GP_INIT: init_to_uniform(radius), retried until finite ----
                 if (valid) {
                     pe_cur = pen;
                     roles.swap(LL_X, LL_CUR);
                     __syncwarp(gmask);
-                    if (lig == 0) {
-#pragma unroll
-                        for (int j = 0; j < D; ++j) { sh.zp[j] = zn[j]; sh.gp[j] = gn[j]; }
-                    }
+                    if (own) { sh.zp[lig] = zn; sh.gp[lig] = gn; }
                     __syncwarp(gmask);
                     if (W + S == 0) {
                         done = true;
+                    } else if (p.cfg.find_heuristic_step_size && W > 0) {
+                        h_call = 0;
+                        pend = PS_HEUR_BEGIN;
                     } else {
-                        bool heur_running = false;
-                        if (p.cfg.find_heuristic_step_size && W > 0) {
-                            h_call = 0;
-                            heur_running = begin_heuristic();
-                            if (!heur_running) eps = h_step;
-                        }
-                        if (!heur_running) { reset_dual_averaging(); start_transition(); }
+                        pend = PS_RESET;
                     }
                 } else {
                     ++init_attempt;
                     if (init_attempt >= 100u) { failed = 1; done = true; }
                     else init_candidate();
                 }
+            }
+
+            // ---- what the bookkeeping asked for: aim the next leapfrog ----
+            if (pend == PS_HEUR_BEGIN) {
+                h_step = eps; h_last = 0; h_dir = 0; h_att = 0;
+                pend = PS_HEUR;
+            }
+            if (pend == PS_HEUR) {
+                const bool small_ok = (h_step > 2.2250738585072014e-308) || (h_dir >= 0);
+                const bool large_ok = (h_step < 1.7976931348623157e308) || (h_dir <= 0);
+                if (small_ok && large_ok && (h_last == 0 || h_dir == h_last)) {
+                    // next trial
+                    h_step *= (h_dir > 0 ? 2.0 : (h_dir < 0 ? 0.5 : 1.0));
+                    rf = draw_normal_lane_cold<D>(key, h_call, c2word(run_kind, P_HEUR), h_att, jc) * sh.isd[jc];
+                    ++h_att;
+                    h_Er = kinetic<D, GW>(sh.imm[jc], rf, gmask) + pe_cur;
+                    __syncwarp(gmask);
+                    zf = sh.zp[jc]; gf = sh.gp[jc];
+                    e = h_step;
+                    phase = GP_HEUR;
+                } else {
+                    eps = h_step;
+                    pend = PS_RESET;
+                }
+            }
+            if (pend == PS_RESET) {
+                reset_dual_averaging();
+                pend = PS_TRANSITION;
+            }
+            if (pend == PS_TRANSITION) {
+                const double r0 = draw_normal_lane_cold<D>(key, (uint32_t)t, c2word(run_kind, P_MOM), 0u, jc) * sh.isd[jc];
+                E0 = pe_cur + kinetic<D, GW>(sh.imm[jc], r0, gmask);
+                __syncwarp(gmask);
+                if (own) {
+                    const double zj = sh.zp[lig], gj = sh.gp[lig];
+                    sh.zl[lig] = zj; sh.zr[lig] = zj; sh.gl[lig] = gj; sh.gr[lig] = gj;
+                    sh.rl[lig] = r0; sh.rr[lig] = r0;
+                    sh.m_rsum[lig] = r0;
+                }
+                m_weight = 0.0; m_sum_acc = 0.0; m_nprop = 0; m_depth = 0; m_turning = false; m_div = false;
+                m_pe_p = pe_cur;
+                m_is_c = true;  // the tree's proposal is the current state until a subtree's proposal is taken
+                leaf_counter = 0;
+                pend = PS_DOUBLING;
+            }
+            if (pend == PS_DOUBLING) {
+                double u_dir;
+                uniform2(philox4x32(key, (uint32_t)m_depth, (uint32_t)t, c2word(run_kind, P_DIR), 0u), u_dir, u_main);
+                going_right = u_dir < 0.5;
+                s_nprop = 0;
+                __syncwarp(gmask);
+                zf = going_right ? sh.zr[jc] : sh.zl[jc];
+                rf = going_right ? sh.rr[jc] : sh.rl[jc];
+                gf = going_right ? sh.gr[jc] : sh.gl[jc];
+                e = going_right ? eps : -eps;
+                phase = GP_LEAF;
             }
         }
 
@@ -785,10 +723,9 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                 if (p.chain_clock != nullptr) p.chain_clock[((size_t)tax * MDG_NUM_RUNS + run_kind) * 2 + 1] = global_timer_ns();
             }
             __syncwarp(gmask);
-            // the leapfrog source is dead here; saying so keeps it from being carried (spilled: 48 B of local memory
-            // in the PMD kernel) across the evaluation for the paths that end a chain without overwriting it
-#pragma unroll
-            for (int j = 0; j < D; ++j) { zf[j] = 0.0; rf[j] = 0.0; gf[j] = 0.0; }
+            // the leapfrog source is dead here; saying so keeps the compiler from carrying its old value across the
+            // evaluation (in registers, which the evaluation needs) for the paths that end a chain without overwriting it
+            zf = 0.0; rf = 0.0; gf = 0.0;
             phase = GP_FETCH;
         }
     }
