@@ -4,6 +4,9 @@
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
+#include <memory>
+#include <string>
+#include <type_traits>
 #include <vector>
 #include <algorithm>
 
@@ -26,10 +29,16 @@ void set_error(const char* fmt, ...) {
     va_end(ap);
 }
 
-// grow-only device buffer
+// grow-only device buffer, freed by its destructor
 struct DevBuf {
     void* ptr = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() {
+        if (ptr) cudaFree(ptr);
+    }
     int ensure(size_t bytes) {
         if (bytes <= cap) return MDG_OK;
         if (ptr) cudaFree(ptr);
@@ -44,15 +53,23 @@ struct DevBuf {
         cap = bytes;
         return MDG_OK;
     }
-    void release() {
-        if (ptr) cudaFree(ptr);
-        ptr = nullptr;
-        cap = 0;
-    }
     template <typename T> T* as() const { return reinterpret_cast<T*>(ptr); }
 };
 
-constexpr int kNumEvents = 16;
+// owner of a stream, an event or a pinned host allocation, released by its destructor
+template <typename H, auto Release>
+struct Owned {
+    H h = nullptr;
+    Owned() = default;
+    Owned(const Owned&) = delete;
+    Owned& operator=(const Owned&) = delete;
+    ~Owned() {
+        if (h) Release(h);
+    }
+    operator H() const { return h; }
+};
+using CudaStream = Owned<cudaStream_t, cudaStreamDestroy>;
+using CudaEvent = Owned<cudaEvent_t, cudaEventDestroy>;
 
 }  // namespace mdg
 
@@ -60,25 +77,25 @@ constexpr int kNumEvents = 16;
 // same batch or of the next submitted batch) starts under the tail of chunk c, which is a handful of long
 // sequential chains on an otherwise idle GPU.
 struct mdg_fit_lane {
-    cudaStream_t main = nullptr, side[2] = {nullptr, nullptr};  // main: high priority; side[m]: the NUTS launch of model m (0 PMD, 1 null)
-    cudaEvent_t ev[5] = {};  // chunk begin, MAP end, NUTS end, predictive end, done (after assembly + D2H)
-    cudaEvent_t fork_ev = nullptr, join_ev[2] = {nullptr, nullptr};  // join_ev[m]: end of side[m]'s NUTS launch
+    mdg::CudaStream main, side[2];  // main: high priority; side[m]: the NUTS launch of model m (0 PMD, 1 null)
+    mdg::CudaEvent begin, map_end, nuts_end, pred_end, done;  // done: after assembly and the copies back
+    mdg::CudaEvent nuts_fork, nuts_join[2];  // nuts_join[m]: end of side[m]'s NUTS launch
     mdg::DevBuf rec, map, pred, counters, samples, waic, waic_acc[2];
     mdg::DevBuf chain_clock;  // development switch MDG_CHAIN_CLOCK=<file>
     mdg::DevBuf order;        // queue order of the chunk's TaxIDs: [chunk] int order, [chunk] bucket bytes, 3 x kOrderBuckets counters
     int clock_items = 0;
-    unsigned long long* h_leap = nullptr;  // pinned [MDG_NUM_RUNS]
+    mdg::Owned<unsigned long long*, cudaFreeHost> h_leap;  // pinned [MDG_NUM_RUNS]
     bool busy = false;
     int owner = -1;          // ticket slot of the chunk in flight
     uint32_t launches = 0;
 };
 
-// One submitted batch (mdg_fit_batch_submit): staging buffers for MDG_HOST and the accumulated timings.
+// One submitted batch (mdg_fit_batch_submit): its staged inputs / outputs and the accumulated timings.
 struct mdg_fit_ticket_slot {
     bool active = false;
     int64_t id = 0;
-    cudaEvent_t ev_begin = nullptr;
-    mdg::DevBuf in_tax, in_k, in_N, in_m12, in_noise, out_res, out_med, smp, trace, waic;
+    mdg::CudaEvent ev_begin;
+    mdg::DevBuf arena;
     mdg_timings t = {};
     double nuts_begin_ms = 0, nuts_end_ms = 0;
     bool have_nuts = false;
@@ -90,30 +107,24 @@ constexpr int kFitTickets = MDG_MAX_INFLIGHT;
 struct mdg_ctx {
     int device = 0;
     int num_sms = 0;
-    cudaStream_t own_stream = nullptr;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t ev[mdg::kNumEvents] = {};
-    cudaEvent_t epoch = nullptr;       // time zero of mdg_timings.nuts_begin_ms / nuts_end_ms
-    cudaEvent_t inputs_ready = nullptr;
-    // scratch of the synchronous entry points, each named after the entry points that use it (they share a buffer
-    // only where the calls never overlap: each synchronises before it returns)
-    mdg::DevBuf reduce_in;              // mdg_counts_reduce: staged input columns (MDG_HOST)
-    mdg::DevBuf reduce_tsv_out;         // mdg_counts_reduce, mdg_tsv_parse: staged output columns (MDG_HOST)
-    mdg::DevBuf reduce_tsv_scalars;     // mdg_counts_reduce, mdg_tsv_parse: 64 B of device counters and error flags
-    mdg::DevBuf reduce_tiles;           // mdg_counts_reduce: per-tile block bookkeeping and scan chunk totals
-    mdg::DevBuf reduce_tmp;             // mdg_counts_reduce: per-TaxID rows before the permute puts them in order
-    mdg::DevBuf order_tsv_top_in;       // mdg_counts_order, mdg_select_top: staged inputs (MDG_HOST); mdg_tsv_parse: the text
-    mdg::DevBuf order_tsv_top_scratch;  // mdg_counts_order, mdg_tsv_parse, mdg_select_top: per-block counts, scans, histograms
-    mdg::DevBuf test_scratch;           // mdg_test_*, mdg_measure_fp64_peak
-    mdg::DevBuf da_tables;             // sqrt(t) and t^-0.75 for t < kDaTable (dual averaging), filled at the first fit
+    mdg::CudaStream own_stream;
+    cudaStream_t stream = nullptr;  // own_stream, or the caller's (mdg_ctx_set_stream)
+    // timing of the synchronous entry points
+    mdg::CudaEvent call_begin, work_begin, work_end, call_end;
+    mdg::CudaEvent epoch;  // time zero of mdg_timings.nuts_begin_ms / nuts_end_ms
+    mdg::CudaEvent inputs_ready;
+    // staged buffers and scratch of the synchronous entry points (they never overlap: each synchronises before
+    // it returns)
+    mdg::DevBuf arena;
+    mdg::DevBuf test_scratch;  // mdg_test_*, mdg_measure_fp64_peak
+    mdg::DevBuf da_tables;     // sqrt(t) and t^-0.75 for t < kDaTable (dual averaging), filled at the first fit
     mdg_fit_lane lane[kFitLanes];
     mdg_fit_ticket_slot ticket[kFitTickets];
     int next_lane = 0;
     int64_t next_ticket_id = 1;
     double nuts_covered_until_ms = 0;  // union of NUTS intervals harvested so far ends here
     mdg_timings timings = {};
-    // mdg_map_batch: staged inputs / outputs (MDG_HOST), per-run records, counters; apart from the fit lanes' scratch
-    mdg::DevBuf map_in_tax, map_in_k, map_in_N, map_in_m12, map_in_noise, map_out, map_rec, map_counters;
+    mdg::DevBuf map_rec, map_counters;  // mdg_map_batch: per-run records, counters; apart from the fit lanes' scratch
 };
 
 using namespace mdg;
@@ -129,6 +140,66 @@ struct DeviceGuard {
     ~DeviceGuard() {
         if (prev >= 0) cudaSetDevice(prev);
     }
+};
+
+// The device side of one call's buffers. Callers register requests, each naming the launch-struct field that
+// receives the device pointer: inputs (copied in), outputs (copied back by rows) and scratch. commit() lays them
+// out in one grow-only arena, each 256-byte aligned (the 128-bit load / store paths of mdg_counts_reduce depend
+// on it), and enqueues the host-to-device copies. Under MDG_DEVICE inputs and outputs are the caller's pointers
+// and only scratch takes arena space; a NULL input or output stays NULL.
+class Stage {
+public:
+    Stage(DevBuf& arena, bool host, cudaStream_t st) : arena_(arena), host_(host), st_(st) {}
+    template <typename T> void in(T*& field, const void* src, size_t bytes) { add(&field, kIn, const_cast<void*>(src), bytes, 0); }
+    // `rows` rows of `row_bytes` each; copy_back() copies a range of them
+    template <typename T> void out(T*& field, void* dst, size_t row_bytes, size_t rows) { add(&field, kOut, dst, row_bytes * rows, row_bytes); }
+    // copied back in full by every copy_back()
+    template <typename T> void out_all(T*& field, void* dst, size_t bytes) { add(&field, kOut, dst, bytes, 0); }
+    template <typename T> void scratch(T*& field, size_t bytes) { add(&field, kScratch, nullptr, bytes, 0); }
+
+    int commit() {
+        size_t total = 0;
+        for (const Req& r : reqs_) total += staged(r) ? align(r.bytes) : 0;
+        if (int rc = arena_.ensure(total)) return rc;
+        unsigned char* p = arena_.as<unsigned char>();
+        for (const Req& r : reqs_) {
+            void* d = staged(r) ? p : r.user;
+            std::memcpy(r.field, &d, sizeof d);
+            if (!staged(r)) continue;
+            p += align(r.bytes);
+            if (r.kind == kIn && r.bytes) MDG_CUDA_TRY(cudaMemcpyAsync(d, r.user, r.bytes, cudaMemcpyHostToDevice, st_));
+        }
+        return MDG_OK;
+    }
+
+    int copy_back(size_t row0, size_t rows, cudaStream_t st) const {
+        for (const Req& r : reqs_) {
+            if (r.kind != kOut || !staged(r)) continue;
+            unsigned char* d;
+            std::memcpy(&d, r.field, sizeof d);
+            const size_t off = row0 * r.row_bytes, bytes = r.row_bytes ? rows * r.row_bytes : r.bytes;
+            if (bytes) MDG_CUDA_TRY(cudaMemcpyAsync((unsigned char*)r.user + off, d + off, bytes, cudaMemcpyDeviceToHost, st));
+        }
+        return MDG_OK;
+    }
+
+private:
+    enum Kind { kIn, kOut, kScratch };
+    struct Req {
+        void* field;  // a T* launch-struct member (or local)
+        Kind kind;
+        void* user;   // the caller's source / destination
+        size_t bytes, row_bytes;
+    };
+    static size_t align(size_t b) { return (b + 255) & ~(size_t)255; }
+    bool staged(const Req& r) const { return r.kind == kScratch || (host_ && r.user); }
+    template <typename T> void add(T** field, Kind kind, void* user, size_t bytes, size_t row_bytes) {
+        reqs_.push_back({(void*)field, kind, user, bytes, row_bytes});
+    }
+    DevBuf& arena_;
+    const bool host_;
+    const cudaStream_t st_;
+    std::vector<Req> reqs_;
 };
 
 Priors make_priors(const mdg_fit_config& c) {
@@ -222,43 +293,43 @@ int launch_nuts_group(mdg_ctx* ctx, cudaStream_t st, FitLaunch fl, DevBuf& acc) 
     return MDG_OK;
 }
 
-int launch_map(mdg_ctx* ctx, cudaStream_t st, const MapLaunch& ml, int npl) {
-    const long long items = 2ll * ml.n_tax;
-    if (npl == 1) {
-        int grid = persistent_grid(map_kernel<1, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
-        map_kernel<1, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
-    } else if (npl == 2) {
-        int grid = persistent_grid(map_kernel<2, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
-        map_kernel<2, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
-    } else {
-        int grid = persistent_grid(map_kernel<4, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
-        map_kernel<4, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
-    }
-    MDG_CUDA_TRY(cudaGetLastError());
-    ctx->timings.n_launches++;
-    return MDG_OK;
-}
-
-int launch_map_batch(mdg_ctx* ctx, cudaStream_t st, const MapBatchLaunch& ml, int npl) {
-    const long long items = (long long)ml.n_runs * ml.n_tax;
-    if (npl == 1) {
-        int grid = persistent_grid(map_batch_kernel<1, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
-        map_batch_kernel<1, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
-    } else if (npl == 2) {
-        int grid = persistent_grid(map_batch_kernel<2, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
-        map_batch_kernel<2, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
-    } else {
-        int grid = persistent_grid(map_batch_kernel<4, kMapWarps>, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
-        map_batch_kernel<4, kMapWarps><<<grid, kMapWarps * 32, 0, st>>>(ml);
-    }
-    MDG_CUDA_TRY(cudaGetLastError());
-    ctx->timings.n_launches++;
-    return MDG_OK;
-}
-
 int npl_for(int n_obs, int gw) {
     int npl = (n_obs + gw - 1) / gw;
     return npl <= 1 ? 1 : (npl <= 2 ? 2 : 4);
+}
+
+// f(std::integral_constant<int, NPL>{}) for the observations per lane of a warp over n_obs positions
+template <typename F>
+void with_npl(int n_obs, F&& f) {
+    const int npl = npl_for(n_obs, 32);
+    if (npl == 1) f(std::integral_constant<int, 1>{});
+    else if (npl == 2) f(std::integral_constant<int, 2>{});
+    else f(std::integral_constant<int, 4>{});
+}
+
+// map_kernel / map_batch_kernel fit all 2P positions of a TaxID
+int launch_map(mdg_ctx* ctx, cudaStream_t st, const MapLaunch& ml) {
+    const long long items = 2ll * ml.n_tax;
+    with_npl(2 * ml.P, [&](auto npl) {
+        auto kern = map_kernel<decltype(npl)::value, kMapWarps>;
+        int grid = persistent_grid(kern, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
+        kern<<<grid, kMapWarps * 32, 0, st>>>(ml);
+    });
+    MDG_CUDA_TRY(cudaGetLastError());
+    ctx->timings.n_launches++;
+    return MDG_OK;
+}
+
+int launch_map_batch(mdg_ctx* ctx, cudaStream_t st, const MapBatchLaunch& ml) {
+    const long long items = (long long)ml.n_runs * ml.n_tax;
+    with_npl(2 * ml.P, [&](auto npl) {
+        auto kern = map_batch_kernel<decltype(npl)::value, kMapWarps>;
+        int grid = persistent_grid(kern, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
+        kern<<<grid, kMapWarps * 32, 0, st>>>(ml);
+    });
+    MDG_CUDA_TRY(cudaGetLastError());
+    ctx->timings.n_launches++;
+    return MDG_OK;
 }
 
 float elapsed(cudaEvent_t a, cudaEvent_t b) {
@@ -270,8 +341,6 @@ float elapsed(cudaEvent_t a, cudaEvent_t b) {
 }  // namespace
 
 extern "C" {
-
-void mdg_ctx_destroy(mdg_ctx* ctx);
 
 int mdg_version(void) { return MDG_VERSION; }
 
@@ -325,22 +394,19 @@ int mdg_ctx_create(int device, mdg_ctx** out) {
         return MDG_ERR_CUDA;
     }
     *out = nullptr;
-    mdg_ctx* ctx = new mdg_ctx();
+    std::unique_ptr<mdg_ctx> ctx(new mdg_ctx());  // a failure below releases what was created so far
     ctx->device = device;
     ctx->num_sms = prop.multiProcessorCount;
-    // any failure below releases what was created so far (mdg_ctx_destroy tolerates null members)
     auto fail = [&](cudaError_t e, const char* what) {
         set_error("mdg_ctx_create: %s failed: %s", what, cudaGetErrorString(e));
-        mdg_ctx_destroy(ctx);
         return MDG_ERR_CUDA;
     };
     cudaError_t e;
-    if ((e = cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking)) != cudaSuccess) return fail(e, "cudaStreamCreate");
+    if ((e = cudaStreamCreateWithFlags(&ctx->own_stream.h, cudaStreamNonBlocking)) != cudaSuccess) return fail(e, "cudaStreamCreate");
     ctx->stream = ctx->own_stream;
-    for (int i = 0; i < kNumEvents; ++i)
-        if ((e = cudaEventCreate(&ctx->ev[i])) != cudaSuccess) return fail(e, "cudaEventCreate");
-    if ((e = cudaEventCreate(&ctx->epoch)) != cudaSuccess) return fail(e, "cudaEventCreate");
-    if ((e = cudaEventCreateWithFlags(&ctx->inputs_ready, cudaEventDisableTiming)) != cudaSuccess) return fail(e, "cudaEventCreate");
+    for (CudaEvent* ev : {&ctx->call_begin, &ctx->work_begin, &ctx->work_end, &ctx->call_end, &ctx->epoch})
+        if ((e = cudaEventCreate(&ev->h)) != cudaSuccess) return fail(e, "cudaEventCreate");
+    if ((e = cudaEventCreateWithFlags(&ctx->inputs_ready.h, cudaEventDisableTiming)) != cudaSuccess) return fail(e, "cudaEventCreate");
     // The NUTS launches are persistent and fill every CTA slot of the GPU; the short kernels around them (MAP,
     // posterior predictive, assembly) of the OTHER batch in flight must not queue behind the NUTS CTAs that are
     // still waiting for a slot, or a batch could not complete (and the next one not be submitted) before the
@@ -349,22 +415,21 @@ int mdg_ctx_create(int device, mdg_ctx** out) {
     int prio_low = 0, prio_high = 0;
     if ((e = cudaDeviceGetStreamPriorityRange(&prio_low, &prio_high)) != cudaSuccess) return fail(e, "cudaDeviceGetStreamPriorityRange");
     for (auto& ln : ctx->lane) {
-        if ((e = cudaStreamCreateWithPriority(&ln.main, cudaStreamNonBlocking, prio_high)) != cudaSuccess) return fail(e, "cudaStreamCreate");
+        if ((e = cudaStreamCreateWithPriority(&ln.main.h, cudaStreamNonBlocking, prio_high)) != cudaSuccess) return fail(e, "cudaStreamCreate");
         for (auto& sd : ln.side)
-            if ((e = cudaStreamCreateWithPriority(&sd, cudaStreamNonBlocking, prio_low)) != cudaSuccess) return fail(e, "cudaStreamCreate");
-        for (int i = 0; i < 5; ++i)
-            if ((e = cudaEventCreate(&ln.ev[i])) != cudaSuccess) return fail(e, "cudaEventCreate");
-        if ((e = cudaEventCreateWithFlags(&ln.fork_ev, cudaEventDisableTiming)) != cudaSuccess) return fail(e, "cudaEventCreate");
-        for (auto& je : ln.join_ev)
-            if ((e = cudaEventCreateWithFlags(&je, cudaEventDisableTiming)) != cudaSuccess) return fail(e, "cudaEventCreate");
-        if ((e = cudaHostAlloc((void**)&ln.h_leap, MDG_NUM_RUNS * sizeof(unsigned long long), cudaHostAllocDefault)) != cudaSuccess)
+            if ((e = cudaStreamCreateWithPriority(&sd.h, cudaStreamNonBlocking, prio_low)) != cudaSuccess) return fail(e, "cudaStreamCreate");
+        for (CudaEvent* ev : {&ln.begin, &ln.map_end, &ln.nuts_end, &ln.pred_end, &ln.done})
+            if ((e = cudaEventCreate(&ev->h)) != cudaSuccess) return fail(e, "cudaEventCreate");
+        for (CudaEvent* ev : {&ln.nuts_fork, &ln.nuts_join[0], &ln.nuts_join[1]})
+            if ((e = cudaEventCreateWithFlags(&ev->h, cudaEventDisableTiming)) != cudaSuccess) return fail(e, "cudaEventCreate");
+        if ((e = cudaHostAlloc((void**)&ln.h_leap.h, MDG_NUM_RUNS * sizeof(unsigned long long), cudaHostAllocDefault)) != cudaSuccess)
             return fail(e, "cudaHostAlloc");
     }
     for (auto& tk : ctx->ticket)
-        if ((e = cudaEventCreate(&tk.ev_begin)) != cudaSuccess) return fail(e, "cudaEventCreate");
+        if ((e = cudaEventCreate(&tk.ev_begin.h)) != cudaSuccess) return fail(e, "cudaEventCreate");
     if ((e = cudaEventRecord(ctx->epoch, ctx->own_stream)) != cudaSuccess) return fail(e, "cudaEventRecord");
     if ((e = cudaEventSynchronize(ctx->epoch)) != cudaSuccess) return fail(e, "cudaEventSynchronize");
-    *out = ctx;
+    *out = ctx.release();
     return MDG_OK;
 }
 
@@ -372,38 +437,10 @@ void mdg_ctx_destroy(mdg_ctx* ctx) {
     if (!ctx) return;
     DeviceGuard guard(ctx->device);
     for (auto& ln : ctx->lane) {
-        if (ln.main) cudaStreamSynchronize(ln.main);
-        for (cudaStream_t sd : ln.side) if (sd) cudaStreamSynchronize(sd);
+        cudaStreamSynchronize(ln.main);
+        for (cudaStream_t sd : ln.side) cudaStreamSynchronize(sd);
     }
-    if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    for (mdg::DevBuf* b : {&ctx->reduce_in, &ctx->reduce_tsv_out, &ctx->reduce_tsv_scalars, &ctx->reduce_tiles, &ctx->reduce_tmp,
-                           &ctx->order_tsv_top_in, &ctx->order_tsv_top_scratch, &ctx->test_scratch, &ctx->da_tables})
-        b->release();
-    for (int i = 0; i < kNumEvents; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
-    if (ctx->epoch) cudaEventDestroy(ctx->epoch);
-    if (ctx->inputs_ready) cudaEventDestroy(ctx->inputs_ready);
-    for (auto& ln : ctx->lane) {
-        for (mdg::DevBuf* b : {&ln.rec, &ln.map, &ln.pred, &ln.counters, &ln.samples, &ln.waic, &ln.waic_acc[0], &ln.waic_acc[1],
-                               &ln.chain_clock, &ln.order})
-            b->release();
-        for (int i = 0; i < 5; ++i) if (ln.ev[i]) cudaEventDestroy(ln.ev[i]);
-        if (ln.fork_ev) cudaEventDestroy(ln.fork_ev);
-        for (int m = 0; m < 2; ++m) {
-            if (ln.join_ev[m]) cudaEventDestroy(ln.join_ev[m]);
-            if (ln.side[m]) cudaStreamDestroy(ln.side[m]);
-        }
-        if (ln.main) cudaStreamDestroy(ln.main);
-        if (ln.h_leap) cudaFreeHost(ln.h_leap);
-    }
-    for (mdg::DevBuf* b : {&ctx->map_in_tax, &ctx->map_in_k, &ctx->map_in_N, &ctx->map_in_m12, &ctx->map_in_noise, &ctx->map_out,
-                           &ctx->map_rec, &ctx->map_counters})
-        b->release();
-    for (auto& tk : ctx->ticket) {
-        for (mdg::DevBuf* b : {&tk.in_tax, &tk.in_k, &tk.in_N, &tk.in_m12, &tk.in_noise, &tk.out_res, &tk.out_med, &tk.smp, &tk.trace, &tk.waic})
-            b->release();
-        if (tk.ev_begin) cudaEventDestroy(tk.ev_begin);
-    }
-    if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
+    cudaStreamSynchronize(ctx->stream);
     delete ctx;
 }
 
@@ -455,71 +492,59 @@ int mdg_counts_reduce(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_
     if (n_rows == 0) return MDG_OK;
     const int P = max_position, R = 2 * P;
     const size_t n = (size_t)n_rows;
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_begin, st));
 
-    // ---- stage inputs / outputs on the device for MDG_HOST ----
-    CountsLaunch cl = {};
+    // ---- the caller's buffers (MDG_DEVICE) or staged ones (MDG_HOST), and scratch ----
     const bool host = (mem == MDG_HOST);
-    struct OutCopy { void* host_ptr; const void* dev_ptr; size_t elem; bool per_tax; };
-    std::vector<OutCopy> copies;
-    if (host) {
-        // one arena for inputs, one for outputs
-        size_t in_bytes = n * (8 + 4 + 1 + 1) + 256 * 5 + 16 * ((n * 4 + 255) & ~(size_t)255);
-        int rc = ctx->reduce_in.ensure(in_bytes);
-        if (rc) return rc;
-        unsigned char* base = ctx->reduce_in.as<unsigned char>();
-        size_t off = 0;
-        auto put = [&](const void* src, size_t bytes) -> void* {
-            void* d = base + off;
-            cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, st);
-            off += (bytes + 255) & ~(size_t)255;
-            return d;
-        };
-        cl.tax_id = (const long long*)put(tax_id, n * 8);
-        cl.n_align = (const uint32_t*)put(n_alignments, n * 4);
-        cl.is_rev = (const uint8_t*)put(is_reverse, n);
-        cl.pos0 = (const uint8_t*)put(pos0, n);
-        const size_t col_stride = ((n * 4 + 255) & ~(size_t)255) / 4;
-        uint32_t* dcounts = (uint32_t*)(base + off);
+    const size_t ncap = (size_t)out_capacity;
+    CountsLaunch cl = {};
+    Stage stage(ctx->arena, host, st);
+    stage.in(cl.tax_id, tax_id, n * 8);
+    stage.in(cl.n_align, n_alignments, n * 4);
+    stage.in(cl.is_rev, is_reverse, n);
+    stage.in(cl.pos0, pos0, n);
+    // staged counts16 columns start 256 bytes apart, a multiple of 4 rows
+    cl.counts16 = counts16;
+    cl.stride = host ? (long long)(((n * 4 + 255) & ~(size_t)255) / 4) : counts_stride;
+    if (host) stage.scratch(cl.counts16, 16 * (size_t)cl.stride * 4);
+    stage.out_all(cl.n_fwd_row, n_fwd_ref_row, n * 4);
+    stage.out_all(cl.n_rev_row, n_rev_ref_row, n * 4);
+    stage.out_all(cl.f_fwd_row, f_fwd_row, n * 4);
+    stage.out_all(cl.f_rev_row, f_rev_row, n * 4);
+    stage.out_all(cl.z_row, z_row, n);
+    stage.out_all(cl.y_row, y_sum_total_row, n * 8);
+    stage.out_all(cl.keep_row, keep_row, n);
+    stage.out(cl.out_tax, out_tax_id, 8, ncap);
+    stage.out(cl.out_nal, out_n_alignments, 4, ncap);
+    // the noise kernel needs the first rows in final order even if the caller does not want them
+    if (out_first_row || !out_noise) stage.out(cl.out_first, out_first_row, 8, ncap);
+    else stage.scratch(cl.out_first, ncap * 8);
+    stage.out(cl.out_k, out_k, 4 * (size_t)R, ncap);
+    stage.out(cl.out_N, out_N, 4 * (size_t)R, ncap);
+    stage.out(cl.out_noise, out_noise, 24, ncap);
+    long long* d_ntax;  // [0] kept TaxIDs, [1] error flag (int), [2] dense rows reserved
+    stage.scratch(d_ntax, 64);
+    // ---- warp-synchronous streaming kernel (mdg_counts_stream.cuh): one warp per 128 rows ----
+    const long long n_tiles = (n_rows + kStreamRows - 1) / kStreamRows;
+    const long long n_chunks = (n_tiles + kScanChunk - 1) / kScanChunk;
+    CountsPermute cp = {};
+    long long *d_tile_base, *d_final_base, *d_chunk;
+    int* d_tile_cnt;
+    stage.scratch(d_tile_base, (size_t)n_tiles * 8);
+    stage.scratch(d_final_base, (size_t)n_tiles * 8);
+    stage.scratch(d_chunk, (size_t)n_chunks * 8);
+    stage.scratch(d_tile_cnt, (size_t)n_tiles * 4);
+    // the stream kernel writes the per-TaxID rows into temporaries, the permute moves them
+    if (out_tax_id) stage.scratch(cp.t_tax, ncap * 8);
+    if (out_n_alignments) stage.scratch(cp.t_nal, ncap * 4);
+    if (out_first_row || out_noise) stage.scratch(cp.t_first, ncap * 8);
+    if (out_k) stage.scratch(cp.t_k, ncap * R * 4);
+    if (out_N) stage.scratch(cp.t_N, ncap * R * 4);
+    if (int rc = stage.commit()) return rc;
+    if (host)
         for (int c = 0; c < 16; ++c)
-            cudaMemcpyAsync(dcounts + (size_t)c * col_stride, counts16 + (size_t)c * counts_stride, n * 4, cudaMemcpyHostToDevice, st);
-        cl.counts16 = dcounts;
-        cl.stride = (long long)col_stride;
-        MDG_CUDA_TRY(cudaGetLastError());
-        const size_t ncap = (size_t)out_capacity;
-        size_t out_bytes = n * (4 + 4 + 4 + 4 + 1 + 8 + 1) + ncap * (8 + 4 + 8) + ncap * (size_t)R * 8 + ncap * 24 + 256 * 16;
-        rc = ctx->reduce_tsv_out.ensure(out_bytes);
-        if (rc) return rc;
-        unsigned char* ob = ctx->reduce_tsv_out.as<unsigned char>();
-        size_t oo = 0;
-        auto take = [&](void* host_ptr, size_t elem, size_t count, bool per_tax) -> void* {
-            if (!host_ptr) return nullptr;
-            void* d = ob + oo;
-            oo += (elem * count + 255) & ~(size_t)255;
-            copies.push_back({host_ptr, d, elem, per_tax});
-            return d;
-        };
-        cl.n_fwd_row = (uint32_t*)take(n_fwd_ref_row, 4, n, false);
-        cl.n_rev_row = (uint32_t*)take(n_rev_ref_row, 4, n, false);
-        cl.f_fwd_row = (float*)take(f_fwd_row, 4, n, false);
-        cl.f_rev_row = (float*)take(f_rev_row, 4, n, false);
-        cl.z_row = (int8_t*)take(z_row, 1, n, false);
-        cl.y_row = (unsigned long long*)take(y_sum_total_row, 8, n, false);
-        cl.keep_row = (uint8_t*)take(keep_row, 1, n, false);
-        cl.out_tax = (long long*)take(out_tax_id, 8, ncap, true);
-        cl.out_nal = (uint32_t*)take(out_n_alignments, 4, ncap, true);
-        cl.out_first = (long long*)take(out_first_row, 8, ncap, true);
-        cl.out_k = (uint32_t*)take(out_k, 4 * (size_t)R, ncap, true);
-        cl.out_N = (uint32_t*)take(out_N, 4 * (size_t)R, ncap, true);
-        cl.out_noise = (double*)take(out_noise, 24, ncap, true);
-    } else {
-        cl.tax_id = (const long long*)tax_id; cl.n_align = n_alignments; cl.is_rev = is_reverse; cl.pos0 = pos0;
-        cl.counts16 = counts16; cl.stride = counts_stride;
-        cl.n_fwd_row = n_fwd_ref_row; cl.n_rev_row = n_rev_ref_row; cl.f_fwd_row = f_fwd_row; cl.f_rev_row = f_rev_row;
-        cl.z_row = z_row; cl.y_row = (unsigned long long*)y_sum_total_row; cl.keep_row = keep_row;
-        cl.out_tax = (long long*)out_tax_id; cl.out_nal = out_n_alignments; cl.out_first = (long long*)out_first_row;
-        cl.out_k = out_k; cl.out_N = out_N; cl.out_noise = out_noise;
-    }
+            cudaMemcpyAsync((uint32_t*)cl.counts16 + (size_t)c * cl.stride, counts16 + (size_t)c * counts_stride, n * 4, cudaMemcpyHostToDevice, st);
+    MDG_CUDA_TRY(cudaGetLastError());
     cl.n_rows = n_rows;
     cl.fwd_ref = fwd_ref; cl.fwd_obs = fwd_obs; cl.rev_ref = rev_ref; cl.rev_obs = rev_obs;
     cl.P = P; cl.min_align = min_alignments; cl.min_y = min_y_sum;
@@ -530,49 +555,26 @@ int mdg_counts_reduce(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_
     // output bases 16-byte aligned -> 128-bit stores
     cl.vec_out = aligned16(cl.n_fwd_row) && aligned16(cl.n_rev_row) && aligned16(cl.f_fwd_row) && aligned16(cl.f_rev_row) &&
                  aligned16(cl.z_row) && aligned16(cl.y_row) && aligned16(cl.keep_row);
-    int rc = ctx->reduce_tsv_scalars.ensure(64);
-    if (rc) return rc;
-    long long* d_ntax = ctx->reduce_tsv_scalars.as<long long>();  // [0] kept TaxIDs, [1] error flag (int), [2] dense rows reserved
     int* d_err = reinterpret_cast<int*>(d_ntax + 1);
     int h_err = 0;
     long long h_ntax = 0;
-    // ---- warp-synchronous streaming kernel (mdg_counts_stream.cuh): one warp per 128 rows ----
-    const long long n_tiles = (n_rows + kStreamRows - 1) / kStreamRows;
-    const size_t ncap_t = (size_t)out_capacity;
-    const long long n_chunks = (n_tiles + kScanChunk - 1) / kScanChunk;
-    rc = ctx->reduce_tiles.ensure((size_t)n_tiles * (8 + 8 + 4) + (size_t)n_chunks * 8 + 64);
-    if (rc) return rc;
-    long long* d_tile_base = ctx->reduce_tiles.as<long long>();
-    long long* d_final_base = d_tile_base + n_tiles;
-    long long* d_chunk = d_final_base + n_tiles;
-    int* d_tile_cnt = reinterpret_cast<int*>(d_chunk + n_chunks);
-    const size_t tmp_bytes = ncap_t * (8 + 4 + 8 + 8 + (size_t)R * 8) + 256 * 8;
-    rc = ctx->reduce_tmp.ensure(tmp_bytes);
-    if (rc) return rc;
-    unsigned char* tb = ctx->reduce_tmp.as<unsigned char>();
-    size_t to = 0;
-    auto tmp = [&](size_t bytes) { void* q = tb + to; to += (bytes + 255) & ~(size_t)255; return q; };
-    // the noise kernel needs the first rows in final order even if the caller does not want them
-    long long* d_first_final = cl.out_first ? cl.out_first : (cl.out_noise ? (long long*)tmp(ncap_t * 8) : nullptr);
-    CountsPermute cp = {};
     cp.n_tiles = n_tiles; cp.tile_base = d_tile_base; cp.final_base = d_final_base; cp.tile_cnt = d_tile_cnt; cp.R = R;
     cp.chunk_off = d_chunk;
-    cp.out_tax = cl.out_tax; cp.out_nal = cl.out_nal; cp.out_first = d_first_final; cp.out_k = cl.out_k; cp.out_N = cl.out_N;
-    CountsLaunch kl = cl;  // the stream kernel writes the per-TaxID rows into the temporaries, the permute moves them
+    cp.out_tax = cl.out_tax; cp.out_nal = cl.out_nal; cp.out_first = cl.out_first; cp.out_k = cl.out_k; cp.out_N = cl.out_N;
+    CountsLaunch kl = cl;
     kl.out_noise = nullptr;
-    kl.out_first = nullptr;
-    if (cl.out_tax) { cp.t_tax = (long long*)tmp(ncap_t * 8); kl.out_tax = (long long*)cp.t_tax; }
-    if (cl.out_nal) { cp.t_nal = (uint32_t*)tmp(ncap_t * 4); kl.out_nal = (uint32_t*)cp.t_nal; }
-    if (d_first_final) { cp.t_first = (long long*)tmp(ncap_t * 8); kl.out_first = (long long*)cp.t_first; }
-    if (cl.out_k) { cp.t_k = (uint32_t*)tmp(ncap_t * R * 4); kl.out_k = (uint32_t*)cp.t_k; }
-    if (cl.out_N) { cp.t_N = (uint32_t*)tmp(ncap_t * R * 4); kl.out_N = (uint32_t*)cp.t_N; }
+    kl.out_tax = (long long*)cp.t_tax;
+    kl.out_nal = (uint32_t*)cp.t_nal;
+    kl.out_first = (long long*)cp.t_first;
+    kl.out_k = (uint32_t*)cp.t_k;
+    kl.out_N = (uint32_t*)cp.t_N;
     kl.kept_counter = reinterpret_cast<unsigned long long*>(d_ntax + 2);
     kl.tile_base = d_tile_base;
     kl.tile_cnt = d_tile_cnt;
     kl.capacity = out_capacity;
     kl.error_flag = d_err;
     MDG_CUDA_TRY(cudaMemsetAsync(d_ntax, 0, 64, st));
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->work_begin, st));
     counts_stream_kernel<<<(unsigned)((n_tiles + kStreamWarps - 1) / kStreamWarps), kStreamWarps * 32, 0, st>>>(kl);
     MDG_CUDA_TRY(cudaGetLastError());
     counts_scan_local_kernel<<<(unsigned)n_chunks, kScanChunk, 0, st>>>(d_tile_cnt, n_tiles, d_final_base, d_chunk);
@@ -584,13 +586,13 @@ int mdg_counts_reduce(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_
     if (cl.out_noise) {
         NoiseLaunch nl = {};
         nl.n_rows = n_rows; nl.tax_id = cl.tax_id; nl.is_rev = cl.is_rev; nl.pos0 = cl.pos0; nl.counts16 = cl.counts16;
-        nl.stride = cl.stride; nl.P = P; nl.n_tax = d_ntax; nl.first_row = d_first_final; nl.out_noise = cl.out_noise;
+        nl.stride = cl.stride; nl.P = P; nl.n_tax = d_ntax; nl.first_row = cl.out_first; nl.out_noise = cl.out_noise;
         nl.capacity = out_capacity;
         counts_noise_kernel<<<(unsigned)std::max<long long>(1, std::min<long long>((out_capacity + 3) / 4, 16LL * ctx->num_sms)), 128, 0, st>>>(nl);
         MDG_CUDA_TRY(cudaGetLastError());
         ctx->timings.n_launches += 1;
     }
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[2], st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->work_end, st));
     MDG_CUDA_TRY(cudaMemcpyAsync(&h_err, d_err, sizeof(int), cudaMemcpyDeviceToHost, st));
     MDG_CUDA_TRY(cudaMemcpyAsync(&h_ntax, d_ntax, sizeof(long long), cudaMemcpyDeviceToHost, st));
     MDG_CUDA_TRY(cudaStreamSynchronize(st));
@@ -608,16 +610,11 @@ int mdg_counts_reduce(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_
         return MDG_ERR_OVERFLOW;
     }
     *out_n_tax = h_ntax;
-    if (host) {
-        for (const auto& c : copies) {
-            size_t count = c.per_tax ? (size_t)h_ntax : n;
-            if (count) MDG_CUDA_TRY(cudaMemcpyAsync(c.host_ptr, c.dev_ptr, c.elem * count, cudaMemcpyDeviceToHost, st));
-        }
-    }
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[3], st));
+    if (int rc = stage.copy_back(0, (size_t)h_ntax, st)) return rc;
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_end, st));
     MDG_CUDA_TRY(cudaStreamSynchronize(st));
-    ctx->timings.counts_ms = elapsed(ctx->ev[1], ctx->ev[2]);
-    ctx->timings.total_ms = elapsed(ctx->ev[0], ctx->ev[3]);
+    ctx->timings.counts_ms = elapsed(ctx->work_begin, ctx->work_end);
+    ctx->timings.total_ms = elapsed(ctx->call_begin, ctx->call_end);
     return MDG_OK;
 }
 
@@ -638,44 +635,27 @@ int mdg_counts_order(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_i
     if (n_tax == 0) return MDG_OK;
     DeviceGuard guard(ctx->device);
     cudaStream_t st = ctx->stream;
-    const bool host = (mem == MDG_HOST);
     const size_t nr = (size_t)n_rows, nt = (size_t)n_tax;
-    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    int rc;
     OrderLaunch ol = {};
     ol.n_rows = n_rows; ol.n_tax = n_tax;
-    ol.tax_id_row = reinterpret_cast<const long long*>(tax_id_row); ol.z_row = z_row; ol.keep_row = keep_row;
-    ol.first_row = reinterpret_cast<const long long*>(first_row); ol.tax_order = reinterpret_cast<const long long*>(tax_order);
-    ol.perm = reinterpret_cast<long long*>(out_perm);
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
-    if (host) {
-        if ((rc = ctx->order_tsv_top_in.ensure(up(nr * 8) + up(nr) + up(nr) + 2 * up(nt * 8) + up((size_t)perm_capacity * 8)))) return rc;
-        unsigned char* b = ctx->order_tsv_top_in.as<unsigned char>();
-        size_t o = 0;
-        auto put = [&](const void* src, size_t bytes) -> void* {
-            void* d = b + o; o += up(bytes);
-            if (src) cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, st);
-            return d;
-        };
-        ol.tax_id_row = (const long long*)put(tax_id_row, nr * 8);
-        ol.z_row = (const int8_t*)put(z_row, nr);
-        void* kp = put(keep_row, nr);
-        ol.keep_row = keep_row ? (const uint8_t*)kp : nullptr;
-        ol.first_row = (const long long*)put(first_row, nt * 8);
-        ol.tax_order = (const long long*)put(tax_order, nt * 8);
-        ol.perm = (long long*)put(nullptr, (size_t)perm_capacity * 8);
-        MDG_CUDA_TRY(cudaGetLastError());
-    }
-    if ((rc = ctx->order_tsv_top_scratch.ensure(up(nt * 4) + up(nt * 8) + 256))) return rc;
-    unsigned char* sb = ctx->order_tsv_top_scratch.as<unsigned char>();
-    ol.len_sorted = reinterpret_cast<int*>(sb);
-    long long* d_start = reinterpret_cast<long long*>(sb + up(nt * 4));
-    long long* d_total = reinterpret_cast<long long*>(sb + up(nt * 4) + up(nt * 8));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_begin, st));
+    Stage stage(ctx->arena, mem == MDG_HOST, st);
+    stage.in(ol.tax_id_row, tax_id_row, nr * 8);
+    stage.in(ol.z_row, z_row, nr);
+    stage.in(ol.keep_row, keep_row, nr);
+    stage.in(ol.first_row, first_row, nt * 8);
+    stage.in(ol.tax_order, tax_order, nt * 8);
+    stage.out(ol.perm, out_perm, 8, (size_t)perm_capacity);
+    long long *d_start, *d_total;  // d_total: [0] kept rows, [1] error flag (int)
+    stage.scratch(ol.len_sorted, nt * 4);
+    stage.scratch(d_start, nt * 8);
+    stage.scratch(d_total, 16);
+    if (int rc = stage.commit()) return rc;
     ol.out_start = d_start;
     ol.error_flag = reinterpret_cast<int*>(d_total + 1);
     MDG_CUDA_TRY(cudaMemsetAsync(d_total, 0, 16, st));
     const unsigned grid = (unsigned)((n_tax + kOrderWarps - 1) / kOrderWarps);
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->work_begin, st));
     counts_order_kernel<0><<<grid, kOrderWarps * 32, 0, st>>>(ol);
     counts_scan_kernel<<<1, 1024, 0, st>>>(ol.len_sorted, n_tax, d_start, d_total);
     MDG_CUDA_TRY(cudaGetLastError());
@@ -691,13 +671,13 @@ int mdg_counts_order(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_i
     }
     counts_order_kernel<1><<<grid, kOrderWarps * 32, 0, st>>>(ol);
     MDG_CUDA_TRY(cudaGetLastError());
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[2], st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->work_end, st));
     ctx->timings.n_launches = 3;
-    if (host && h_total > 0) MDG_CUDA_TRY(cudaMemcpyAsync(out_perm, ol.perm, (size_t)h_total * 8, cudaMemcpyDeviceToHost, st));
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[3], st));
+    if (int rc = stage.copy_back(0, (size_t)h_total, st)) return rc;
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_end, st));
     MDG_CUDA_TRY(cudaStreamSynchronize(st));
-    ctx->timings.counts_ms = elapsed(ctx->ev[1], ctx->ev[2]);
-    ctx->timings.total_ms = elapsed(ctx->ev[0], ctx->ev[3]);
+    ctx->timings.counts_ms = elapsed(ctx->work_begin, ctx->work_end);
+    ctx->timings.total_ms = elapsed(ctx->call_begin, ctx->call_end);
     *out_n_rows = h_total;
     return MDG_OK;
 }
@@ -748,51 +728,34 @@ int mdg_tsv_parse(mdg_ctx* ctx, int mem, const char* text, int64_t n_bytes, int6
     if (out_n_cols) *out_n_cols = n_cols;
     DeviceGuard guard(ctx->device);
     cudaStream_t st = ctx->stream;
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_begin, st));
     const bool host = (mem == MDG_HOST);
     const size_t cap = (size_t)capacity;
     TsvLaunch tl = {};
     tl.n_bytes = n_bytes; tl.first = first; tl.n_cols = n_cols; tl.capacity = capacity;
     tl.n_blocks = (n_bytes - first + kTsvBlockBytes - 1) / kTsvBlockBytes;
-    int rc;
-    if ((rc = ctx->order_tsv_top_in.ensure((size_t)n_bytes + 16))) return rc;
-    MDG_CUDA_TRY(cudaMemcpyAsync(ctx->order_tsv_top_in.ptr, text, (size_t)n_bytes, cudaMemcpyHostToDevice, st));
-    tl.text = ctx->order_tsv_top_in.as<char>();
-    if ((rc = ctx->order_tsv_top_scratch.ensure((size_t)tl.n_blocks * 12 + (cap + 2) * 8 + 256))) return rc;
-    tl.block_base = ctx->order_tsv_top_scratch.as<long long>();
-    tl.line_start = tl.block_base + tl.n_blocks;
-    tl.block_cnt = reinterpret_cast<int*>(tl.line_start + cap + 2);
-    if ((rc = ctx->reduce_tsv_scalars.ensure(64))) return rc;
-    long long* d_scal = ctx->reduce_tsv_scalars.as<long long>();  // [0] newline total, [1] error flag (int), [2] error line
+    Stage stage(ctx->arena, host, st);
+    stage.scratch(tl.text, (size_t)n_bytes);  // copied below: `text` is a host pointer whatever `mem` says
+    stage.scratch(tl.block_base, (size_t)tl.n_blocks * 8);
+    stage.scratch(tl.line_start, (cap + 2) * 8);
+    stage.scratch(tl.block_cnt, (size_t)tl.n_blocks * 4);
+    long long* d_scal;  // [0] newline total, [1] error flag (int), [2] error line
+    stage.scratch(d_scal, 64);
+    stage.out(tl.tax_id, tax_id, 8, cap);
+    stage.out(tl.n_align, n_alignments, 4, cap);
+    stage.out(tl.is_rev, is_reverse, 1, cap);
+    stage.out(tl.pos0, pos0, 1, cap);
+    stage.out(tl.name_span, name_span, 16, cap);
+    stage.out(tl.rank_span, rank_span, 16, cap);
+    // staged counts16 columns start (cap rounded up to 64 rows) * 4 bytes apart
+    tl.counts16 = counts16;
+    tl.stride = host ? (long long)((cap + 63) & ~(size_t)63) : counts_stride;
+    if (host) stage.scratch(tl.counts16, 16 * (size_t)tl.stride * 4);
+    if (int rc = stage.commit()) return rc;
+    MDG_CUDA_TRY(cudaMemcpyAsync((char*)tl.text, text, (size_t)n_bytes, cudaMemcpyHostToDevice, st));
     tl.n_lines = d_scal; tl.error_flag = reinterpret_cast<int*>(d_scal + 1); tl.error_line = d_scal + 2;
     MDG_CUDA_TRY(cudaMemsetAsync(d_scal, 0, 64, st));
-    struct OutCopy { void* host_ptr; const void* dev_ptr; size_t bytes_per_row; };
-    std::vector<OutCopy> copies;
-    if (host) {
-        const size_t stride_dev = (cap + 63) & ~(size_t)63;
-        if ((rc = ctx->reduce_tsv_out.ensure(cap * (8 + 4 + 1 + 1 + 32) + 16 * stride_dev * 4 + 4096))) return rc;
-        unsigned char* ob = ctx->reduce_tsv_out.as<unsigned char>();
-        size_t oo = 0;
-        auto take = [&](void* hp, size_t elem) -> void* {
-            void* d = ob + oo;
-            oo += (elem * cap + 255) & ~(size_t)255;
-            if (hp) copies.push_back({hp, d, elem});
-            return d;
-        };
-        tl.tax_id = (long long*)take(tax_id, 8);
-        tl.n_align = (uint32_t*)take(n_alignments, 4);
-        tl.is_rev = (uint8_t*)take(is_reverse, 1);
-        tl.pos0 = (uint8_t*)take(pos0, 1);
-        tl.name_span = name_span ? (long long*)take(name_span, 16) : nullptr;
-        tl.rank_span = rank_span ? (long long*)take(rank_span, 16) : nullptr;
-        tl.counts16 = reinterpret_cast<uint32_t*>(ob + oo);
-        tl.stride = (long long)stride_dev;
-    } else {
-        tl.tax_id = (long long*)tax_id; tl.n_align = n_alignments; tl.is_rev = is_reverse; tl.pos0 = pos0;
-        tl.counts16 = counts16; tl.stride = counts_stride;
-        tl.name_span = (long long*)name_span; tl.rank_span = (long long*)rank_span;
-    }
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->work_begin, st));
     tsv_count_kernel<<<(unsigned)tl.n_blocks, kTsvThreads, 0, st>>>(tl);
     MDG_CUDA_TRY(cudaGetLastError());
     counts_scan_kernel<<<1, 1024, 0, st>>>(tl.block_cnt, tl.n_blocks, tl.block_base, tl.n_lines);
@@ -811,23 +774,22 @@ int mdg_tsv_parse(mdg_ctx* ctx, int mem, const char* text, int64_t n_bytes, int6
         tsv_parse_kernel<<<(unsigned)((n_lines + kTsvThreads - 1) / kTsvThreads), kTsvThreads, 0, st>>>(tl, n_lines);
         MDG_CUDA_TRY(cudaGetLastError());
     }
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[2], st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->work_end, st));
     ctx->timings.n_launches = 4;
     int h_err[2] = {0, 0};
     long long h_line = 0;
     MDG_CUDA_TRY(cudaMemcpyAsync(h_err, tl.error_flag, 4, cudaMemcpyDeviceToHost, st));
     MDG_CUDA_TRY(cudaMemcpyAsync(&h_line, tl.error_line, 8, cudaMemcpyDeviceToHost, st));
+    if (int rc = stage.copy_back(0, (size_t)n_lines, st)) return rc;
     if (host && n_lines > 0) {
-        for (const auto& c : copies)
-            MDG_CUDA_TRY(cudaMemcpyAsync(c.host_ptr, c.dev_ptr, c.bytes_per_row * (size_t)n_lines, cudaMemcpyDeviceToHost, st));
         for (int c = 0; c < 16; ++c)
             MDG_CUDA_TRY(cudaMemcpyAsync(counts16 + (size_t)c * counts_stride, tl.counts16 + (size_t)c * tl.stride,
                                          (size_t)n_lines * 4, cudaMemcpyDeviceToHost, st));
     }
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[3], st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_end, st));
     MDG_CUDA_TRY(cudaStreamSynchronize(st));
-    ctx->timings.counts_ms = elapsed(ctx->ev[1], ctx->ev[2]);
-    ctx->timings.total_ms = elapsed(ctx->ev[0], ctx->ev[3]);
+    ctx->timings.counts_ms = elapsed(ctx->work_begin, ctx->work_end);
+    ctx->timings.total_ms = elapsed(ctx->call_begin, ctx->call_end);
     if (h_err[0] != TE_NONE) {
         static const char* what[] = {"", "wrong number of fields", "malformed number", "value out of range", ""};
         set_error("mdg_tsv_parse: %s in data line %lld", what[h_err[0] & 3], h_line + 1);
@@ -849,57 +811,37 @@ int mdg_select_top(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_id_
         set_error("mdg_select_top: invalid argument");
         return MDG_ERR_INVALID;
     }
-    MDG_CUDA_TRY(cudaSetDevice(ctx->device));
+    DeviceGuard guard(ctx->device);
     cudaStream_t st = ctx->stream;
     ctx->timings = mdg_timings{};
     const long long take = std::min<long long>(n_top, n_tax);
     *out_n = take;
     if (n_tax == 0 || (take == 0 && !out_weight)) { *out_n = 0; return MDG_OK; }
-    const bool host = (mem == MDG_HOST);
     const size_t nr = (size_t)n_rows, nt = (size_t)n_tax;
-    int rc;
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
-    const long long* d_tax_row = reinterpret_cast<const long long*>(tax_id_row);
-    const uint32_t* d_nal_row = n_alignments_row; const uint8_t* d_keep = keep_row;
-    const long long* d_tax = reinterpret_cast<const long long*>(tax_id);
-    const long long* d_first = reinterpret_cast<const long long*>(first_row);
-    unsigned long long* d_weight = reinterpret_cast<unsigned long long*>(out_weight);
-    long long* d_index = reinterpret_cast<long long*>(out_index);
-    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    if (host) {
-        const size_t in_bytes = up(nr * 8) + up(nr * 4) + up(nr) + 2 * up(nt * 8);
-        if ((rc = ctx->order_tsv_top_in.ensure(in_bytes))) return rc;
-        unsigned char* b = ctx->order_tsv_top_in.as<unsigned char>();
-        size_t o = 0;
-        auto put = [&](const void* src, size_t bytes) -> void* {
-            void* d = b + o; o += up(bytes);
-            if (src) cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, st);
-            return d;
-        };
-        d_tax_row = (const long long*)put(tax_id_row, nr * 8);
-        d_nal_row = (const uint32_t*)put(n_alignments_row, nr * 4);
-        void* kp = put(keep_row, nr);
-        d_keep = keep_row ? (const uint8_t*)kp : nullptr;
-        d_tax = (const long long*)put(tax_id, nt * 8);
-        d_first = (const long long*)put(first_row, nt * 8);
-        MDG_CUDA_TRY(cudaGetLastError());
-    }
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_begin, st));
     const int n_blocks = (int)((n_tax + kTopThreads - 1) / kTopThreads);
-    const size_t scratch = up(kTopPasses * 256 * 4) + up((size_t)n_blocks * 4) + up((size_t)n_blocks * 8) + up(8) +
-                           ((host || !out_weight) ? up(nt * 8) : 0) + (host ? up((size_t)take * 8 + 8) : 0);
-    if ((rc = ctx->order_tsv_top_scratch.ensure(scratch))) return rc;
-    unsigned char* sb = ctx->order_tsv_top_scratch.as<unsigned char>();
-    size_t so = 0;
-    auto carve = [&](size_t bytes) { void* q = sb + so; so += up(bytes); return q; };
     TopLaunch tl = {};
     tl.n_tax = n_tax; tl.n_top = take;
-    tl.hist = (unsigned int*)carve(kTopPasses * 256 * 4);
-    tl.block_cnt = (int*)carve((size_t)n_blocks * 4);
-    tl.block_base = (long long*)carve((size_t)n_blocks * 8);
-    long long* d_total = (long long*)carve(8);
-    if (host || !out_weight) d_weight = (unsigned long long*)carve(nt * 8);
-    if (host) d_index = (long long*)carve((size_t)take * 8 + 8);
-    tl.weight = d_weight; tl.tax_id = d_tax; tl.out_index = d_index;
+    const long long *d_tax_row, *d_first;
+    const uint32_t* d_nal_row;
+    const uint8_t* d_keep;
+    unsigned long long* d_weight;
+    long long* d_total;
+    Stage stage(ctx->arena, mem == MDG_HOST, st);
+    stage.in(d_tax_row, tax_id_row, nr * 8);
+    stage.in(d_nal_row, n_alignments_row, nr * 4);
+    stage.in(d_keep, keep_row, nr);
+    stage.in(tl.tax_id, tax_id, nt * 8);
+    stage.in(d_first, first_row, nt * 8);
+    stage.out(tl.out_index, out_index, 8, (size_t)take);
+    if (out_weight) stage.out_all(d_weight, out_weight, nt * 8);
+    else stage.scratch(d_weight, nt * 8);
+    stage.scratch(tl.hist, kTopPasses * 256 * 4);
+    stage.scratch(tl.block_cnt, (size_t)n_blocks * 4);
+    stage.scratch(tl.block_base, (size_t)n_blocks * 8);
+    stage.scratch(d_total, 8);
+    if (int rc = stage.commit()) return rc;
+    tl.weight = d_weight;
     MDG_CUDA_TRY(cudaMemsetAsync(tl.hist, 0, kTopPasses * 256 * 4, st));
     top_weight_kernel<<<(unsigned)((n_tax * 32 + kTopThreads - 1) / kTopThreads), kTopThreads, 0, st>>>(
         n_rows, d_tax_row, d_nal_row, d_keep, n_tax, d_first, d_weight);
@@ -924,17 +866,12 @@ int mdg_select_top(mdg_ctx* ctx, int mem, int64_t n_rows, const int64_t* tax_id_
         MDG_CUDA_TRY(cudaGetLastError());
         ctx->timings.n_launches += 3;
     }
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[9], st));
-    if (host) {
-        if (take > 0) MDG_CUDA_TRY(cudaMemcpyAsync(out_index, d_index, (size_t)take * 8, cudaMemcpyDeviceToHost, st));
-        if (out_weight) MDG_CUDA_TRY(cudaMemcpyAsync(out_weight, d_weight, nt * 8, cudaMemcpyDeviceToHost, st));
-    }
+    MDG_CUDA_TRY(cudaEventRecord(ctx->work_end, st));
+    if (int rc = stage.copy_back(0, (size_t)take, st)) return rc;
     long long h_total = 0;
     MDG_CUDA_TRY(cudaMemcpyAsync(&h_total, d_total, 8, cudaMemcpyDeviceToHost, st));
     MDG_CUDA_TRY(cudaStreamSynchronize(st));
-    float ms = 0;
-    cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[9]);
-    ctx->timings.total_ms = ms;
+    ctx->timings.total_ms = elapsed(ctx->call_begin, ctx->work_end);
     if (h_total != take) {
         set_error("mdg_select_top: selected %lld of %lld (duplicate tax ids in the per-TaxID arrays?)", h_total, take);
         return MDG_ERR_INVALID;
@@ -954,18 +891,18 @@ double ms_since_epoch(mdg_ctx* ctx, cudaEvent_t ev) { return (double)elapsed(ctx
 // Wait (on the host) for the chunk in flight on a lane and book its CUDA-event times on its ticket.
 int harvest_lane(mdg_ctx* ctx, mdg_fit_lane& ln) {
     if (!ln.busy) return MDG_OK;
-    MDG_CUDA_TRY(cudaEventSynchronize(ln.ev[4]));
+    MDG_CUDA_TRY(cudaEventSynchronize(ln.done));
     mdg_fit_ticket_slot& tk = ctx->ticket[ln.owner];
-    tk.t.map_ms += elapsed(ln.ev[0], ln.ev[1]);
-    tk.t.nuts_ms += elapsed(ln.ev[1], ln.ev[2]);
-    tk.t.ppc_ms += elapsed(ln.ev[2], ln.ev[3]);
-    tk.t.assemble_ms += elapsed(ln.ev[3], ln.ev[4]);
-    tk.t.total_ms = std::max(tk.t.total_ms, elapsed(tk.ev_begin, ln.ev[4]));
+    tk.t.map_ms += elapsed(ln.begin, ln.map_end);
+    tk.t.nuts_ms += elapsed(ln.map_end, ln.nuts_end);
+    tk.t.ppc_ms += elapsed(ln.nuts_end, ln.pred_end);
+    tk.t.assemble_ms += elapsed(ln.pred_end, ln.done);
+    tk.t.total_ms = std::max(tk.t.total_ms, elapsed(tk.ev_begin, ln.done));
     tk.t.n_launches += ln.launches;
     for (int r = 0; r < MDG_NUM_RUNS; ++r) tk.t.leapfrogs[r] += ln.h_leap[r];
     // NUTS-active time as a union of intervals over everything harvested on this ctx (chunks of overlapping
     // batches run their NUTS launches concurrently; chunks are harvested in submission order)
-    const double a = ms_since_epoch(ctx, ln.ev[1]), b = ms_since_epoch(ctx, ln.ev[2]);
+    const double a = ms_since_epoch(ctx, ln.map_end), b = ms_since_epoch(ctx, ln.nuts_end);
     tk.t.nuts_union_ms += (float)std::max(0.0, b - std::max(a, ctx->nuts_covered_until_ms));
     ctx->nuts_covered_until_ms = std::max(ctx->nuts_covered_until_ms, b);
     if (!tk.have_nuts) { tk.nuts_begin_ms = a; tk.nuts_end_ms = b; tk.have_nuts = true; }
@@ -981,6 +918,35 @@ int harvest_lane(mdg_ctx* ctx, mdg_fit_lane& ln) {
     ln.busy = false;
     ln.owner = -1;
     return MDG_OK;
+}
+
+// Frees the slot of a batch whose submit failed, after waiting for its chunks already enqueued: no lane may keep an
+// owner that points at a free slot, and the next batch must not stage into the slot's arena under a running chunk.
+void abandon_ticket(mdg_ctx* ctx, int slot) {
+    const std::string error = g_error;  // the submit's error, not one of the waits'
+    for (auto& ln : ctx->lane)
+        if (ln.busy && ln.owner == slot && harvest_lane(ctx, ln) != MDG_OK) {
+            ln.busy = false;
+            ln.owner = -1;
+        }
+    ctx->ticket[slot].active = false;
+    set_error("%s", error.c_str());
+}
+
+// the five per-TaxID inputs of mdg_fit_batch_submit and mdg_map_batch
+struct FitInputs {
+    const int64_t* tax;
+    const uint32_t *k, *N, *m12;
+    const double* noise;
+};
+
+void stage_fit_inputs(Stage& stage, FitInputs& d, size_t nt, int R, const int64_t* tax_id, const uint32_t* k,
+                      const uint32_t* N, const uint32_t* mism12, const double* noise3) {
+    stage.in(d.tax, tax_id, nt * 8);
+    stage.in(d.k, k, nt * R * 4);
+    stage.in(d.N, N, nt * R * 4);
+    stage.in(d.m12, mism12, nt * R * 12 * 4);
+    stage.in(d.noise, noise3, nt * 24);
 }
 
 }  // namespace
@@ -1018,8 +984,20 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
     tk.id = ctx->next_ticket_id++;
     tk.active = true;
     *out_ticket = tk.id;
+    // from here on every error return frees the slot again
+    struct Abandon {
+        mdg_ctx* ctx;
+        int slot;
+        bool armed = true;
+        ~Abandon() {
+            if (armed) abandon_ticket(ctx, slot);
+        }
+    } abandon{ctx, slot};
     MDG_CUDA_TRY(cudaEventRecord(tk.ev_begin, st));
-    if (n_tax == 0) return MDG_OK;
+    if (n_tax == 0) {
+        abandon.armed = false;
+        return MDG_OK;
+    }
     const int P = max_position, R = 2 * P, S = cfg->num_samples, W = cfg->num_warmup;
     const bool host = (mem == MDG_HOST);
     const bool fwd_rev = cfg->do_fwd_rev != 0;
@@ -1039,62 +1017,30 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
     }
     const long long chunk_max = std::min<long long>(n_tax, chunk_cap);
 
-    // ---- staged inputs / outputs for MDG_HOST (whole batch, owned by the ticket) ----
+    // ---- the caller's buffers (MDG_DEVICE) or staged ones (MDG_HOST: whole batch, owned by the ticket) ----
     int rc;
-    const int64_t* d_tax = tax_id; const uint32_t* d_k = k; const uint32_t* d_N = N; const uint32_t* d_m12 = mism12;
-    const double* d_noise = noise3;
-    mdg_fit_result* d_out = out; float* d_med = out_median; float* d_lo = out_hpdi_lo; float* d_hi = out_hpdi_hi;
-    double* d_samples = out_samples; double* d_trace = out_trace; double* d_waic_user = out_waic;
     const size_t nt = (size_t)n_tax;
-    auto bail = [&](int code) { tk.active = false; return code; };
-    if (host) {
-        if ((rc = tk.in_tax.ensure(nt * 8))) return bail(rc);
-        if ((rc = tk.in_k.ensure(nt * R * 4))) return bail(rc);
-        if ((rc = tk.in_N.ensure(nt * R * 4))) return bail(rc);
-        MDG_CUDA_TRY(cudaMemcpyAsync(tk.in_tax.ptr, tax_id, nt * 8, cudaMemcpyHostToDevice, st));
-        MDG_CUDA_TRY(cudaMemcpyAsync(tk.in_k.ptr, k, nt * R * 4, cudaMemcpyHostToDevice, st));
-        MDG_CUDA_TRY(cudaMemcpyAsync(tk.in_N.ptr, N, nt * R * 4, cudaMemcpyHostToDevice, st));
-        d_tax = tk.in_tax.as<int64_t>(); d_k = tk.in_k.as<uint32_t>(); d_N = tk.in_N.as<uint32_t>();
-        if (mism12) {
-            if ((rc = tk.in_m12.ensure(nt * R * 12 * 4))) return bail(rc);
-            MDG_CUDA_TRY(cudaMemcpyAsync(tk.in_m12.ptr, mism12, nt * R * 12 * 4, cudaMemcpyHostToDevice, st));
-            d_m12 = tk.in_m12.as<uint32_t>();
-        }
-        if (noise3) {
-            if ((rc = tk.in_noise.ensure(nt * 24))) return bail(rc);
-            MDG_CUDA_TRY(cudaMemcpyAsync(tk.in_noise.ptr, noise3, nt * 24, cudaMemcpyHostToDevice, st));
-            d_noise = tk.in_noise.as<double>();
-        }
-        if ((rc = tk.out_res.ensure(nt * sizeof(mdg_fit_result)))) return bail(rc);
-        d_out = tk.out_res.as<mdg_fit_result>();
-        if ((rc = tk.out_med.ensure(nt * R * 4 * 3))) return bail(rc);
-        d_med = tk.out_med.as<float>(); d_lo = d_med + nt * R; d_hi = d_lo + nt * R;
-        if (out_samples) {
-            if ((rc = tk.smp.ensure(nt * MDG_NUM_RUNS * S * 4 * 8))) return bail(rc);
-            d_samples = tk.smp.as<double>();
-        }
-        if (out_trace) {
-            if ((rc = tk.trace.ensure(nt * MDG_NUM_RUNS * (size_t)(W + S) * 4 * 8))) return bail(rc);
-            d_trace = tk.trace.as<double>();
-        }
-        if (out_waic) {
-            if ((rc = tk.waic.ensure(nt * MDG_NUM_RUNS * 2 * R * 8))) return bail(rc);
-            d_waic_user = tk.waic.as<double>();
-        }
-    } else {
-        if (!d_med || !d_lo || !d_hi) {
-            if ((rc = tk.out_med.ensure(nt * R * 4 * 3))) return bail(rc);
-            float* base = tk.out_med.as<float>();
-            if (!d_med) d_med = base;
-            if (!d_lo) d_lo = base + nt * R;
-            if (!d_hi) d_hi = base + 2 * nt * R;
-        }
+    FitInputs d;
+    mdg_fit_result* d_out;
+    float *d_med, *d_lo, *d_hi;
+    double *d_samples, *d_trace, *d_waic_user;
+    Stage stage(tk.arena, host, st);
+    stage_fit_inputs(stage, d, nt, R, tax_id, k, N, mism12, noise3);
+    stage.out(d_out, out, sizeof(mdg_fit_result), nt);
+    // the assembly writes the medians and HPDI bounds whether or not the caller wants them
+    for (auto [field, dst] : {std::make_pair(&d_med, out_median), std::make_pair(&d_lo, out_hpdi_lo), std::make_pair(&d_hi, out_hpdi_hi)}) {
+        if (dst) stage.out(*field, dst, (size_t)R * 4, nt);
+        else stage.scratch(*field, nt * R * 4);
     }
+    stage.out(d_samples, out_samples, (size_t)MDG_NUM_RUNS * S * 4 * 8, nt);
+    stage.out(d_trace, out_trace, (size_t)MDG_NUM_RUNS * (W + S) * 4 * 8, nt);
+    stage.out(d_waic_user, out_waic, (size_t)MDG_NUM_RUNS * 2 * R * 8, nt);
+    if ((rc = stage.commit())) return rc;
     if (!ctx->da_tables.ptr) {
         // the same libm calls as the reference arithmetic (t^-0.75 by pow, sqrt), made once on the host
         std::vector<double> tab(2 * kDaTable);
         for (int t = 0; t < kDaTable; ++t) { tab[t] = sqrt((double)t); tab[kDaTable + t] = t ? pow((double)t, -0.75) : 0.0; }
-        if ((rc = ctx->da_tables.ensure(tab.size() * sizeof(double)))) return bail(rc);
+        if ((rc = ctx->da_tables.ensure(tab.size() * sizeof(double)))) return rc;
         MDG_CUDA_TRY(cudaMemcpyAsync(ctx->da_tables.ptr, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, st));
         MDG_CUDA_TRY(cudaStreamSynchronize(st));  // `tab` is a stack-lifetime source
     }
@@ -1108,14 +1054,14 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
         const int nc = (int)std::min<long long>(chunk_cap, n_tax - c0);
         mdg_fit_lane& ln = ctx->lane[ctx->next_lane];
         ctx->next_lane = (ctx->next_lane + 1) % kFitLanes;
-        if ((rc = harvest_lane(ctx, ln))) return bail(rc);  // the lane's previous chunk (host wait only if it is still running)
+        if ((rc = harvest_lane(ctx, ln))) return rc;  // the lane's previous chunk (host wait only if it is still running)
         // ---- per-lane scratch ----
-        if ((rc = ln.rec.ensure((size_t)chunk_max * MDG_NUM_RUNS * sizeof(RunRecord)))) return bail(rc);
-        if ((rc = ln.map.ensure((size_t)chunk_max * 2 * sizeof(MapRecord)))) return bail(rc);
-        if ((rc = ln.pred.ensure((size_t)chunk_max * items_per_tax * 3 * sizeof(double)))) return bail(rc);
-        if ((rc = ln.counters.ensure(256))) return bail(rc);  // work counters + leapfrog totals
-        if (!out_samples && (rc = ln.samples.ensure((size_t)chunk_max * sample_runs * S * 4 * sizeof(double)))) return bail(rc);
-        if (!out_waic && (rc = ln.waic.ensure((size_t)chunk_max * MDG_NUM_RUNS * 2 * R * sizeof(double)))) return bail(rc);
+        if ((rc = ln.rec.ensure((size_t)chunk_max * MDG_NUM_RUNS * sizeof(RunRecord)))) return rc;
+        if ((rc = ln.map.ensure((size_t)chunk_max * 2 * sizeof(MapRecord)))) return rc;
+        if ((rc = ln.pred.ensure((size_t)chunk_max * items_per_tax * 3 * sizeof(double)))) return rc;
+        if ((rc = ln.counters.ensure(256))) return rc;  // work counters + leapfrog totals
+        if (!out_samples && (rc = ln.samples.ensure((size_t)chunk_max * sample_runs * S * 4 * sizeof(double)))) return rc;
+        if (!out_waic && (rc = ln.waic.ensure((size_t)chunk_max * MDG_NUM_RUNS * 2 * R * sizeof(double)))) return rc;
         cudaStream_t ls = ln.main;
         const uint32_t launches_before = ctx->timings.n_launches;
         MDG_CUDA_TRY(cudaStreamWaitEvent(ls, ctx->inputs_ready, 0));
@@ -1131,18 +1077,18 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
         MDG_CUDA_TRY(cudaMemsetAsync(d_rec, 0, (size_t)nc * MDG_NUM_RUNS * sizeof(RunRecord), ls));
 
         // ---- K3 MAP ----
-        MDG_CUDA_TRY(cudaEventRecord(ln.ev[0], ls));
+        MDG_CUDA_TRY(cudaEventRecord(ln.begin, ls));
         if (cfg->do_map) {
             MapLaunch ml = {};
-            ml.tax_id = d_tax + c0; ml.k = d_k + (size_t)c0 * R; ml.N = d_N + (size_t)c0 * R;
+            ml.tax_id = d.tax + c0; ml.k = d.k + (size_t)c0 * R; ml.N = d.N + (size_t)c0 * R;
             ml.n_tax = nc; ml.P = P; ml.pr = pr; ml.work_counter = d_counters + 0; ml.rec = d_map;
-            if ((rc = launch_map(ctx, ls, ml, npl_for(R, 32)))) return bail(rc);
+            if ((rc = launch_map(ctx, ls, ml))) return rc;
         }
-        MDG_CUDA_TRY(cudaEventRecord(ln.ev[1], ls));
+        MDG_CUDA_TRY(cudaEventRecord(ln.map_end, ls));
 
         // ---- K4 NUTS: one launch per model, each on its own stream (they share the SMs as CTAs retire) ----
         FitLaunch fl = {};
-        fl.tax_id = d_tax + c0; fl.k = d_k + (size_t)c0 * R; fl.N = d_N + (size_t)c0 * R;
+        fl.tax_id = d.tax + c0; fl.k = d.k + (size_t)c0 * R; fl.N = d.N + (size_t)c0 * R;
         fl.n_tax = nc; fl.P = P; fl.cfg = *cfg; fl.pr = pr;
         fl.n_windows = adaptation_window_ends(W, fl.win_end);
         fl.rec = d_rec; fl.waic = d_waic; fl.samples = d_smp; fl.sample_runs = sample_runs;
@@ -1155,7 +1101,7 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
         const int order_mode = env_int("MDG_NUTS_ORDER", 1);
         if (order_mode == 2 || (order_mode == 1 && nc >= kOrderMinChunk)) {
             const size_t off_bucket = (size_t)chunk_max * sizeof(int), off_cnt = (off_bucket + (size_t)chunk_max + 15) & ~(size_t)15;
-            if ((rc = ln.order.ensure(off_cnt + 3 * kOrderBuckets * sizeof(unsigned int)))) return bail(rc);
+            if ((rc = ln.order.ensure(off_cnt + 3 * kOrderBuckets * sizeof(unsigned int)))) return rc;
             int* d_order = ln.order.as<int>();
             unsigned char* d_bucket = ln.order.as<unsigned char>() + off_bucket;
             unsigned int* d_cnt = reinterpret_cast<unsigned int*>(ln.order.as<unsigned char>() + off_cnt);
@@ -1175,7 +1121,7 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
             fl.n_prio = (fwd_rev && fl.order != nullptr && frac > 0) ? nc / frac : 0;
         }
         if (getenv("MDG_CHAIN_CLOCK")) {
-            if ((rc = ln.chain_clock.ensure((size_t)chunk_max * MDG_NUM_RUNS * 16))) return bail(rc);
+            if ((rc = ln.chain_clock.ensure((size_t)chunk_max * MDG_NUM_RUNS * 16))) return rc;
             MDG_CUDA_TRY(cudaMemsetAsync(ln.chain_clock.ptr, 0, (size_t)nc * MDG_NUM_RUNS * 16, ls));
             fl.chain_clock = ln.chain_clock.as<unsigned long long>();
             ln.clock_items = nc * MDG_NUM_RUNS;
@@ -1186,9 +1132,9 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
         // until the other chunk's PMD launch is through and only its null launch (short, uniform chains) is still
         // running.
         for (auto& other : ctx->lane)
-            if (&other != &ln && other.busy) MDG_CUDA_TRY(cudaStreamWaitEvent(ls, other.join_ev[0], 0));
-        MDG_CUDA_TRY(cudaEventRecord(ln.fork_ev, ls));
-        for (cudaStream_t sd : ln.side) MDG_CUDA_TRY(cudaStreamWaitEvent(sd, ln.fork_ev, 0));
+            if (&other != &ln && other.busy) MDG_CUDA_TRY(cudaStreamWaitEvent(ls, other.nuts_join[0], 0));
+        MDG_CUDA_TRY(cudaEventRecord(ln.nuts_fork, ls));
+        for (cudaStream_t sd : ln.side) MDG_CUDA_TRY(cudaStreamWaitEvent(sd, ln.nuts_fork, 0));
         {
             // Launch order = dispatch order of the persistent CTAs: the kernels share the SMs as CTAs
             // retire, so the whole step behaves like one list schedule over all (TaxID, run) items.
@@ -1202,19 +1148,19 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
             a.n_items = fwd_rev ? 3 * nc : nc; a.n_items_all = nc; a.work_counter = d_counters + 1;
             FitLaunch b = a;   // null
             b.work_counter = d_counters + 2;
-            if ((rc = launch_nuts_group<0>(ctx, ln.side[0], a, ln.waic_acc[0]))) return bail(rc);
-            if ((rc = launch_nuts_group<1>(ctx, ln.side[1], b, ln.waic_acc[1]))) return bail(rc);
+            if ((rc = launch_nuts_group<0>(ctx, ln.side[0], a, ln.waic_acc[0]))) return rc;
+            if ((rc = launch_nuts_group<1>(ctx, ln.side[1], b, ln.waic_acc[1]))) return rc;
         }
         for (int m = 0; m < 2; ++m) {
-            MDG_CUDA_TRY(cudaEventRecord(ln.join_ev[m], ln.side[m]));
-            MDG_CUDA_TRY(cudaStreamWaitEvent(ls, ln.join_ev[m], 0));
+            MDG_CUDA_TRY(cudaEventRecord(ln.nuts_join[m], ln.side[m]));
+            MDG_CUDA_TRY(cudaStreamWaitEvent(ls, ln.nuts_join[m], 0));
         }
-        MDG_CUDA_TRY(cudaEventRecord(ln.ev[2], ls));
+        MDG_CUDA_TRY(cudaEventRecord(ln.nuts_end, ls));
 
         // ---- K6 posterior predictive ----
         {
             PpcLaunch pl = {};
-            pl.tax_id = d_tax + c0; pl.N = d_N + (size_t)c0 * R; pl.n_tax = nc; pl.P = P; pl.cfg = *cfg; pl.pr = pr;
+            pl.tax_id = d.tax + c0; pl.N = d.N + (size_t)c0 * R; pl.n_tax = nc; pl.P = P; pl.cfg = *cfg; pl.pr = pr;
             pl.samples = d_smp; pl.sample_runs = sample_runs;
             for (int r = 0; r < MDG_NUM_RUNS; ++r) pl.sample_slot[r] = fl.sample_slot[r];
             pl.rec = d_rec; pl.work_counter = d_counters + 5; pl.items_per_tax = items_per_tax;
@@ -1229,14 +1175,14 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
             MDG_CUDA_TRY(cudaGetLastError());
             ctx->timings.n_launches++;
         }
-        MDG_CUDA_TRY(cudaEventRecord(ln.ev[3], ls));
+        MDG_CUDA_TRY(cudaEventRecord(ln.pred_end, ls));
 
         // ---- K5/K7 assembly ----
         {
             AssembleLaunch al = {};
-            al.tax_id = d_tax + c0; al.k = d_k + (size_t)c0 * R; al.N = d_N + (size_t)c0 * R;
-            al.mism12 = d_m12 ? d_m12 + (size_t)c0 * R * 12 : nullptr;
-            al.noise3 = d_noise ? d_noise + (size_t)c0 * 3 : nullptr;
+            al.tax_id = d.tax + c0; al.k = d.k + (size_t)c0 * R; al.N = d.N + (size_t)c0 * R;
+            al.mism12 = d.m12 ? d.m12 + (size_t)c0 * R * 12 : nullptr;
+            al.noise3 = d.noise ? d.noise + (size_t)c0 * 3 : nullptr;
             al.n_tax = nc; al.P = P; al.cfg = *cfg; al.rec = d_rec; al.map = cfg->do_map ? d_map : nullptr;
             al.waic = d_waic; al.pred = d_pred; al.items_per_tax = items_per_tax;
             al.out = d_out + c0; al.out_median = d_med + (size_t)c0 * R; al.out_lo = d_lo + (size_t)c0 * R;
@@ -1246,23 +1192,14 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
             ctx->timings.n_launches++;
         }
         // ---- this chunk's results back to the caller's host buffers ----
-        if (host) {
-            const size_t o = (size_t)c0, n_ = (size_t)nc;
-            MDG_CUDA_TRY(cudaMemcpyAsync(out + o, d_out + o, n_ * sizeof(mdg_fit_result), cudaMemcpyDeviceToHost, ls));
-            if (out_median) MDG_CUDA_TRY(cudaMemcpyAsync(out_median + o * R, d_med + o * R, n_ * R * 4, cudaMemcpyDeviceToHost, ls));
-            if (out_hpdi_lo) MDG_CUDA_TRY(cudaMemcpyAsync(out_hpdi_lo + o * R, d_lo + o * R, n_ * R * 4, cudaMemcpyDeviceToHost, ls));
-            if (out_hpdi_hi) MDG_CUDA_TRY(cudaMemcpyAsync(out_hpdi_hi + o * R, d_hi + o * R, n_ * R * 4, cudaMemcpyDeviceToHost, ls));
-            const size_t so = o * MDG_NUM_RUNS * S * 4, to = o * MDG_NUM_RUNS * (size_t)(W + S) * 4, wo = o * MDG_NUM_RUNS * 2 * R;
-            if (out_samples) MDG_CUDA_TRY(cudaMemcpyAsync(out_samples + so, d_samples + so, n_ * MDG_NUM_RUNS * S * 4 * 8, cudaMemcpyDeviceToHost, ls));
-            if (out_trace) MDG_CUDA_TRY(cudaMemcpyAsync(out_trace + to, d_trace + to, n_ * MDG_NUM_RUNS * (size_t)(W + S) * 4 * 8, cudaMemcpyDeviceToHost, ls));
-            if (out_waic) MDG_CUDA_TRY(cudaMemcpyAsync(out_waic + wo, d_waic_user + wo, n_ * MDG_NUM_RUNS * 2 * R * 8, cudaMemcpyDeviceToHost, ls));
-        }
+        if ((rc = stage.copy_back((size_t)c0, (size_t)nc, ls))) return rc;
         MDG_CUDA_TRY(cudaMemcpyAsync(ln.h_leap, d_leap, MDG_NUM_RUNS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ls));
-        MDG_CUDA_TRY(cudaEventRecord(ln.ev[4], ls));
+        MDG_CUDA_TRY(cudaEventRecord(ln.done, ls));
         ln.launches = ctx->timings.n_launches - launches_before;
         ln.busy = true;
         ln.owner = slot;
     }
+    abandon.armed = false;
     return MDG_OK;
 }
 
@@ -1278,7 +1215,7 @@ int mdg_fit_batch_wait(mdg_ctx* ctx, int64_t ticket, mdg_timings* out_timings) {
         mdg_fit_lane& ln = ctx->lane[(ctx->next_lane + i) % kFitLanes];
         if (ln.busy && ln.owner == slot) {
             // later work on the ctx stream (e.g. the caller's consumers of device-resident results) follows the chunk
-            MDG_CUDA_TRY(cudaStreamWaitEvent(ctx->stream, ln.ev[4], 0));
+            MDG_CUDA_TRY(cudaStreamWaitEvent(ctx->stream, ln.done, 0));
             int rc = harvest_lane(ctx, ln);
             if (rc) return rc;
         }
@@ -1315,73 +1252,53 @@ int mdg_map_batch(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position, const 
     ctx->timings = mdg_timings{};
     const int P = max_position, R = 2 * P;
     const int n_runs = cfg->do_fwd_rev ? MDG_NUM_RUNS : 2;
-    const bool host = (mem == MDG_HOST);
     const size_t nt = (size_t)n_tax;
     // TaxIDs per piece: bounds the per-run records (624 MB per 2^20 TaxIDs); results go straight to their rows
     const long long piece = 1ll << 20;
     const long long piece_max = std::min<long long>(n_tax, piece);
     int rc;
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
-    const int64_t* d_tax = tax_id; const uint32_t* d_k = k; const uint32_t* d_N = N; const uint32_t* d_m12 = mism12;
-    const double* d_noise = noise3;
-    mdg_map_result* d_out = out;
-    if (n_tax > 0 && host) {
-        if ((rc = ctx->map_in_tax.ensure(nt * 8))) return rc;
-        if ((rc = ctx->map_in_k.ensure(nt * R * 4))) return rc;
-        if ((rc = ctx->map_in_N.ensure(nt * R * 4))) return rc;
-        MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_tax.ptr, tax_id, nt * 8, cudaMemcpyHostToDevice, st));
-        MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_k.ptr, k, nt * R * 4, cudaMemcpyHostToDevice, st));
-        MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_N.ptr, N, nt * R * 4, cudaMemcpyHostToDevice, st));
-        d_tax = ctx->map_in_tax.as<int64_t>(); d_k = ctx->map_in_k.as<uint32_t>(); d_N = ctx->map_in_N.as<uint32_t>();
-        if (mism12) {
-            if ((rc = ctx->map_in_m12.ensure(nt * R * 12 * 4))) return rc;
-            MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_m12.ptr, mism12, nt * R * 12 * 4, cudaMemcpyHostToDevice, st));
-            d_m12 = ctx->map_in_m12.as<uint32_t>();
-        }
-        if (noise3) {
-            if ((rc = ctx->map_in_noise.ensure(nt * 24))) return rc;
-            MDG_CUDA_TRY(cudaMemcpyAsync(ctx->map_in_noise.ptr, noise3, nt * 24, cudaMemcpyHostToDevice, st));
-            d_noise = ctx->map_in_noise.as<double>();
-        }
-        if ((rc = ctx->map_out.ensure(nt * sizeof(mdg_map_result)))) return rc;
-        d_out = ctx->map_out.as<mdg_map_result>();
-    }
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_begin, st));
+    FitInputs d;
+    mdg_map_result* d_out;
+    Stage stage(ctx->arena, mem == MDG_HOST, st);
+    stage_fit_inputs(stage, d, nt, R, tax_id, k, N, mism12, noise3);
+    stage.out(d_out, out, sizeof(mdg_map_result), nt);
+    if ((rc = stage.commit())) return rc;
     if ((rc = ctx->map_counters.ensure(256))) return rc;
     unsigned int* d_counter = ctx->map_counters.as<unsigned int>();                           // [1] work counter
     unsigned long long* d_evals = reinterpret_cast<unsigned long long*>(d_counter + 16);      // [6] gradient evaluations
     MDG_CUDA_TRY(cudaMemsetAsync(d_counter, 0, 256, st));
     if (n_tax > 0 && (rc = ctx->map_rec.ensure((size_t)piece_max * MDG_NUM_RUNS * sizeof(mdg_map_run)))) return rc;
     const Priors pr = make_priors(*cfg);
-    const int npl = npl_for(R, 32);  // map_kernel's layout: the all-position fits are mdg_fit_batch's
     for (long long c0 = 0; c0 < n_tax; c0 += piece) {
         const int nc = (int)std::min<long long>(piece, n_tax - c0);
         if (c0 > 0) MDG_CUDA_TRY(cudaMemsetAsync(d_counter, 0, sizeof(unsigned int), st));
-        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
+        MDG_CUDA_TRY(cudaEventRecord(ctx->work_begin, st));
         MapBatchLaunch ml = {};
-        ml.k = d_k + (size_t)c0 * R; ml.N = d_N + (size_t)c0 * R; ml.n_tax = nc; ml.P = P; ml.n_runs = n_runs;
+        ml.k = d.k + (size_t)c0 * R; ml.N = d.N + (size_t)c0 * R; ml.n_tax = nc; ml.P = P; ml.n_runs = n_runs;
         ml.pr = pr; ml.work_counter = d_counter; ml.rec = ctx->map_rec.as<mdg_map_run>();
-        if ((rc = launch_map_batch(ctx, st, ml, npl))) return rc;
-        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[2], st));
+        if ((rc = launch_map_batch(ctx, st, ml))) return rc;
+        MDG_CUDA_TRY(cudaEventRecord(ctx->work_end, st));
         MapAssembleLaunch al = {};
-        al.tax_id = d_tax + c0; al.k = ml.k; al.N = ml.N;
-        al.mism12 = d_m12 ? d_m12 + (size_t)c0 * R * 12 : nullptr;
-        al.noise3 = d_noise ? d_noise + (size_t)c0 * 3 : nullptr;
+        al.tax_id = d.tax + c0; al.k = ml.k; al.N = ml.N;
+        al.mism12 = d.m12 ? d.m12 + (size_t)c0 * R * 12 : nullptr;
+        al.noise3 = d.noise ? d.noise + (size_t)c0 * 3 : nullptr;
         al.n_tax = nc; al.P = P; al.n_runs = n_runs; al.rec = ml.rec; al.out = d_out + c0; al.eval_totals = d_evals;
         map_assemble_kernel<<<(nc + 127) / 128, 128, 0, st>>>(al);
         MDG_CUDA_TRY(cudaGetLastError());
         ctx->timings.n_launches++;
-        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[3], st));
-        MDG_CUDA_TRY(cudaEventSynchronize(ctx->ev[3]));  // the events are reused by the next piece
-        ctx->timings.map_ms += elapsed(ctx->ev[1], ctx->ev[2]);
-        ctx->timings.assemble_ms += elapsed(ctx->ev[2], ctx->ev[3]);
+        MDG_CUDA_TRY(cudaEventRecord(ctx->call_end, st));  // the piece's end here; the call's at the end
+        MDG_CUDA_TRY(cudaEventSynchronize(ctx->call_end));  // the events are reused by the next piece
+        ctx->timings.map_ms += elapsed(ctx->work_begin, ctx->work_end);
+        ctx->timings.assemble_ms += elapsed(ctx->work_end, ctx->call_end);
     }
-    if (n_tax > 0 && host) MDG_CUDA_TRY(cudaMemcpyAsync(out, d_out, nt * sizeof(mdg_map_result), cudaMemcpyDeviceToHost, st));
+    if ((rc = stage.copy_back(0, nt, st))) return rc;
     unsigned long long evals[MDG_NUM_RUNS];
     MDG_CUDA_TRY(cudaMemcpyAsync(evals, d_evals, sizeof evals, cudaMemcpyDeviceToHost, st));
-    MDG_CUDA_TRY(cudaEventRecord(ctx->ev[4], st));
-    MDG_CUDA_TRY(cudaEventSynchronize(ctx->ev[4]));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_end, st));
+    MDG_CUDA_TRY(cudaEventSynchronize(ctx->call_end));
     for (int r = 0; r < MDG_NUM_RUNS; ++r) ctx->timings.leapfrogs[r] = evals[r];
-    ctx->timings.total_ms = elapsed(ctx->ev[0], ctx->ev[4]);
+    ctx->timings.total_ms = elapsed(ctx->call_begin, ctx->call_end);
     return MDG_OK;
 }
 
@@ -1545,12 +1462,12 @@ int mdg_test_logp_grad(mdg_ctx* ctx, int max_position, const uint32_t* k, const 
     MDG_CUDA_TRY(cudaMemsetAsync(dll, 0, ne * R * 8, st));
     const Priors pr = make_priors(*cfg);
     const int n_obs = lane_mask == 0 ? R : P;
-    const int npl = npl_for(n_obs, 32);
     const unsigned grid = (unsigned)n_eval;
-#define MDG_LAUNCH_LOGP(M, NPL_) test_logp_kernel<M, NPL_><<<grid, 32, 0, st>>>(P, dk, dN, pr, lane_mask, with_jacobian, n_eval, du, dlogp, dgrad, out_ll ? dll : nullptr)
-    if (model == 0) { if (npl == 1) MDG_LAUNCH_LOGP(0, 1); else if (npl == 2) MDG_LAUNCH_LOGP(0, 2); else MDG_LAUNCH_LOGP(0, 4); }
-    else { if (npl == 1) MDG_LAUNCH_LOGP(1, 1); else if (npl == 2) MDG_LAUNCH_LOGP(1, 2); else MDG_LAUNCH_LOGP(1, 4); }
-#undef MDG_LAUNCH_LOGP
+    with_npl(n_obs, [&](auto npl) {
+        constexpr int NPL = decltype(npl)::value;
+        auto kern = model == 0 ? test_logp_kernel<0, NPL> : test_logp_kernel<1, NPL>;
+        kern<<<grid, 32, 0, st>>>(P, dk, dN, pr, lane_mask, with_jacobian, n_eval, du, dlogp, dgrad, out_ll ? dll : nullptr);
+    });
     MDG_CUDA_TRY(cudaGetLastError());
     MDG_CUDA_TRY(cudaMemcpyAsync(out_logp, dlogp, ne * 8, cudaMemcpyDeviceToHost, st));
     MDG_CUDA_TRY(cudaMemcpyAsync(out_grad, dgrad, ne * 32, cudaMemcpyDeviceToHost, st));
@@ -1569,12 +1486,12 @@ int mdg_measure_fp64_peak(mdg_ctx* ctx, double* out_tflops) {
     fp64_peak_kernel<<<blocks, threads, 0, st>>>(ctx->test_scratch.as<double>(), 1000);  // warm-up
     double best = 0.0;
     for (int rep = 0; rep < 3; ++rep) {
-        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[10], st));
+        MDG_CUDA_TRY(cudaEventRecord(ctx->work_begin, st));
         fp64_peak_kernel<<<blocks, threads, 0, st>>>(ctx->test_scratch.as<double>(), iters);
-        MDG_CUDA_TRY(cudaEventRecord(ctx->ev[11], st));
+        MDG_CUDA_TRY(cudaEventRecord(ctx->work_end, st));
         MDG_CUDA_TRY(cudaStreamSynchronize(st));
         MDG_CUDA_TRY(cudaGetLastError());
-        const double ms = elapsed(ctx->ev[10], ctx->ev[11]);
+        const double ms = elapsed(ctx->work_begin, ctx->work_end);
         const double flops = 2.0 * 8.0 * iters * (double)threads * blocks;
         best = std::max(best, flops / (ms * 1e-3) / 1e12);
     }

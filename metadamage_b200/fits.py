@@ -19,8 +19,7 @@ import pandas as pd
 
 from . import _lib, io, utils
 from ._abi import FIT_COV_INVALID, FIT_FAILED, FIT_MAP_NOT_CONVERGED, MAP_RESULT_DTYPE
-from .backend import Context
-from .counts import dense_from_df_counts
+from .counts import dense_from_df_counts, get_context
 from .parallel import run_on_gpus
 
 logger = logging.getLogger(__name__)
@@ -54,15 +53,6 @@ _MAP_RUN_COLUMNS = {
     **{name: (0, name) for name in ("q", "q_std", "A", "A_std", "c", "c_std", "phi", "phi_std", "logp", "loglik")},
     **{"null_" + name: (1, name) for name in ("q", "q_std", "phi", "phi_std", "logp", "loglik")},
 }
-
-_contexts = {}
-
-
-def _context(device):
-    if device not in _contexts:
-        _contexts[device] = Context(device)
-    return _contexts[device]
-
 
 def mcmc_kwargs_default():
     """fits.py:792-799."""
@@ -102,7 +92,7 @@ def fit_dense(dense, cfg, fit_cfg, n_gpus=1):
 
     def worker(rank, start, stop):
         sl = slice(start, stop)
-        return _context(rank).fit_batch(dense["tax_id"][sl], dense["k"][sl], dense["N"][sl], fit_cfg,
+        return get_context(rank).fit_batch(dense["tax_id"][sl], dense["k"][sl], dense["N"][sl], fit_cfg,
                                         mism12=dense["mism12"][sl] if dense.get("mism12") is not None else None,
                                         noise3=dense["noise"][sl] if dense.get("noise") is not None else None)
 
@@ -119,7 +109,7 @@ def map_dense(dense, cfg, fit_cfg, n_gpus=1):
 
     def worker(rank, start, stop):
         sl = slice(start, stop)
-        return _context(rank).map_batch(dense["tax_id"][sl], dense["k"][sl], dense["N"][sl], fit_cfg,
+        return get_context(rank).map_batch(dense["tax_id"][sl], dense["k"][sl], dense["N"][sl], fit_cfg,
                                         mism12=dense["mism12"][sl] if dense.get("mism12") is not None else None,
                                         noise3=dense["noise"][sl] if dense.get("noise") is not None else None)
 
@@ -134,7 +124,7 @@ def select_top_dense(df_counts, dense, n_fits, ctx=None):
     n_tax = len(dense["tax_id"])
     if n_fits is None or n_fits <= 0 or n_fits >= n_tax:
         return dense
-    ctx = ctx or _context(0)
+    ctx = ctx or get_context(0)
     idx = ctx.select_top(df_counts["tax_id"].to_numpy(np.int64), df_counts["N_alignments"].to_numpy(np.uint32), None,
                          dense["tax_id"], dense["first_row"], int(n_fits))
     out = dict(dense)
