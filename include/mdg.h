@@ -253,6 +253,36 @@ MDG_STATIC_ASSERT(offsetof(mdg_map_result, D_max) == 16 && offsetof(mdg_map_resu
                   offsetof(mdg_map_result, N_z1_forward) == 144 && offsetof(mdg_map_result, run) == 208,
                   "mdg_map_result layout");
 
+/*
+ * Profile intervals of D_max = A + c for the MAP-only rows (mdg_map_profile). For one PMD run (all positions,
+ * forward only, reverse only) with mode logp^ at D^ = A + c, the profile of the constrained-space log posterior
+ * (the density the MAP fit maximises: no Jacobian term, log C(N,k) included) is
+ *     pl(D) = max over (q, A, c, phi) with A + c = D of log p(q, A, c, phi | k, N),
+ * and the interval at level alpha is {D : 2 (logp^ - pl(D)) <= t}, t = (Phi^-1((1 + alpha) / 2))^2, the
+ * chi-square(1) quantile. Each end is the root of h(D) = 2 (logp^ - pl(D)) - t on its side of D^. It is a profile
+ * interval of the posterior mode, not an HPDI of the posterior; it respects 0 < D < 1 and may be asymmetric.
+ */
+#define MDG_PROFILE_AT_BOUND 0x20u /* no crossing up to D = 0 / D = 1: the end is that bound */
+#define MDG_PROFILE_FAILED 0x40u   /* root search or an inner fit failed: D is NaN */
+
+typedef struct mdg_profile_end {
+    double D;               /* the interval end */
+    double q, A, c, phi;    /* maximiser of log p on A + c = D (at a bound: of the last point solved, within 1e-9 of it) */
+    double logp;            /* pl(D) */
+    uint32_t n_eval, flags; /* gradient evaluations spent on this end; MDG_PROFILE_* / MDG_FIT_FAILED (run unusable) */
+} mdg_profile_end;
+
+typedef struct mdg_map_interval {
+    int64_t tax_id;
+    uint32_t status;           /* OR of the flags of the two all-position ends */
+    uint32_t reserved;
+    double level, threshold;   /* alpha, t */
+    mdg_profile_end end[3][2]; /* [all, forward, reverse][lower, upper] */
+} mdg_map_interval;
+
+MDG_STATIC_ASSERT(sizeof(mdg_profile_end) == 56 && offsetof(mdg_profile_end, n_eval) == 48, "mdg_profile_end layout");
+MDG_STATIC_ASSERT(sizeof(mdg_map_interval) == 368 && offsetof(mdg_map_interval, end) == 32, "mdg_map_interval layout");
+
 int mdg_version(void);
 const char* mdg_last_error(void);
 int mdg_device_count(void);
@@ -353,6 +383,22 @@ int mdg_map_batch(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
                   const int64_t* tax_id, const uint32_t* k, const uint32_t* N,
                   const uint32_t* mism12, const double* noise3,
                   const mdg_fit_config* cfg, mdg_map_result* out);
+
+/*
+ * K3p — profile intervals of D_max for rows of mdg_map_batch (see mdg_map_interval). `map` holds the rows
+ * mdg_map_batch returned for the same k, N and cfg; every end of every PMD run it made (run kinds 0, 2, 4) is
+ * profiled, at `level` (0 < level < 1; 0.68 is fit_results' HPDI level). Inner fits at fixed D are LM-damped
+ * Newton over (logit q, logit(A / D), log(phi - phi_min)), warm-started from the nearest point already solved;
+ * each end is bracketed by expanding from D^ +- 2 D_max_std towards the bound and refined by the Illinois method
+ * to a bracket of 1e-9 or |h| <= 1e-7. A run with MDG_FIT_FAILED or MDG_FIT_MAP_NOT_CONVERGED gives NaN ends with
+ * MDG_FIT_FAILED; a run not made (n_eval = 0, all NaN) gives NaN ends with flags = n_eval = 0. Synchronous; `mem` as for
+ * mdg_map_batch; any n_tax in one call; no random numbers, so the result is a pure function of (k, N, cfg, map,
+ * level). mdg_ctx_get_timings afterwards: map_ms (the profile kernel), total_ms, n_launches, and leapfrogs[0/2/4] =
+ * the gradient evaluations spent on the ends of that run kind; the other fields are 0.
+ */
+int mdg_map_profile(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
+                    const uint32_t* k, const uint32_t* N, const mdg_fit_config* cfg,
+                    const mdg_map_result* map, double level, mdg_map_interval* out);
 
 /*
  * K0 — tsv_parse: the step before the hot path (SURVEY.md 8f N2). Tokenises a mismatch-matrix

@@ -20,6 +20,8 @@ FIT_MAP_NOT_CONVERGED = 0x2
 FIT_HAS_DIVERGENCES = 0x4
 FIT_BUDGET_EXCEEDED = 0x8
 FIT_COV_INVALID = 0x10
+PROFILE_AT_BOUND = 0x20
+PROFILE_FAILED = 0x40
 
 
 class FitConfig(C.Structure):
@@ -162,6 +164,18 @@ MAP_RESULT_DTYPE = np.dtype(
         "normalized_noise", "normalized_noise_forward", "normalized_noise_reverse")]
     + [(name, "<u8") for name in _REFERENCE_INT_FIELDS]
     + [("run", MAP_RUN_DTYPE, (NUM_RUNS,))],
+    align=True,
+)
+
+PROFILE_END_DTYPE = np.dtype(
+    [(name, "<f8") for name in ("D", "q", "A", "c", "phi", "logp")] + [("n_eval", "<u4"), ("flags", "<u4")],
+    align=True,
+)
+
+# end[i][j]: i = all positions, forward only, reverse only; j = lower, upper
+MAP_INTERVAL_DTYPE = np.dtype(
+    [("tax_id", "<i8"), ("status", "<u4"), ("reserved", "<u4"), ("level", "<f8"), ("threshold", "<f8"),
+     ("end", PROFILE_END_DTYPE, (3, 2))],
     align=True,
 )
 

@@ -26,6 +26,7 @@ EXPORTED_SYMBOLS = (
     "mdg_fit_batch_submit",
     "mdg_fit_batch_wait",
     "mdg_map_batch",
+    "mdg_map_profile",
     "mdg_select_top",
     "mdg_test_lgamma_digamma",
     "mdg_test_logp_grad",
@@ -78,6 +79,7 @@ def load():
     lib.mdg_fit_batch_submit.argtypes = lib.mdg_fit_batch.argtypes + [C.POINTER(i64)]
     lib.mdg_fit_batch_wait.argtypes = [vp, i64, C.POINTER(Timings)]
     lib.mdg_map_batch.argtypes = [vp, i32, i64, i32, vp, vp, vp, vp, vp, C.POINTER(FitConfig), vp]
+    lib.mdg_map_profile.argtypes = [vp, i32, i64, i32, vp, vp, C.POINTER(FitConfig), vp, C.c_double, vp]
     lib.mdg_select_top.argtypes = [vp, i32, i64, vp, vp, vp, i64, vp, vp, i64, vp, vp, C.POINTER(i64)]
     lib.mdg_test_lgamma_digamma.argtypes = [vp, i64, vp, vp, vp]
     lib.mdg_test_exp_log.argtypes = [vp, i64, vp, vp, vp]

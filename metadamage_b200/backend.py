@@ -6,7 +6,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._abi import FIT_RESULT_DTYPE, MAP_RESULT_DTYPE, MDG_DEVICE, MDG_HOST, NUM_RUNS, Timings, ptr
+from ._abi import FIT_RESULT_DTYPE, MAP_INTERVAL_DTYPE, MAP_RESULT_DTYPE, MDG_DEVICE, MDG_HOST, NUM_RUNS, Timings, ptr
 
 BASES = "ACGT"
 OFFDIAG_COLUMNS = [r + o for r in BASES for o in BASES if r != o]  # AC,AG,AT,CA,CG,CT,GA,GC,GT,TA,TC,TG
@@ -389,6 +389,34 @@ class Context:
             raise ValueError("out buffer too small")
         _lib.check(self._lib.mdg_map_batch(self._h, MDG_DEVICE, n_tax, R // 2, _dptr(tax_id), _dptr(k), _dptr(N), _dptr(mism12),
                                            _dptr(noise3), C.byref(cfg), _dptr(out)))
+
+    def map_profile(self, k, N, map_rows, cfg=None, level=0.68):
+        """mdg_map_profile on host numpy arrays: profile intervals of D_max at `level` for the rows `map_rows` that
+        map_batch returned for the same k, N and cfg. Returns a MAP_INTERVAL_DTYPE array."""
+        cfg = cfg or _lib.default_config()
+        k = np.ascontiguousarray(k, dtype=np.uint32)
+        N = np.ascontiguousarray(N, dtype=np.uint32)
+        map_rows = np.ascontiguousarray(map_rows, dtype=MAP_RESULT_DTYPE)
+        if k.ndim != 2 or k.shape != N.shape or k.shape[0] != len(map_rows) or k.shape[1] % 2:
+            raise ValueError("k and N must be [n_tax][2*max_position], one map row per TaxID")
+        n_tax, R = k.shape
+        res = np.zeros(n_tax, dtype=MAP_INTERVAL_DTYPE)
+        _lib.check(self._lib.mdg_map_profile(self._h, MDG_HOST, n_tax, R // 2, ptr(k), ptr(N), C.byref(cfg), ptr(map_rows),
+                                             float(level), ptr(res)))
+        return res
+
+    def map_profile_device(self, k, N, map_rows, out, cfg=None, level=0.68):
+        """mdg_map_profile on torch CUDA tensors (k, N: [n_tax][2P] int32 bits of uint32; map_rows: uint8 bytes of
+        n_tax MAP_RESULT_DTYPE rows, e.g. map_batch_device's `out`); `out` is a uint8 CUDA tensor of at least
+        n_tax * MAP_INTERVAL_DTYPE.itemsize bytes. Synchronous."""
+        cfg = cfg or _lib.default_config()
+        n_tax, R = k.shape
+        if map_rows.numel() * map_rows.element_size() < n_tax * MAP_RESULT_DTYPE.itemsize:
+            raise ValueError("map_rows buffer too small")
+        if out.numel() * out.element_size() < n_tax * MAP_INTERVAL_DTYPE.itemsize:
+            raise ValueError("out buffer too small")
+        _lib.check(self._lib.mdg_map_profile(self._h, MDG_DEVICE, n_tax, R // 2, _dptr(k), _dptr(N), C.byref(cfg),
+                                             _dptr(map_rows), float(level), _dptr(out)))
 
     # ------------------------------------------------------------------ test hooks
     def lgamma_digamma(self, x):

@@ -1,6 +1,6 @@
 """`metadamage fit` command line (cli.py:97-159): same options and defaults, plus
 `--max-position` (documented upstream, README.md:121, but never wired: cli.py:105,143) and
-`--gpus`, and `--map-only` (MAP-only screening). The `dashboard` sub-command is a visualisation front-end outside this build's scope."""
+`--gpus`, `--map-only` (MAP-only screening) and `--profile-interval` (profile intervals of D_max for it). The `dashboard` sub-command is a visualisation front-end outside this build's scope."""
 from pathlib import Path
 from typing import List, Optional
 
@@ -38,12 +38,16 @@ def cli_fit(
     gpus: int = typer.Option(1, help="number of B200s of this box to partition the TaxIDs over"),
     map_only: bool = typer.Option(False, "--map-only", help="MAP fits with Laplace uncertainties and a likelihood-ratio "
                                   "test only (no MCMC): writes map_results/<name>.parquet instead of the fit_* tables"),
+    profile_interval: bool = typer.Option(False, "--profile-interval", help="with --map-only: add 0.68 profile intervals "
+                                          "of D_max (all, forward and reverse positions) to map_results"),
 ):
     """Fitting Ancient Damage. FILENAMES are the mismatch-matrix files to fit, e.g.
 
     \b
         $ metadamage fit --max-fits 10 --max-cores 2 ./data/input/data_ancient.txt
     """
+    if profile_interval and not map_only:
+        raise typer.BadParameter("--profile-interval needs --map-only", param_hint="--profile-interval")
     from .main import main  # deferred: importing the backend needs the built CUDA library
 
     cfg = utils.Config(
@@ -54,7 +58,10 @@ def cli_fit(
         forced=forced, version="0.0.0", gpus=gpus,
     )
     cfg.add_filenames(filenames)
-    main(filenames, cfg, map_only=map_only)
+    if profile_interval:  # passed only when set: the default call is the one without intervals
+        main(filenames, cfg, map_only=map_only, profile_interval=True)
+    else:
+        main(filenames, cfg, map_only=map_only)
 
 
 @cli_app.command("dashboard")

@@ -16,6 +16,7 @@
 #include "mdg_select_kernel.cuh"
 #include "mdg_post_kernels.cuh"
 #include "mdg_map_batch_kernel.cuh"
+#include "mdg_map_profile_kernel.cuh"
 #include "mdg_nuts_kernel.cuh"
 
 namespace mdg {
@@ -324,6 +325,18 @@ int launch_map_batch(mdg_ctx* ctx, cudaStream_t st, const MapBatchLaunch& ml) {
     const long long items = (long long)ml.n_runs * ml.n_tax;
     with_npl(2 * ml.P, [&](auto npl) {
         auto kern = map_batch_kernel<decltype(npl)::value, kMapWarps>;
+        int grid = persistent_grid(kern, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
+        kern<<<grid, kMapWarps * 32, 0, st>>>(ml);
+    });
+    MDG_CUDA_TRY(cudaGetLastError());
+    ctx->timings.n_launches++;
+    return MDG_OK;
+}
+
+int launch_map_profile(mdg_ctx* ctx, cudaStream_t st, const MapProfileLaunch& ml) {
+    const long long items = 2ll * ml.n_prof * ml.n_tax;
+    with_npl(2 * ml.P, [&](auto npl) {
+        auto kern = map_profile_kernel<decltype(npl)::value, kMapWarps>;
         int grid = persistent_grid(kern, kMapWarps * 32, 0, ctx->num_sms, items, kMapWarps);
         kern<<<grid, kMapWarps * 32, 0, st>>>(ml);
     });
@@ -1291,6 +1304,65 @@ int mdg_map_batch(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position, const 
         MDG_CUDA_TRY(cudaEventSynchronize(ctx->call_end));  // the events are reused by the next piece
         ctx->timings.map_ms += elapsed(ctx->work_begin, ctx->work_end);
         ctx->timings.assemble_ms += elapsed(ctx->work_end, ctx->call_end);
+    }
+    if ((rc = stage.copy_back(0, nt, st))) return rc;
+    unsigned long long evals[MDG_NUM_RUNS];
+    MDG_CUDA_TRY(cudaMemcpyAsync(evals, d_evals, sizeof evals, cudaMemcpyDeviceToHost, st));
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_end, st));
+    MDG_CUDA_TRY(cudaEventSynchronize(ctx->call_end));
+    for (int r = 0; r < MDG_NUM_RUNS; ++r) ctx->timings.leapfrogs[r] = evals[r];
+    ctx->timings.total_ms = elapsed(ctx->call_begin, ctx->call_end);
+    return MDG_OK;
+}
+
+int mdg_map_profile(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position, const uint32_t* k, const uint32_t* N,
+                    const mdg_fit_config* cfg, const mdg_map_result* map, double level, mdg_map_interval* out) {
+    if (!ctx) { set_error("ctx is NULL"); return MDG_ERR_INVALID; }
+    if (!cfg || n_tax < 0 || max_position < 1 || max_position > MDG_MAX_POSITION || (mem != MDG_HOST && mem != MDG_DEVICE) ||
+        !(level > 0.0 && level < 1.0)) {
+        set_error("mdg_map_profile: invalid argument (need 0 < level < 1)");
+        return MDG_ERR_INVALID;
+    }
+    if (n_tax > 0 && (!k || !N || !map || !out)) { set_error("mdg_map_profile: NULL k/N/map/out"); return MDG_ERR_INVALID; }
+    DeviceGuard guard(ctx->device);
+    cudaStream_t st = ctx->stream;
+    ctx->timings = mdg_timings{};
+    const int P = max_position, R = 2 * P;
+    const int n_prof = cfg->do_fwd_rev ? 3 : 1;
+    const size_t nt = (size_t)n_tax;
+    // TaxIDs per launch: keeps the item index (6 per TaxID) in 32 bits
+    const long long piece = 1ll << 20;
+    int rc;
+    MDG_CUDA_TRY(cudaEventRecord(ctx->call_begin, st));
+    const uint32_t *d_k, *d_N;
+    const mdg_map_result* d_map;
+    mdg_map_interval* d_out;
+    Stage stage(ctx->arena, mem == MDG_HOST, st);
+    stage.in(d_k, k, nt * R * 4);
+    stage.in(d_N, N, nt * R * 4);
+    stage.in(d_map, map, nt * sizeof(mdg_map_result));
+    stage.out(d_out, out, sizeof(mdg_map_interval), nt);
+    if ((rc = stage.commit())) return rc;
+    if ((rc = ctx->map_counters.ensure(256))) return rc;
+    unsigned int* d_counter = ctx->map_counters.as<unsigned int>();                       // [1] work counter
+    unsigned long long* d_evals = reinterpret_cast<unsigned long long*>(d_counter + 16);  // [6] gradient evaluations
+    MDG_CUDA_TRY(cudaMemsetAsync(d_counter, 0, 256, st));
+    const Priors pr = make_priors(*cfg);
+    for (long long c0 = 0; c0 < n_tax; c0 += piece) {
+        const int nc = (int)std::min<long long>(piece, n_tax - c0);
+        if (c0 > 0) MDG_CUDA_TRY(cudaMemsetAsync(d_counter, 0, sizeof(unsigned int), st));
+        MDG_CUDA_TRY(cudaEventRecord(ctx->work_begin, st));
+        MapProfileLaunch ml = {};
+        ml.k = d_k + (size_t)c0 * R; ml.N = d_N + (size_t)c0 * R; ml.map = d_map + c0;
+        ml.n_tax = nc; ml.P = P; ml.n_prof = n_prof; ml.pr = pr; ml.level = level;
+        ml.work_counter = d_counter; ml.eval_totals = d_evals; ml.out = d_out + c0;
+        if ((rc = launch_map_profile(ctx, st, ml))) return rc;
+        MDG_CUDA_TRY(cudaEventRecord(ctx->work_end, st));
+        map_interval_header_kernel<<<(nc + 127) / 128, 128, 0, st>>>(ml.map, nc, n_prof, level, ml.out);
+        MDG_CUDA_TRY(cudaGetLastError());
+        ctx->timings.n_launches++;
+        MDG_CUDA_TRY(cudaEventSynchronize(ctx->work_end));  // the events are reused by the next piece
+        ctx->timings.map_ms += elapsed(ctx->work_begin, ctx->work_end);
     }
     if ((rc = stage.copy_back(0, nt, st))) return rc;
     unsigned long long evals[MDG_NUM_RUNS];

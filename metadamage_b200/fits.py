@@ -10,7 +10,8 @@ so that the two reference schemas stay unchanged.
 
 `get_map_fits` / `compute_map_fits` are the MAP-only screening mode (`metadamage fit --map-only`): six MAP
 fits per TaxID with Laplace uncertainties and a likelihood-ratio statistic through `mdg_map_batch`, no NUTS,
-one table in map_results/<shortname>.parquet.
+one table in map_results/<shortname>.parquet. With `profile_interval` (`--profile-interval`) the table also gets
+profile intervals of D_max at level 0.68 through `mdg_map_profile` (MAP_INTERVAL_COLUMNS).
 """
 import logging
 
@@ -18,7 +19,7 @@ import numpy as np
 import pandas as pd
 
 from . import _lib, io, utils
-from ._abi import FIT_COV_INVALID, FIT_FAILED, FIT_MAP_NOT_CONVERGED, MAP_RESULT_DTYPE
+from ._abi import FIT_COV_INVALID, FIT_FAILED, FIT_MAP_NOT_CONVERGED, MAP_INTERVAL_DTYPE, MAP_RESULT_DTYPE, PROFILE_FAILED
 from .counts import dense_from_df_counts, get_context
 from .parallel import run_on_gpus
 
@@ -53,6 +54,12 @@ _MAP_RUN_COLUMNS = {
     **{name: (0, name) for name in ("q", "q_std", "A", "A_std", "c", "c_std", "phi", "phi_std", "logp", "loglik")},
     **{"null_" + name: (1, name) for name in ("q", "q_std", "phi", "phi_std", "logp", "loglik")},
 }
+# profile intervals of D_max appended to the MAP-only table with --profile-interval, at the level of fit_results' HPDI
+# (fits.py:119). interval_valid: both all-position ends were found (an end at a bound included).
+PROFILE_INTERVAL_LEVEL = 0.68
+MAP_INTERVAL_COLUMNS = ["D_max_lower", "D_max_upper", "forward_D_max_lower", "forward_D_max_upper", "reverse_D_max_lower",
+                        "reverse_D_max_upper", "interval_valid"]
+
 
 def mcmc_kwargs_default():
     """fits.py:792-799."""
@@ -100,21 +107,30 @@ def fit_dense(dense, cfg, fit_cfg, n_gpus=1):
     return {key: np.concatenate([p[key] for p in parts]) for key in ("result", "median", "hpdi_lo", "hpdi_hi")}
 
 
-def map_dense(dense, cfg, fit_cfg, n_gpus=1):
-    """Run mdg_map_batch over `n_gpus` contiguous shares of the dense batch (as fit_dense); host-side concat."""
+def map_dense(dense, cfg, fit_cfg, n_gpus=1, level=None):
+    """Run mdg_map_batch over `n_gpus` contiguous shares of the dense batch (as fit_dense); host-side concat. With
+    `level`, each GPU also profiles its share (mdg_map_profile) right after its MAP pass, and (rows, intervals) is
+    returned."""
     n_tax = len(dense["tax_id"])
     if n_tax == 0:
-        return np.zeros(0, MAP_RESULT_DTYPE)
+        rows = np.zeros(0, MAP_RESULT_DTYPE)
+        return rows if level is None else (rows, np.zeros(0, MAP_INTERVAL_DTYPE))
     n_dev = max(1, min(int(n_gpus), _lib.load().mdg_device_count() or 1))
 
     def worker(rank, start, stop):
         sl = slice(start, stop)
-        return get_context(rank).map_batch(dense["tax_id"][sl], dense["k"][sl], dense["N"][sl], fit_cfg,
-                                        mism12=dense["mism12"][sl] if dense.get("mism12") is not None else None,
-                                        noise3=dense["noise"][sl] if dense.get("noise") is not None else None)
+        ctx = get_context(rank)
+        rows = ctx.map_batch(dense["tax_id"][sl], dense["k"][sl], dense["N"][sl], fit_cfg,
+                             mism12=dense["mism12"][sl] if dense.get("mism12") is not None else None,
+                             noise3=dense["noise"][sl] if dense.get("noise") is not None else None)
+        if level is None:
+            return rows
+        return rows, ctx.map_profile(dense["k"][sl], dense["N"][sl], rows, fit_cfg, level)
 
     parts = [p for p in run_on_gpus(n_tax, n_dev, worker) if p is not None]
-    return np.concatenate(parts)
+    if level is None:
+        return np.concatenate(parts)
+    return np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts])
 
 
 def select_top_dense(df_counts, dense, n_fits, ctx=None):
@@ -205,10 +221,11 @@ def make_df_fit_map(res, dense, ok, cfg):
     return pd.DataFrame(data, copy=False)
 
 
-def make_df_map_results(res, dense, cfg):
+def make_df_map_results(res, dense, cfg, intervals=None):
     """The MAP-only table: one row per TaxID in df_counts order, columns MAP_RESULT_COLUMNS in their final dtypes
     (as make_df_fit_results). TaxIDs whose all-position PMD or null fit had no finite starting point are dropped with
-    the same warning. `valid`: both all-position fits converged and have a Laplace covariance."""
+    the same warning. `valid`: both all-position fits converged and have a Laplace covariance. `intervals` (the
+    MAP_INTERVAL_DTYPE rows of mdg_map_profile for the same TaxIDs) appends MAP_INTERVAL_COLUMNS."""
     ok = (res["status"] & FIT_FAILED) == 0
     for tax in dense["tax_id"][~ok]:
         logger.warning("Fit: no valid fit for tax_id %s. Skipping for now", tax)
@@ -234,15 +251,24 @@ def make_df_map_results(res, dense, cfg):
             data[col] = pd.Categorical.from_codes(np.zeros(n, np.int8), categories=[cfg.shortname])
         else:
             data[col] = _final_dtype(r[col], col)
+    if intervals is not None:
+        ends = intervals[ok]["end"]
+        for i, prefix in enumerate(("", "forward_", "reverse_")):
+            data[prefix + "D_max_lower"] = _final_dtype(ends[:, i, 0]["D"], "D")
+            data[prefix + "D_max_upper"] = _final_dtype(ends[:, i, 1]["D"], "D")
+        data["interval_valid"] = (intervals[ok]["status"] & (PROFILE_FAILED | FIT_FAILED)) == 0
     return pd.DataFrame(data, copy=False)
 
 
-def compute_map_fits(df_counts, cfg, n_fits=None):
+def compute_map_fits(df_counts, cfg, n_fits=None, profile_interval=False):
     """MAP-only screening of every TaxID of df_counts (or of the top `n_fits`, as compute_fits): the table of
-    make_df_map_results."""
+    make_df_map_results, with the profile intervals of D_max at PROFILE_INTERVAL_LEVEL if `profile_interval`."""
     dense = select_top_dense(df_counts, dense_from_df_counts(df_counts, cfg), n_fits)
-    res = map_dense(dense, cfg, fit_config_from(cfg), n_gpus=getattr(cfg, "gpus", 1))
-    return make_df_map_results(res, dense, cfg)
+    n_gpus = getattr(cfg, "gpus", 1)
+    if not profile_interval:
+        return make_df_map_results(map_dense(dense, cfg, fit_config_from(cfg), n_gpus=n_gpus), dense, cfg)
+    res, intervals = map_dense(dense, cfg, fit_config_from(cfg), n_gpus=n_gpus, level=PROFILE_INTERVAL_LEVEL)
+    return make_df_map_results(res, dense, cfg, intervals)
 
 
 def compute_fits(df_counts, cfg, mcmc_kwargs=None, return_map=False, n_fits=None):
@@ -282,14 +308,19 @@ def get_fits(df_counts, cfg):
     return df_fit_results, df_fit_predictions
 
 
-def get_map_fits(df_counts, cfg):
-    """`metadamage fit --map-only`: the cache rules of get_fits on map_results/<shortname>.parquet."""
+def get_map_fits(df_counts, cfg, profile_interval=False):
+    """`metadamage fit --map-only [--profile-interval]`: the cache rules of get_fits on map_results/<shortname>.parquet.
+    With intervals the metadata also records "profile_interval": PROFILE_INTERVAL_LEVEL, and a cached table is reused
+    only if its own key matches (a missing key means a table without intervals)."""
     pq = io.Parquet(cfg.filename_map_results)
+    meta = cfg.to_dict()
+    if profile_interval:
+        meta["profile_interval"] = PROFILE_INTERVAL_LEVEL
     if pq.exists(cfg.forced):
-        if utils.metadata_is_similar(pq.load_metadata(), cfg.to_dict(), include=CACHE_KEYS):
+        if utils.metadata_is_similar(pq.load_metadata(), meta, include=CACHE_KEYS + ["profile_interval"]):
             logger.info("Fit: Loading MAP fits from parquet-file.")
             return pq.load()
     logger.info("Fit: Generating MAP fits and saving to file.")
-    df_map_results = compute_map_fits(df_counts, cfg, n_fits=cfg.N_fits)
-    pq.save(df_map_results, metadata=cfg.to_dict())
+    df_map_results = compute_map_fits(df_counts, cfg, n_fits=cfg.N_fits, profile_interval=profile_interval)
+    pq.save(df_map_results, metadata=meta)
     return df_map_results

@@ -1,12 +1,14 @@
-"""Throughput of the MAP-only screening path (mdg_map_batch, device-resident inputs) on one GPU.
+"""Throughput of the MAP-only screening path (mdg_map_batch, device-resident inputs) and of its profile intervals
+(mdg_map_profile at level 0.68, device-resident inputs and MAP rows) on one GPU.
 
 Sizes: 10 000 fitted TaxIDs of the cfg2 generator and 1 000 000 of the cfg3 generator (eight independently generated
 shares, rank r = jumped block r, as bench.py's multi-GPU workload). Every size gets a warm-up call, then calls are
 repeated until at least `--min-seconds` of work has been timed: CUDA events around the whole window and the host clock
 around it (ending in a synchronise). For the ratio, one timed mdg_fit_batch step (six NUTS runs per TaxID) on the
-10 000-TaxID batch after a warm-up step. Prints one JSON line; writes nothing unless --out is given.
+10 000-TaxID batch after a warm-up step. The profile block times mdg_map_profile the same way at both sizes, on the
+rows of one mdg_map_batch call. Prints one JSON line; writes nothing unless --out is given.
 
-    python tools/bench_map.py [--out profiles/r03_map_only_1gpu.json]
+    python tools/bench_map.py [--out profiles/r05_map_profile_1gpu.json]
 """
 import argparse
 import json
@@ -79,6 +81,47 @@ def time_map(ctx, dev, name, tid, k, N, min_seconds):
     }
 
 
+def time_profile(ctx, dev, name, tid, k, N, min_seconds):
+    import torch
+
+    from metadamage_b200._abi import MAP_INTERVAL_DTYPE, MAP_RESULT_DTYPE, PROFILE_AT_BOUND
+
+    n = len(tid)
+    dt, dk, dN = to_device(dev, tid, k, N)
+    rows = torch.empty(n * MAP_RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
+    ctx.map_batch_device(dt, dk, dN, rows)
+    out = torch.empty(n * MAP_INTERVAL_DTYPE.itemsize, dtype=torch.uint8, device=dev)
+    ctx.map_profile_device(dk, dN, rows, out)  # warm-up at this size
+    torch.cuda.synchronize(dev)
+    start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    calls, kern_ms, evals = 0, 0.0, 0
+    t0 = time.perf_counter()
+    start.record()
+    while True:
+        ctx.map_profile_device(dk, dN, rows, out)
+        t = ctx.timings()
+        calls += 1
+        kern_ms += t["map_ms"]
+        evals += sum(t["leapfrogs"])
+        if time.perf_counter() - t0 >= min_seconds:
+            break
+    stop.record()
+    torch.cuda.synchronize(dev)
+    host_s = time.perf_counter() - t0
+    ev_s = start.elapsed_time(stop) / 1e3
+    iv = np.frombuffer(out.cpu().numpy().tobytes(), MAP_INTERVAL_DTYPE)
+    ends = iv["end"][:, 0]
+    return {
+        "workload": name, "taxids": n, "calls": calls, "event_s": round(ev_s, 4), "host_s": round(host_s, 4),
+        "ms_per_call": round(ev_s * 1e3 / calls, 3), "profile_kernel_ms_per_call": round(kern_ms / calls, 3),
+        "taxids_per_s": round(n * calls / ev_s), "ends_per_s": round(6 * n * calls / ev_s),
+        "grad_evals_per_s": round(evals / ev_s), "grad_evals_per_taxid": round(evals / (n * calls), 1),
+        "interval_valid_share": round(float(np.mean((iv["status"] & 0x41) == 0)), 4),
+        "all_position_ends_at_bound_share": round(float(np.mean((ends["flags"] & PROFILE_AT_BOUND) != 0)), 5),
+        "ends_at_bound_share": round(float(np.mean((iv["end"]["flags"] & PROFILE_AT_BOUND) != 0)), 5),
+    }
+
+
 def time_fit(ctx, dev, tid, k, N):
     import torch
 
@@ -121,12 +164,15 @@ def main():
 
     large = syn.dense_fit_batch_shares(1_000_000, 8)
     sizes = [time_map(ctx, dev, "cfg2", *small, args.min_seconds), time_map(ctx, dev, "cfg3", *large, args.min_seconds)]
+    profile = [time_profile(ctx, dev, "cfg2", *small, args.min_seconds), time_profile(ctx, dev, "cfg3", *large, args.min_seconds)]
     fit = time_fit(ctx, dev, *small)
     ctx.close()
     line = {
-        "metric": "mdg_map_batch throughput, device-resident inputs, 1 GPU",
+        "metric": "mdg_map_batch and mdg_map_profile (level 0.68) throughput, device-resident inputs, 1 GPU",
         "gpu": info["name"], "power_limit": info["power.limit"], "sm_clock": info["clocks.sm"], "sm_clock_max": info["clocks.max.sm"],
         "sizes": sizes,
+        "profile_sizes": profile,
+        "profile_vs_map_time": [round(p["ms_per_call"] / m["ms_per_call"], 2) for p, m in zip(profile, sizes)],
         "fit_batch_step": fit,
         "map_vs_fit_speedup_10k": round(fit["event_s"] / (sizes[0]["event_s"] / sizes[0]["calls"]), 1),
     }
