@@ -481,6 +481,12 @@ int mdg_test_exp_log(mdg_ctx* ctx, int64_t n, const double* x, double* out_exp, 
 int mdg_test_philox(mdg_ctx* ctx, int64_t n, const uint32_t* key2, const uint32_t* ctr4,
                     uint32_t* out4);
 
+/* n_draws BetaBinomial(alpha, beta, n) variates from the posterior predictive's own samplers (a Beta variate from two
+ * Marsaglia-Tsang gammas, then Binomial by BINV / BTRS), draw i on the Philox stream keyed by (seed, tax id 12345) at
+ * counter (0, i, MDG_RUN_PMD_ALL | purpose 6 << 8, i >> 32). Needs alpha > 0, beta > 0, n >= 0; out: host [n_draws] */
+int mdg_test_betabinom_draws(mdg_ctx* ctx, uint64_t seed, int64_t n_draws, double alpha, double beta, double n,
+                             double* out);
+
 /* measured FP64 FMA peak of this GPU (dependent-free DFMA loop), in TFLOP/s */
 int mdg_measure_fp64_peak(mdg_ctx* ctx, double* out_tflops);
 

@@ -32,6 +32,7 @@ EXPORTED_SYMBOLS = (
     "mdg_test_logp_grad",
     "mdg_test_exp_log",
     "mdg_test_philox",
+    "mdg_test_betabinom_draws",
     "mdg_measure_fp64_peak",
 )
 
@@ -85,6 +86,7 @@ def load():
     lib.mdg_test_exp_log.argtypes = [vp, i64, vp, vp, vp]
     lib.mdg_test_logp_grad.argtypes = [vp, i32, vp, vp, C.POINTER(FitConfig), i32, i32, i32, i64, vp, vp, vp, vp]
     lib.mdg_test_philox.argtypes = [vp, i64, vp, vp, vp]
+    lib.mdg_test_betabinom_draws.argtypes = [vp, u64, i64, C.c_double, C.c_double, C.c_double, vp]
     lib.mdg_measure_fp64_peak.argtypes = [vp, C.POINTER(C.c_double)]
     _lib = lib
     return lib

@@ -440,6 +440,13 @@ class Context:
         _lib.check(self._lib.mdg_test_philox(self._h, len(ctr4), ptr(key2), ptr(ctr4), ptr(out)))
         return out
 
+    def test_betabinom_draws(self, alpha, beta, n, n_draws, seed=1):
+        """n_draws BetaBinomial(alpha, beta, n) variates from the posterior predictive's device samplers."""
+        out = np.empty(int(n_draws))
+        _lib.check(self._lib.mdg_test_betabinom_draws(self._h, C.c_uint64(seed), len(out), float(alpha), float(beta),
+                                                      float(n), ptr(out)))
+        return out
+
     def logp_grad(self, k, N, u, cfg=None, model=0, lane_mask=0, with_jacobian=True):
         cfg = cfg or _lib.default_config()
         k = np.ascontiguousarray(k, dtype=np.uint32).ravel()

@@ -976,8 +976,10 @@ int mdg_fit_batch_submit(mdg_ctx* ctx, int mem, int64_t n_tax, int max_position,
         return MDG_ERR_INVALID;
     }
     if (cfg->num_samples < 1 || cfg->num_samples > 4096 || cfg->num_warmup < 0 || cfg->max_tree_depth < 1 ||
-        cfg->max_tree_depth > kMaxTreeDepth || cfg->max_leapfrogs_per_run < 0) {
-        set_error("mdg_fit_batch: need 1 <= num_samples <= 4096, num_warmup >= 0, 1 <= max_tree_depth <= %d, max_leapfrogs_per_run >= 0",
+        cfg->max_tree_depth > kMaxTreeDepth || cfg->max_leapfrogs_per_run < 0 || !(cfg->hpdi_prob > 0.0 && cfg->hpdi_prob <= 1.0)) {
+        // K6's HPDI window is buf[i .. i + (int)(hpdi_prob * S)], clamped to S - 1 from above only
+        set_error("mdg_fit_batch: need 1 <= num_samples <= 4096, num_warmup >= 0, 1 <= max_tree_depth <= %d, max_leapfrogs_per_run >= 0, "
+                  "0 < hpdi_prob <= 1",
                   kMaxTreeDepth);
         return MDG_ERR_INVALID;
     }
@@ -1409,6 +1411,17 @@ __global__ void test_philox_kernel(long long n, const uint32_t* key2, const uint
     }
 }
 
+__global__ void test_betabinom_kernel(uint64_t seed, long long n, double alpha, double beta, double trials, double* out) {
+    long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    log_table_init();
+    if (i < n) {
+        Stream st;
+        st.key = make_key(seed, 12345); st.c0 = 0u; st.c1 = (uint32_t)i; st.c2 = c2word(0, P_PPC); st.c3 = (uint32_t)(i >> 32); st.have = false; st.stash = 0.0;
+        const double p = beta_variate(st, alpha, beta);
+        out[i] = binomial_variate(st, trials, p);
+    }
+}
+
 template <int MODEL, int NPL>
 __global__ void test_logp_kernel(int P, const uint32_t* k, const uint32_t* N, Priors pr, int mask, int jac,
                                  long long n_eval, const double* u, double* out_logp, double* out_grad, double* out_ll) {
@@ -1502,6 +1515,23 @@ int mdg_test_philox(mdg_ctx* ctx, int64_t n, const uint32_t* key2, const uint32_
     test_philox_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(n, d, d + 2 * n, d + 6 * n);
     MDG_CUDA_TRY(cudaGetLastError());
     MDG_CUDA_TRY(cudaMemcpyAsync(out4, d + 6 * n, (size_t)n * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    MDG_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    return MDG_OK;
+}
+
+int mdg_test_betabinom_draws(mdg_ctx* ctx, uint64_t seed, int64_t n_draws, double alpha, double beta, double n, double* out) {
+    if (!ctx || n_draws < 0 || (n_draws > 0 && !out) || !(alpha > 0.0) || !(beta > 0.0) || !(n >= 0.0)) {
+        set_error("mdg_test_betabinom_draws: need n_draws >= 0, out, alpha > 0, beta > 0, n >= 0");
+        return MDG_ERR_INVALID;
+    }
+    if (n_draws == 0) return MDG_OK;
+    DeviceGuard guard(ctx->device);
+    int rc = ctx->test_scratch.ensure((size_t)n_draws * 8);
+    if (rc) return rc;
+    double* d = ctx->test_scratch.as<double>();
+    test_betabinom_kernel<<<(unsigned)((n_draws + 255) / 256), 256, 0, ctx->stream>>>(seed, n_draws, alpha, beta, n, d);
+    MDG_CUDA_TRY(cudaGetLastError());
+    MDG_CUDA_TRY(cudaMemcpyAsync(out, d, (size_t)n_draws * 8, cudaMemcpyDeviceToHost, ctx->stream));
     MDG_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return MDG_OK;
 }

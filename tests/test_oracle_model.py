@@ -141,19 +141,6 @@ def test_adaptation_schedule(oracle):
     assert oracle.adaptation_schedule(100) == [(0, 14), (15, 89), (90, 99)]
 
 
-@pytest.mark.parametrize("alpha,beta,n", [(0.3, 4.0, 12), (2.0, 30.0, 40), (150.0, 2000.0, 5000), (0.002, 1.5, 300)])
-def test_betabinomial_sampler_distribution(oracle, alpha, beta, n):
-    """The predictive's Beta->Binomial sampler (fits.py:89-106) against scipy's beta-binomial."""
-    draws = oracle.betabinom_draws(alpha, beta, n, 40000, seed=7)
-    dist = stats.betabinom(n, alpha, beta)
-    assert abs(draws.mean() - dist.mean()) < 5 * dist.std() / np.sqrt(len(draws))
-    qs = [0.05, 0.25, 0.5, 0.75, 0.95]
-    emp = np.quantile(draws, qs)
-    for q_, e_ in zip(qs, emp):
-        # the empirical quantile must sit inside the exact CDF band
-        assert dist.cdf(e_) >= q_ - 0.015 and dist.cdf(e_ - 1) <= q_ + 0.015
-
-
 def test_map_matches_independent_optimiser(oracle, sample_inputs):
     """MAP (new deliverable): LM-Newton result vs scipy on the same constrained-space density."""
     for name, idx in (("ancient", 0), ("control", 0), ("control", 2)):
