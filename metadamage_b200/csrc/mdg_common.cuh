@@ -237,6 +237,10 @@ __device__ __forceinline__ void normal2(uint4 o, double& n0, double& n1) {
 // instructions and every one of them is issued for ONE chain): the library call only backs up arguments
 // outside the fast paths' domain.
 __device__ MDG_COLD double exp_cold(double x) { return exp_fast(x); }
+// exp_fast with its library branches out of line: the same value for every x, for callers that run once per
+// transition and want only exp_core's instructions inline
+__device__ MDG_COLD double exp_fast_outside(double x) { return x != x ? x : (x < -700.0 ? (x < -745.2 ? 0.0 : exp(x)) : exp(x)); }
+__device__ __forceinline__ double exp_fast_split(double x) { return (x >= -700.0 && x <= 700.0) ? exp_core(x) : exp_fast_outside(x); }
 __device__ MDG_COLD double log_cold(double x) { return (x >= 2.2250738585072014e-308 && x < INFINITY) ? log_pos(x) : log(x); }
 __device__ MDG_COLD double sigmoid_cold(double x) {
     const double e = exp_fast(-fabs(x));  // in (0, 1]

@@ -232,11 +232,189 @@ __device__ __forceinline__ void eval_group(const double2* __restrict__ kn, doubl
     valid = isfinite(logp) && !any_bad;
 }
 
+// ---- the cold paths of nuts_group_kernel, out of line ----------------------------------------------------------
+// Once per chain (start, initial point, end), once per adaptation window, the step-size heuristic, fallbacks that
+// never run at the default configuration, and the optional stores. Called from the loop body, they leave a call
+// there instead of their code, so the warm code (leapfrog, leaf, subtree end, transition end, transition start,
+// doubling) is one contiguous block of SASS (tools/sass_layout.py; profiles/r06_nuts_code_layout.md). Each does the
+// operations the inlined code did on the same operands in the same order; a call passes values exactly. They read
+// the launch's parameters in place (`p` is a __grid_constant__ kernel parameter).
+template <int D>  // layout: cold
+__device__ MDG_COLD void reset_dual_averaging(GroupShared<D>& sh) {
+    sh.da_x = 0.0; sh.da_xavg = 0.0; sh.da_gavg = 0.0; sh.da_t = 0; sh.da_prox = log_cold(10.0 * sh.eps);
+}
+
+// the next (TaxID, run) item of a group: {k, N} of the run into the warp's slots, the WAIC accumulators and the chain
+// state in shared memory cleared; returns {TaxID index, run mask, Philox key}. Inlined: as a call (in either form,
+// with or without the key) it made ptxas spill the phase across the whole leapfrog loop (4 B stored and loaded per
+// trip in the PMD kernel); inlined, its code still lies ahead of the loop, outside the warm block.
+template <int MODEL, int GW, int D>
+__device__ __forceinline__ int4 chain_start(const FitLaunch& p, GroupShared<D>& sh, unsigned item, double2* kn, double* wacc, int lane,
+                                     int lig, unsigned gmask) {
+    const int P = p.P, NS = p.n_slots;
+    const size_t wstride = (size_t)NS * 32;
+    int tax, mask;
+    {
+        const unsigned prio = 2u * (unsigned)p.n_prio, n_all = (unsigned)p.n_items_all;
+        const bool is_all = item >= prio && item < prio + n_all;
+        const unsigned w = is_all ? item - prio : (item < prio ? item : item - n_all);  // half runs: 2 * position + strand
+        const unsigned q = is_all ? w : (w >> 1);  // queue position of the TaxID
+        tax = p.order != nullptr ? __ldg(p.order + q) : (int)q;
+        mask = is_all ? 0 : 1 + (int)(w & 1u);
+    }
+    const int run_kind = mask * 2 + MODEL;
+    const int n_obs = mask == 0 ? 2 * P : P;
+    const uint2 key = make_key(p.cfg.seed, p.tax_id[tax]);
+    if (p.chain_clock != nullptr && lig == 0) p.chain_clock[((size_t)tax * MDG_NUM_RUNS + run_kind) * 2] = global_timer_ns();
+    const uint32_t* kk = p.k + (size_t)tax * 2 * P + (mask == 2 ? P : 0);
+    const uint32_t* NN = p.N + (size_t)tax * 2 * P + (mask == 2 ? P : 0);
+#pragma unroll 1
+    for (int s = 0; s < NS; ++s) {
+        const int j = s * GW + lig - 1;
+        const bool a = (unsigned)j < (unsigned)n_obs;
+        kn[s * 32 + lane] = make_double2(a ? (double)__ldg(kk + j) : 0.0, a ? (double)__ldg(NN + j) : 0.0);
+        wacc[0 * wstride + s * 32] = -INFINITY;  // running max of the streaming log-sum-exp
+        wacc[1 * wstride + s * 32] = 0.0;        // its sum
+        wacc[2 * wstride + s * 32] = 0.0;        // Welford mean
+        wacc[3 * wstride + s * 32] = 0.0;        // Welford M2
+    }
+    __syncwarp(gmask);
+    if (lig < D) { sh.imm[lig] = 1.0; sh.isd[lig] = 1.0; sh.wf_mean[lig] = 0.0; sh.wf_m2[lig] = 0.0; }
+    sh.E0 = 0.0; sh.s_weight = 0.0; sh.s_sum_acc = 0.0;
+    sh.eps = p.cfg.init_step_size; sh.pe_cur = 0.0;
+    sh.da_x = 0.0; sh.da_xavg = 0.0; sh.da_gavg = 0.0; sh.da_prox = 0.0; sh.da_t = 0; sh.wf_n = 0; sh.window_idx = 0;
+    sh.mean_accept = 0.0; sh.n_div = 0u;
+    sh.m_weight = 0.0; sh.m_sum_acc = 0.0; sh.m_pe_p = 0.0; sh.u_main = 0.0; sh.m_nprop = 0; sh.s_pe_p = 0.0;
+    sh.h_step = 0.0; sh.h_Er = 0.0; sh.h_last = 0; sh.h_dir = 0; sh.h_att = 0u; sh.h_call = 0u; sh.init_attempt = 0u;
+    if (lig == 0) {
+#pragma unroll
+        for (int j = 0; j < 5; ++j) { sh.acc_mean[j] = 0.0; sh.acc_m2[j] = 0.0; }
+    }
+    __syncwarp(gmask);
+    return make_int4(tax, mask, (int)key.x, (int)key.y);
+}
+
+// init_to_uniform(radius): component jc of the initial-point candidate number `attempt` (component j is the (j % 2)-th
+// uniform of the Philox block j / 2)
+__device__ MDG_COLD double init_position(const FitLaunch& p, uint2 key, int jc, uint32_t attempt, int run_kind) {
+    double u0, u1;
+    uniform2(philox4x32(key, (uint32_t)(jc >> 1), attempt, c2word(run_kind, P_INIT), 0u), u0, u1);
+    return p.cfg.init_radius * (2.0 * ((jc & 1) ? u1 : u0) - 1.0);
+}
+
+// sqrt(t) and t^-0.75 of the dual averaging past the launch's tables
+__device__ MDG_COLD double da_sqrt_cold(int t) { return sqrt((double)t); }
+__device__ MDG_COLD double da_pow_cold(int t) { return exp_cold(-0.75 * log_cold((double)t)); }
+
+// end of a middle adaptation window: the regularised variance of the window's draws becomes the mass matrix diagonal
+// (warmup_adapter); returns whether the step-size heuristic runs next (else dual averaging restarts here)
+template <int D>
+__device__ MDG_COLD bool window_end(const FitLaunch& p, GroupShared<D>& sh, int lig, unsigned gmask) {
+    __syncwarp(gmask);
+    if (lig < D) {
+        const int wf_n = sh.wf_n;
+        const double cov = sh.wf_m2[lig] / (wf_n - 1);
+        const double v = ((double)wf_n / (wf_n + 5.0)) * cov + 1e-3 * (5.0 / (wf_n + 5.0));
+        sh.imm[lig] = v;
+        sh.isd[lig] = 1.0 / sqrt(v);
+        sh.wf_mean[lig] = 0.0; sh.wf_m2[lig] = 0.0;
+    }
+    __syncwarp(gmask);
+    sh.wf_n = 0;
+    const bool want_heur = p.cfg.find_heuristic_step_size != 0;
+    if (!want_heur) reset_dual_averaging(sh);
+    return want_heur;
+}
+
+// hmc_util.find_reasonable_step_size. heur_record: the direction of the trial just evaluated. heur_next (at `begin`:
+// first sets up the search at eps): its next trial, returned as {momentum component jc, 1} (the leapfrog starts from
+// the chain state with step h_step), or its end, {0, 0}, with eps = the step found.
+template <int D, int GW>
+__device__ MDG_COLD void heur_record(GroupShared<D>& sh, int jc, double rn, double pen, unsigned gmask) {
+    const double log_target_heur = -0.22314355131420976;  // log(0.8)
+    const double delta = (kinetic<D, GW>(sh.imm[jc], rn, gmask) + pen) - sh.h_Er;
+    const int dir_new = (log_target_heur < -delta) ? 1 : -1;  // NaN -> -1
+    sh.h_last = sh.h_dir;
+    sh.h_dir = dir_new;
+}
+
+template <int D, int GW>
+__device__ MDG_COLD double2 heur_next(GroupShared<D>& sh, bool begin, uint2 key, int run_kind, int jc, unsigned gmask) {
+    if (begin) { sh.h_step = sh.eps; sh.h_last = 0; sh.h_dir = 0; sh.h_att = 0; }
+    const double h_step = sh.h_step;
+    const int h_dir = sh.h_dir, h_last = sh.h_last;
+    const bool small_ok = (h_step > 2.2250738585072014e-308) || (h_dir >= 0);
+    const bool large_ok = (h_step < 1.7976931348623157e308) || (h_dir <= 0);
+    if (small_ok && large_ok && (h_last == 0 || h_dir == h_last)) {
+        sh.h_step = h_step * (h_dir > 0 ? 2.0 : (h_dir < 0 ? 0.5 : 1.0));
+        const double rf = draw_normal_lane_cold<D>(key, sh.h_call, c2word(run_kind, P_HEUR), sh.h_att, jc) * sh.isd[jc];
+        ++sh.h_att;
+        sh.h_Er = kinetic<D, GW>(sh.imm[jc], rf, gmask) + sh.pe_cur;
+        return make_double2(rf, 1.0);
+    }
+    sh.eps = h_step;
+    return make_double2(0.0, 0.0);
+}
+
+// the optional outputs: the chain's trace (one value per lane < 4) and the kept constrained draw
+__device__ MDG_COLD void store_trace(const FitLaunch& p, int tax, int run_kind, int t, int lig, double v) {
+    p.trace[(((size_t)tax * MDG_NUM_RUNS + run_kind) * (p.cfg.num_warmup + p.cfg.num_samples) + t) * 4 + lig] = v;
+}
+
+__device__ MDG_COLD void store_sample(const FitLaunch& p, int tax, int slot, int si, double th0, double th1, double th2, double th3) {
+    double* dst = p.samples + (((size_t)tax * p.sample_runs + slot) * p.cfg.num_samples + si) * 4;
+    dst[0] = th0; dst[1] = th1; dst[2] = th2; dst[3] = th3;
+}
+
+// a finished chain: per-position lppd / pWAIC (with log C(N,k)) and the run record
+template <int GW, int D>
+__device__ MDG_COLD void chain_end(const FitLaunch& p, GroupShared<D>& sh, const double2* kn, const double* wacc, int tax, int run_kind,
+                                   int mask, int n_obs, int ns, int failed, uint32_t n_grad, int lane, int lig, unsigned gmask) {
+    const int P = p.P, S = p.cfg.num_samples;
+    const size_t wstride = (size_t)p.n_slots * 32;
+    double waic_sum = 0.0, lppd_sum = 0.0;
+    const size_t R = 2 * (size_t)P;
+    double* wout = p.waic + ((size_t)tax * MDG_NUM_RUNS + run_kind) * 2 * R;
+#pragma unroll 1
+    for (int s = 0; s < ns; ++s) {
+        const int j = s * GW + lig - 1;
+        if ((unsigned)j < (unsigned)n_obs && !failed && S > 0) {
+            const double2 d = kn[s * 32 + lane];
+            const double logC = lgam(d.y + 1.0) - lgam(d.x + 1.0) - lgam(d.y - d.x + 1.0);  // log C(N,k)
+            const int dense = (mask == 2 ? P : 0) + j;
+            const double lppd_i = logC + wacc[0 * wstride + s * 32] + log_cold(wacc[1 * wstride + s * 32]) - log_cold((double)S);
+            const double pw_i = wacc[3 * wstride + s * 32] / (double)S;
+            wout[dense] = lppd_i;
+            wout[R + dense] = pw_i;
+            lppd_sum += lppd_i;
+            waic_sum += -2.0 * (lppd_i - pw_i);
+        }
+    }
+    waic_sum = group_sum<GW>(waic_sum, gmask);
+    lppd_sum = group_sum<GW>(lppd_sum, gmask);
+    __syncwarp(gmask);
+    if (lig == 0) {
+        RunRecord& r = p.rec[(size_t)tax * MDG_NUM_RUNS + run_kind];
+        r.step_size = sh.eps;
+        r.mean_accept = sh.mean_accept;
+        r.n_leapfrog = n_grad;
+        r.n_divergent = sh.n_div;
+        r.waic = waic_sum;
+        r.lppd = lppd_sum;
+#pragma unroll
+        for (int j = 0; j < 5; ++j) { r.mean[j] = sh.acc_mean[j]; r.sd[j] = S > 0 ? sqrt(sh.acc_m2[j] / (double)S) : 0.0; }
+        r.failed = (uint32_t)failed;
+        r.pad = 0;
+        if (p.chain_clock != nullptr) p.chain_clock[((size_t)tax * MDG_NUM_RUNS + run_kind) * 2 + 1] = global_timer_ns();
+    }
+    __syncwarp(gmask);
+}
+
 #ifndef MDG_NUTS_MINBLOCKS
 #define MDG_NUTS_MINBLOCKS 4  // CTAs of four warps per SM: 128 registers per thread, 16 warps per SM (3 / 5 / 6 were measured slower: profiles/r01_nuts_tuning.md)
 #endif
 template <int MODEL, int GW, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nuts_group_kernel(const FitLaunch p) {
+__global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nuts_group_kernel(__grid_constant__ const FitLaunch p) {  // layout: setup
     constexpr int D = ModelDim<MODEL>::value;
     constexpr int GROUPS = 32 / GW;
     // one lane per component (the lane-order sums of kinetic / is_turning) and one per trace column
@@ -265,7 +443,6 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
 
     const int W = p.cfg.num_warmup, S = p.cfg.num_samples, P = p.P;
     const int max_depth = p.cfg.max_tree_depth < kMaxTreeDepth ? p.cfg.max_tree_depth : kMaxTreeDepth;
-    const double log_target_heur = -0.22314355131420976;  // log(0.8)
     const uint32_t budget = p.cfg.max_leapfrogs_per_run > 0 ? (uint32_t)p.cfg.max_leapfrogs_per_run : 0u;
     log_table_init();
     prior_table_init<MODEL>(sh_prior, p.pr, 1);
@@ -298,78 +475,34 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
     double& mean_accept = sh.mean_accept; uint32_t& n_div = sh.n_div;
     double& m_weight = sh.m_weight; double& m_sum_acc = sh.m_sum_acc; double& m_pe_p = sh.m_pe_p; double& u_main = sh.u_main;
     int& m_nprop = sh.m_nprop; double& s_pe_p = sh.s_pe_p;
-    double& h_step = sh.h_step; double& h_Er = sh.h_Er; int& h_last = sh.h_last; int& h_dir = sh.h_dir;
-    uint32_t& h_att = sh.h_att; uint32_t& h_call = sh.h_call; uint32_t& init_attempt = sh.init_attempt;
+    double& h_step = sh.h_step; uint32_t& h_call = sh.h_call; uint32_t& init_attempt = sh.init_attempt;
 
-    auto init_candidate = [&]() {
-        // component j is the (j % 2)-th uniform of the Philox block j / 2
-        double u0, u1;
-        uniform2(philox4x32(key, (uint32_t)(jc >> 1), init_attempt, c2word(run_kind, P_INIT), 0u), u0, u1);
-        zf = p.cfg.init_radius * (2.0 * ((jc & 1) ? u1 : u0) - 1.0);
-        rf = 0.0; gf = 0.0;
-        e = 0.0;
-        phase = GP_INIT;
-    };
-
-    auto reset_dual_averaging = [&]() {
-        da_x = 0.0; da_xavg = 0.0; da_gavg = 0.0; da_t = 0; da_prox = log_cold(10.0 * eps);
-    };
-
-    for (;;) {
+    for (;;) {  // layout: head
         // ================= a group without a chain pulls the next (TaxID, run) item =================
-        if (phase == GP_FETCH) {
+        if (phase == GP_FETCH) {  // layout: fetch
             unsigned item = 0u;
             if (lig == 0) item = atomicAdd(p.work_counter, 1u);
             item = __shfl_sync(gmask, item, 0, GW);
             if (item >= (unsigned)p.n_items) {
                 phase = GP_IDLE;
             } else {
-                {
-                    const unsigned prio = 2u * (unsigned)p.n_prio, n_all = (unsigned)p.n_items_all;
-                    const bool is_all = item >= prio && item < prio + n_all;
-                    const unsigned w = is_all ? item - prio : (item < prio ? item : item - n_all);  // half runs: 2 * position + strand
-                    const unsigned q = is_all ? w : (w >> 1);  // queue position of the TaxID
-                    tax = p.order != nullptr ? __ldg(p.order + q) : (int)q;
-                    mask = is_all ? 0 : 1 + (int)(w & 1u);
-                }
+                const int4 c = chain_start<MODEL, GW, D>(p, sh, item, kn, wacc_of_lane(), lane, lig, gmask);
+                tax = c.x;
+                mask = c.y;
+                key = make_uint2((uint32_t)c.z, (uint32_t)c.w);
                 run_kind = mask * 2 + MODEL;
                 n_obs = mask == 0 ? 2 * P : P;
                 ns = (n_obs + GW) / GW;  // index 0 is the spare
-                key = make_key(p.cfg.seed, p.tax_id[tax]);
-                if (p.chain_clock != nullptr && lig == 0) p.chain_clock[((size_t)tax * MDG_NUM_RUNS + run_kind) * 2] = global_timer_ns();
-                const uint32_t* kk = p.k + (size_t)tax * 2 * P + (mask == 2 ? P : 0);
-                const uint32_t* NN = p.N + (size_t)tax * 2 * P + (mask == 2 ? P : 0);
-                double* const wacc = wacc_of_lane();
-#pragma unroll 1
-                for (int s = 0; s < NS; ++s) {
-                    const int j = s * GW + lig - 1;
-                    const bool a = (unsigned)j < (unsigned)n_obs;
-                    kn[s * 32 + lane] = make_double2(a ? (double)__ldg(kk + j) : 0.0, a ? (double)__ldg(NN + j) : 0.0);
-                    wacc[0 * wstride + s * 32] = -INFINITY;  // running max of the streaming log-sum-exp
-                    wacc[1 * wstride + s * 32] = 0.0;        // its sum
-                    wacc[2 * wstride + s * 32] = 0.0;        // Welford mean
-                    wacc[3 * wstride + s * 32] = 0.0;        // Welford M2
-                }
                 roles.v = 0xE4u;
                 m_is_c = true;
                 n_grad = 0; failed = 0; m_depth = 0; m_turning = false; m_div = false; going_right = true;
                 s_nprop = 0; s_div = false; leaf_counter = 0; t = 0;
-                __syncwarp(gmask);
-                if (own) { sh.imm[lig] = 1.0; sh.isd[lig] = 1.0; sh.wf_mean[lig] = 0.0; sh.wf_m2[lig] = 0.0; }
-                E0 = 0.0; s_weight = 0.0; s_sum_acc = 0.0;
-                eps = p.cfg.init_step_size; pe_cur = 0.0;
-                da_x = 0.0; da_xavg = 0.0; da_gavg = 0.0; da_prox = 0.0; da_t = 0; wf_n = 0; window_idx = 0;
-                mean_accept = 0.0; n_div = 0u;
-                m_weight = 0.0; m_sum_acc = 0.0; m_pe_p = 0.0; u_main = 0.0; m_nprop = 0; s_pe_p = 0.0;
-                h_step = 0.0; h_Er = 0.0; h_last = 0; h_dir = 0; h_att = 0u; h_call = 0u; init_attempt = 0u;
-                if (lig == 0) {
-#pragma unroll
-                    for (int j = 0; j < 5; ++j) { sh.acc_mean[j] = 0.0; sh.acc_m2[j] = 0.0; }
-                }
-                __syncwarp(gmask);
-                init_candidate();
+                zf = init_position(p, key, jc, 0u, run_kind);
+                rf = 0.0; gf = 0.0; e = 0.0;
+                phase = GP_INIT;
             }
         }
+        // layout: head
         if (__all_sync(0xffffffffu, phase == GP_IDLE)) break;
         if (phase == GP_IDLE) continue;
 
@@ -393,7 +526,7 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                 // bounded work per run: the analogue of the reference's per-fit timeout (fits.py:472-474)
                 failed = 2;
                 done = true;
-            } else if (phase == GP_LEAF) {
+            } else if (phase == GP_LEAF) {  // layout: leaf
                 // ---- hmc_util._build_basetree ----
                 double dE = pen + kinetic<D, GW>(sh.imm[jc], rn, gmask) - E0;
                 if (isnan(dE)) dE = INFINITY;
@@ -451,7 +584,7 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                 if (s_nprop < (1 << m_depth) && !turning && !s_div) {
                     // keep extending the subtree from the leaf just built
                     zf = zn; rf = rn; gf = gn;
-                } else {
+                } else {  // layout: subtree_end
                     // ---- subtree finished: _combine_tree(..., biased_transition=True) ----
                     const double dlt_m = s_weight - m_weight;
                     // min(1, e^d) and logaddexp share one exponential e^-|d| (u_main < 1, so a
@@ -482,7 +615,7 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                     m_nprop += s_nprop;
                     if (m_depth < max_depth && !m_turning && !m_div) {
                         pend = PS_DOUBLING;
-                    } else {
+                    } else {  // layout: transition_end
                         // ================= transition finished (hmc.py sample_kernel) =================
                         const double accept_prob = m_sum_acc * rcp_pos((double)m_nprop);
                         pe_cur = m_pe_p;
@@ -490,16 +623,16 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                         __syncwarp(gmask);
                         const double zc = sh.zp[jc];
                         bool want_heur = false;
-                        if (t < W) {
+                        if (t < W) {  // layout: adapt
                             // ---- warmup_adapter.update_fn ----
                             da_t += 1;
                             const double inv_t10 = rcp_pos((double)(da_t + 10));
                             da_gavg = (1.0 - inv_t10) * da_gavg + (p.cfg.target_accept - accept_prob) * inv_t10;
                             // sqrt(t) / gamma and t^-kappa (gamma = 0.05, kappa = 0.75) from the launch's tables (host libm)
                             const bool tab = da_t < kDaTable;
-                            const double sq_t = tab ? __ldg(p.da_sqrt + da_t) : sqrt((double)da_t);
+                            const double sq_t = tab ? __ldg(p.da_sqrt + da_t) : da_sqrt_cold(da_t);
                             da_x = da_prox - sq_t * 20.0 * da_gavg;
-                            const double wt = tab ? __ldg(p.da_pow + da_t) : exp_cold(-0.75 * log_cold((double)da_t));
+                            const double wt = tab ? __ldg(p.da_pow + da_t) : da_pow_cold(da_t);
                             da_xavg = (1.0 - wt) * da_xavg + wt * da_x;
                             eps = exp_cold((t == W - 1) ? da_xavg : da_x);
                             eps = fmax(eps, 2.2250738585072014e-308);
@@ -518,21 +651,8 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                             const bool at_end = (t == p.win_end[window_idx]);
                             __syncwarp(gmask);  // every lane has read window_idx before it moves
                             if (at_end) window_idx += 1;
-                            if (at_end && is_middle) {
-                                __syncwarp(gmask);
-                                if (own) {
-                                    const double cov = sh.wf_m2[lig] / (wf_n - 1);
-                                    const double v = ((double)wf_n / (wf_n + 5.0)) * cov + 1e-3 * (5.0 / (wf_n + 5.0));
-                                    sh.imm[lig] = v;
-                                    sh.isd[lig] = 1.0 / sqrt(v);
-                                    sh.wf_mean[lig] = 0.0; sh.wf_m2[lig] = 0.0;
-                                }
-                                __syncwarp(gmask);
-                                wf_n = 0;
-                                want_heur = p.cfg.find_heuristic_step_size != 0;
-                                if (!want_heur) reset_dual_averaging();
-                            }
-                        } else {
+                            if (at_end && is_middle) want_heur = window_end(p, sh, lig, gmask);
+                        } else {  // layout: kept_draw
                             // ---- after warm-up: keep the draw ----
                             const int si = t - W;
                             const double inv_n = rcp_pos((double)(si + 1));
@@ -542,7 +662,7 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                             double th[4];
                             {
                                 const double myu = zc;
-                                const double Ev = exp_fast(lig == D - 1 ? myu : -fabs(myu));
+                                const double Ev = exp_fast_split(lig == D - 1 ? myu : -fabs(myu));
                                 const double iv = rcp_pos(1.0 + Ev);
                                 const double val = (lig == D - 1) ? Ev + p.pr.phi_min : (myu >= 0.0 ? iv : Ev * iv);
                                 th[0] = __shfl_sync(gmask, val, 0, GW);
@@ -560,10 +680,7 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                                     sh.acc_m2[j] += dpre * (v[j] - mn);
                                 }
                                 const int slot = p.sample_slot[run_kind];
-                                if (p.samples != nullptr && slot >= 0) {
-                                    double* dst = p.samples + (((size_t)tax * p.sample_runs + slot) * S + si) * 4;
-                                    dst[0] = th[0]; dst[1] = th[1]; dst[2] = th[2]; dst[3] = th[3];
-                                }
+                                if (p.samples != nullptr && slot >= 0) store_sample(p, tax, slot, si, th[0], th[1], th[2], th[3]);
                             }
                             __syncwarp(gmask);
                             // WAIC: streaming logsumexp + Welford of this lane's log-likelihoods (fits.py:147-165)
@@ -584,8 +701,8 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                                 wacc[2 * wstride + s * 32] = wmean; wacc[3 * wstride + s * 32] = wm2;
                             }
                         }
-                        if (p.trace != nullptr && lig < 4)
-                            p.trace[(((size_t)tax * MDG_NUM_RUNS + run_kind) * (W + S) + t) * 4 + lig] = own ? zc : nan("");
+                        // layout: transition_end
+                        if (p.trace != nullptr && lig < 4) store_trace(p, tax, run_kind, t, lig, own ? zc : nan(""));
                         __syncwarp(gmask);
                         t += 1;
                         if (t >= W + S) {
@@ -598,13 +715,10 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                         }
                     }
                 }
-            } else if (phase == GP_HEUR) {
-                const double delta = (kinetic<D, GW>(sh.imm[jc], rn, gmask) + pen) - h_Er;
-                const int dir_new = (log_target_heur < -delta) ? 1 : -1;  // NaN -> -1
-                h_last = h_dir;
-                h_dir = dir_new;
+            } else if (phase == GP_HEUR) {  // layout: heuristic
+                heur_record<D, GW>(sh, jc, rn, pen, gmask);
                 pend = PS_HEUR;
-            } else {
+            } else {  // layout: init
                 // ---- GP_INIT: init_to_uniform(radius), retried until finite ----
                 if (valid) {
                     pe_cur = pen;
@@ -622,39 +736,35 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                     }
                 } else {
                     ++init_attempt;
-                    if (init_attempt >= 100u) { failed = 1; done = true; }
-                    else init_candidate();
+                    if (init_attempt >= 100u) {
+                        failed = 1; done = true;
+                    } else {
+                        zf = init_position(p, key, jc, init_attempt, run_kind);
+                        rf = 0.0; gf = 0.0; e = 0.0;
+                        phase = GP_INIT;
+                    }
                 }
             }
 
             // ---- what the bookkeeping asked for: aim the next leapfrog ----
-            if (pend == PS_HEUR_BEGIN) {
-                h_step = eps; h_last = 0; h_dir = 0; h_att = 0;
-                pend = PS_HEUR;
-            }
-            if (pend == PS_HEUR) {
-                const bool small_ok = (h_step > 2.2250738585072014e-308) || (h_dir >= 0);
-                const bool large_ok = (h_step < 1.7976931348623157e308) || (h_dir <= 0);
-                if (small_ok && large_ok && (h_last == 0 || h_dir == h_last)) {
-                    // next trial
-                    h_step *= (h_dir > 0 ? 2.0 : (h_dir < 0 ? 0.5 : 1.0));
-                    rf = draw_normal_lane_cold<D>(key, h_call, c2word(run_kind, P_HEUR), h_att, jc) * sh.isd[jc];
-                    ++h_att;
-                    h_Er = kinetic<D, GW>(sh.imm[jc], rf, gmask) + pe_cur;
+            if (pend == PS_HEUR_BEGIN || pend == PS_HEUR) {  // layout: heuristic
+                const double2 trial = heur_next<D, GW>(sh, pend == PS_HEUR_BEGIN, key, run_kind, jc, gmask);
+                if (trial.y != 0.0) {
+                    rf = trial.x;
                     __syncwarp(gmask);
                     zf = sh.zp[jc]; gf = sh.gp[jc];
                     e = h_step;
                     phase = GP_HEUR;
+                    pend = PS_HEUR;
                 } else {
-                    eps = h_step;
                     pend = PS_RESET;
                 }
             }
             if (pend == PS_RESET) {
-                reset_dual_averaging();
+                reset_dual_averaging(sh);
                 pend = PS_TRANSITION;
             }
-            if (pend == PS_TRANSITION) {
+            if (pend == PS_TRANSITION) {  // layout: transition_start
                 const double r0 = draw_normal_lane_cold<D>(key, (uint32_t)t, c2word(run_kind, P_MOM), 0u, jc) * sh.isd[jc];
                 E0 = pe_cur + kinetic<D, GW>(sh.imm[jc], r0, gmask);
                 __syncwarp(gmask);
@@ -670,7 +780,7 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
                 leaf_counter = 0;
                 pend = PS_DOUBLING;
             }
-            if (pend == PS_DOUBLING) {
+            if (pend == PS_DOUBLING) {  // layout: doubling
                 double u_dir;
                 uniform2(philox4x32(key, (uint32_t)m_depth, (uint32_t)t, c2word(run_kind, P_DIR), 0u), u_dir, u_main);
                 going_right = u_dir < 0.5;
@@ -685,44 +795,8 @@ __global__ void __launch_bounds__(WARPS * 32, MDG_NUTS_MINBLOCKS * 4 / WARPS) nu
         }
 
         // ================= chain finished: per-run outputs, then fetch the next item =================
-        if (done) {
-            double waic_sum = 0.0, lppd_sum = 0.0;
-            const size_t R = 2 * (size_t)P;
-            double* wout = p.waic + ((size_t)tax * MDG_NUM_RUNS + run_kind) * 2 * R;
-            double* const wacc = wacc_of_lane();
-#pragma unroll 1
-            for (int s = 0; s < ns; ++s) {
-                const int j = s * GW + lig - 1;
-                if ((unsigned)j < (unsigned)n_obs && !failed && S > 0) {
-                    const double2 d = kn[s * 32 + lane];
-                    const double logC = lgam(d.y + 1.0) - lgam(d.x + 1.0) - lgam(d.y - d.x + 1.0);  // log C(N,k)
-                    const int dense = (mask == 2 ? P : 0) + j;
-                    const double lppd_i = logC + wacc[0 * wstride + s * 32] + log_cold(wacc[1 * wstride + s * 32]) - log_cold((double)S);
-                    const double pw_i = wacc[3 * wstride + s * 32] / (double)S;
-                    wout[dense] = lppd_i;
-                    wout[R + dense] = pw_i;
-                    lppd_sum += lppd_i;
-                    waic_sum += -2.0 * (lppd_i - pw_i);
-                }
-            }
-            waic_sum = group_sum<GW>(waic_sum, gmask);
-            lppd_sum = group_sum<GW>(lppd_sum, gmask);
-            __syncwarp(gmask);
-            if (lig == 0) {
-                RunRecord& r = p.rec[(size_t)tax * MDG_NUM_RUNS + run_kind];
-                r.step_size = eps;
-                r.mean_accept = mean_accept;
-                r.n_leapfrog = n_grad;
-                r.n_divergent = n_div;
-                r.waic = waic_sum;
-                r.lppd = lppd_sum;
-#pragma unroll
-                for (int j = 0; j < 5; ++j) { r.mean[j] = sh.acc_mean[j]; r.sd[j] = S > 0 ? sqrt(sh.acc_m2[j] / (double)S) : 0.0; }
-                r.failed = (uint32_t)failed;
-                r.pad = 0;
-                if (p.chain_clock != nullptr) p.chain_clock[((size_t)tax * MDG_NUM_RUNS + run_kind) * 2 + 1] = global_timer_ns();
-            }
-            __syncwarp(gmask);
+        if (done) {  // layout: chain_end
+            chain_end<GW, D>(p, sh, kn, wacc_of_lane(), tax, run_kind, mask, n_obs, ns, failed, n_grad, lane, lig, gmask);
             // the leapfrog source is dead here; saying so keeps the compiler from carrying its old value across the
             // evaluation (in registers, which the evaluation needs) for the paths that end a chain without overwriting it
             zf = 0.0; rf = 0.0; gf = 0.0;
